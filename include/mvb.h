@@ -51,12 +51,11 @@ int64_t mvb_launch_count(void);
 /* enable (default) / disable the tcgen05 3xTF32 tensor-core kernels for the dense contractions;
  * disabled, the strict-fp32 FFMA kernels run everywhere.  Returns the previous setting. */
 int mvb_set_tensor_cores(int enable);
-/* Tuning hooks for A/B measurement runs (scripts/, tests) - not part of the operator API.  spec is a list
- * "key=a[,b];key=..." (keys: tc_tuning, tc_balance, tc_tma, layer_tuning, fused_recurrence, spmm_shape, spmm_mode, overlap,
- * mesh_tc, mesh_dbg, stream_tc, stream_nt, conv_lanes, pdl, wgrad_perm, defer_wgrad, background_div; documented next to
- * mvb_tune in csrc/mvb_api.cu).  Results are bit-identical for every setting of the grid-shape / launch keys; mesh_tc /
- * fused_recurrence / stream_tc / tc_tma select between implementations tested against each other.  The mvb Python package
- * applies the environment variable MVB_TUNE through this call when it is imported. */
+/* Run-time switches for tests and the step engine - not part of the operator API.  spec is a list
+ * "key=a[,b];key=..." (keys: mesh_tc, fused_recurrence, stream_tc, pdl, defer_wgrad; documented next to mvb_tune in
+ * csrc/mvb_api.cu); any other key is rejected with MVB_EINVAL.  mesh_tc / fused_recurrence / stream_tc select between
+ * implementations tested against each other; pdl and defer_wgrad change only how kernels are launched and joined.  The
+ * mvb Python package applies the environment variable MVB_TUNE through this call when it is imported. */
 int mvb_tune(const char *spec);
 /* Deferred side chains: with mvb_tune("defer_wgrad=1") the weight-gradient reductions of mvb_cheb_layer_bwd run on an
  * internal per-device side stream (as does the weight-gradient branch of mvb_cheb_bwd) and are NOT joined into the

@@ -113,11 +113,11 @@ def check(rc: int, what: str = ""):
 
 
 def tune(spec: str):
-    """A/B tuning hooks (include/mvb.h: mvb_tune), e.g. tune("spmm_mode=1;mesh_tc=1,2")"""
+    """run-time switches (include/mvb.h: mvb_tune), e.g. tune("fused_recurrence=0;mesh_tc=1,2")"""
     check(lib.mvb_tune(spec.encode()), "mvb_tune")
 
 
-if os.environ.get("MVB_TUNE"):          # A/B runs of the tuning hooks (tests, bench, scripts alike)
+if os.environ.get("MVB_TUNE"):          # A/B runs of the switches (tests, bench, scripts alike)
     tune(os.environ["MVB_TUNE"])
 
 

@@ -299,7 +299,6 @@ struct SideStream {
     cudaEvent_t fork = nullptr, join = nullptr;
     bool ok = false;
 };
-static int g_overlap = 1;
 static SideStream *side_stream() {
     static thread_local SideStream s;
     static thread_local bool tried = false;
@@ -327,9 +326,8 @@ static SideStream *side_stream() {
 // first encoder layer, which needs no dX, keeps the basis form: its basis is only 3-4 columns wide).
 static bool adjoint_form(int Fin, int Fout, int need_dx) { return need_dx && 25 * Fout <= 30 * Fin && Fout % 4 == 0; }
 
-// fork the per-thread side stream from `st` (NULL when overlap is off or the fork fails)
+// fork the per-thread side stream from `st` (NULL when the fork fails)
 static SideStream *fork_side(cudaStream_t st) {
-    if (!g_overlap) return nullptr;
     SideStream *side = side_stream();
     if (!side) return nullptr;
     if (cudaEventRecord(side->fork, st) != cudaSuccess || cudaStreamWaitEvent(side->stream, side->fork, 0) != cudaSuccess) {
@@ -349,21 +347,6 @@ struct JoinGuard {   // the side stream must rejoin on every exit path (a captur
     }
 };
 
-// the same fork / join for other translation units (mvb_layer.cu): returns the side stream or NULL
-namespace mvb {
-cudaStream_t side_fork(cudaStream_t st) {
-    SideStream *s = fork_side(st);
-    return s ? s->stream : nullptr;
-}
-void side_join(cudaStream_t side, cudaStream_t st) {
-    SideStream *s = side_stream();
-    if (side && s && s->stream == side) {
-        cudaEventRecord(s->join, s->stream);
-        cudaStreamWaitEvent(st, s->join, 0);
-    }
-}
-}  // namespace mvb
-
 // ---------------------------------------------------------------------------------------------
 // Deferred side chains.  The weight-gradient reduction of a mesh-resident layer (tc_wgrad + finalize kernels, 10-20 us)
 // is not on the critical path of the backward pass: nothing reads dW / db before the optimizer.  In deferred mode
@@ -381,22 +364,17 @@ struct LazySide {
     cudaEvent_t fork = nullptr, join = nullptr;
     bool tried = false, ok = false, pending = false;
 };
-constexpr int LAZY_SLOTS = 8;       // slot 1 = lane 1 (dense-layer weight gradients); slots 0, 2..7 = lane 0 (convolution weight gradients:
-                                    // successive chains go round robin over g_conv_lanes of them, so that chains can overlap each other)
+constexpr int LAZY_SLOTS = 4;       // slot 1 = lane 1 (dense-layer weight gradients); slots 0, 2, 3 = lane 0 (convolution weight gradients:
+                                    // successive chains go round robin over CONV_LANES of them, so that chains can overlap each other)
 static LazySide g_lazy[64][LAZY_SLOTS];
-static int g_conv_lanes = 3;        // tuning: conv_lanes=1..7; same-box A/B (bench.py, 300 steps, second pass): 1 lane 0.9197 ms per step,
-                                    // 2: 0.9152, 3: 0.9116, 4: 0.9109, 5: 0.9111, 7: 0.9109 - the chains queued behind each other in the tail of the
+constexpr int CONV_LANES = 3;       // same-box A/B (bench.py, 300 steps, second pass): 1 lane 0.9197 ms per step, 2: 0.9152, 3: 0.9116,
+                                    // 4: 0.9109, 5: 0.9111, 7: 0.9109 - the chains queued behind each other in the tail of the
                                     // backward pass (the last layers' reductions) now run side by side
 static int g_conv_next[64] = {0};
-void set_conv_lanes(int v) { if (v >= 1 && v <= 7) g_conv_lanes = v; }
-static const int kConvSlot[7] = {0, 2, 3, 4, 5, 6, 7};
+static const int kConvSlot[CONV_LANES] = {0, 2, 3};
 static std::mutex g_lazy_mu;
 static int g_defer_wgrad = 0;
 void set_defer_wgrad(int v) { g_defer_wgrad = v ? 1 : 0; }
-static int g_background_div = 0;        // deferred level-0 weight-gradient reduction: SMs per CTA, 0 = the usual two CTAs per SM
-                                        // (tuning: background_div; measured at 64 meshes: 0 -> 921 us per step, 1 -> 948, 2 -> 988:
-                                        // the slower reduction delays every chain queued behind it more than it spares the main stream)
-void set_background_div(int v) { g_background_div = v < 0 ? 0 : v; }
 
 static LazySide *lazy_side(int slot) {
     int dev = 0;
@@ -436,8 +414,8 @@ cudaStream_t lazy_fork(cudaStream_t st, int lane) {
     if (lane == 0) {
         int dev = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-        slot = kConvSlot[g_conv_next[dev] % g_conv_lanes];
-        g_conv_next[dev] = (g_conv_next[dev] + 1) % g_conv_lanes;
+        slot = kConvSlot[g_conv_next[dev]];
+        g_conv_next[dev] = (g_conv_next[dev] + 1) % CONV_LANES;
     }
     LazySide *s = lazy_side(slot);
     if (!s) return nullptr;
@@ -478,7 +456,7 @@ extern "C" int mvb_side_join_lane(void *stream, int lane) {
     if (lane == 1) {
         mvb::lazy_join_locked(mvb::lazy_side(1), (cudaStream_t)stream);
     } else {
-        for (int c = 0; c < 7; ++c) mvb::lazy_join_locked(mvb::lazy_side(mvb::kConvSlot[c]), (cudaStream_t)stream);
+        for (int c = 0; c < mvb::CONV_LANES; ++c) mvb::lazy_join_locked(mvb::lazy_side(mvb::kConvSlot[c]), (cudaStream_t)stream);
     }
     return MVB_OK;
 }
@@ -730,9 +708,6 @@ static int cheb_bwd_adjoint(int N, int B, int Fin, int Fout, int K, int n_active
         wa.n_out = Fin;
         wa.partials = partA;
         wa.partial_bytes = partA_bytes;
-        // (tuning hook) deferred chain of a level too large for L2: fewer CTAs, so that the HBM-bound kernels of the
-        // critical path that follow keep more of the memory system - measured a net loss, off by default
-        wa.background = (lazy && rows_act * (int64_t)K * Fout * 4 > (int64_t)64 << 20) ? g_background_div : 0;
         rc = launch_wgrad_partials(wa, 0, &nA, &m4A, wst);
         if (rc) return rc;
     }
@@ -773,24 +748,12 @@ extern "C" int mvb_stream_wait_external_event(void *stream, void *event) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// tuning hooks for A/B runs (scripts/, tests): NOT part of the operator API.  spec = "key=a[,b];key=..."
-//   tc_tuning=pg,cap   planes staged at a time by the 6-plane row GEMM (1,2,3,6) / resident CTAs per SM (1..4)
-//   tc_balance=0|1     equal tile counts per row-GEMM block
-//   layer_tuning=p,c   FFMA mesh-layer backward: blocks per SM, concurrent halves
-//   fused_recurrence=v 0 off, 1 on, >= 64 on with that many threads
-//   spmm_shape=tx,chunk / spmm_mode=m   SpMM block shape / size (0 = automatic)
-//   overlap=0|1        side-stream fork inside mvb_cheb_bwd
+// run-time switches (tests, the step engine): NOT part of the operator API.  spec = "key=a[,b];key=..."
 //   mesh_tc=e,c        tensor-core mesh layers on/off, CTAs per mesh (0 = automatic)
-//   defer_wgrad=0|1    weight-gradient chains of the mesh layers joined lazily (engine only; see mvb_side_join)
+//   fused_recurrence=0|1  one-launch Chebyshev recurrence for the levels that fit shared memory off / on
 //   stream_tc=e,sw     row-streaming fused level-0 layers (mvb_cheb_stream_*) on/off, meshes per slab (8 / 16, 0 = least work per CTA)
-//   stream_nt=n        threads per CTA of that kernel (1024 / 768)
-//   tc_tma=e,ring      TMA-fed row GEMM for the 16-wide planes on/off, hi tiles in the ring (3 / 4)
-//   conv_lanes=n       side streams the deferred convolution weight-gradient chains rotate over (1..7, default 3)
 //   pdl=0|1            programmatic dependent launch of the step's kernels (default on; the engine switches it off for N > 1)
-//   wgrad_perm=0|1     conflict-free lane order of the staging stores in tc_wgrad (default off)
-//   background_div=d   grid of the deferred level-0 weight-gradient reduction: one CTA per d SMs (0 = two per SM)
-//   mesh_dbg=bits      timing probes of the tensor-core mesh forward kernel (1 no MMAs, 2 no recurrence, 4 no epilogue):
-//                      results are then wrong - scripts/mesh_tc_probe.py only
+//   defer_wgrad=0|1    weight-gradient chains of the mesh layers joined lazily (engine only; see mvb_side_join)
 // ---------------------------------------------------------------------------------------------
 extern "C" int mvb_tune(const char *spec) {
     MVB_REQUIRE(spec != nullptr, "mvb_tune: null spec");
@@ -813,23 +776,11 @@ extern "C" int mvb_tune(const char *spec) {
         }
         while (*p && *p != ';') ++p;
         if (*p == ';') ++p;
-        if (!strcmp(key, "tc_tuning")) { if (v[0]) set_tc_pg6(v[0]); if (v[1]) set_tc_cap(v[1]); }
-        else if (!strcmp(key, "tc_balance")) set_tc_balance(v[0]);
-        else if (!strcmp(key, "tc_tma")) set_tc_tma(v[0], v[1]);
-        else if (!strcmp(key, "layer_tuning")) set_layer_tuning(v[0], v[1]);
+        if (!strcmp(key, "mesh_tc")) set_mesh_tc(v[0], v[1]);
         else if (!strcmp(key, "fused_recurrence")) set_recur_fused(v[0]);
-        else if (!strcmp(key, "spmm_shape")) set_spmm_shape(v[0], v[1]);
-        else if (!strcmp(key, "spmm_mode")) set_spmm_mode(v[0] & 15);
-        else if (!strcmp(key, "overlap")) g_overlap = v[0] ? 1 : 0;
-        else if (!strcmp(key, "mesh_tc")) set_mesh_tc(v[0], v[1]);
-        else if (!strcmp(key, "mesh_dbg")) set_mesh_dbg(v[0]);
         else if (!strcmp(key, "stream_tc")) set_stream_tc(v[0], nv > 1 ? v[1] : -1);
-        else if (!strcmp(key, "stream_nt")) set_stream_nt(v[0]);
-        else if (!strcmp(key, "wgrad_perm")) set_wgrad_perm(v[0]);
-        else if (!strcmp(key, "conv_lanes")) set_conv_lanes(v[0]);
         else if (!strcmp(key, "pdl")) set_pdl(v[0]);
         else if (!strcmp(key, "defer_wgrad")) set_defer_wgrad(v[0]);
-        else if (!strcmp(key, "background_div")) set_background_div(v[0]);
         else if (key[0]) return set_err(MVB_EINVAL, "mvb_tune: unknown key '%s'", key);
     }
     return MVB_OK;

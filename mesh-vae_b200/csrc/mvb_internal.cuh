@@ -181,10 +181,6 @@ struct WgradArgs {
     const int32_t *row_sel;
     int sel_group;
     int64_t plane_rows;
-    // > 0: a reduction that runs as a deferred side chain next to kernels of the critical path - one CTA per
-    // `background` SMs... i.e. the grid is num_sms() / background instead of two CTAs per SM, so that it takes a
-    // fraction of the block slots and of the memory system instead of half of them
-    int background;
 };
 size_t wgrad_partial_bytes(int M, int n_out);
 int launch_wgrad_partials(const WgradArgs &a, int has_bias, int *nparts, int *m4_out, cudaStream_t st);
@@ -207,21 +203,11 @@ int launch_contract_tc(const ContractArgs &a, cudaStream_t st);
 int tc_enabled();
 int launch_wgrad_tc(const WgradArgs &a, int has_bias, int M4, int N4, int *nparts, cudaStream_t st);
 
-// tuning setters behind mvb_tune (mvb_api.cu)
-void set_tc_pg6(int v);
-void set_tc_cap(int v);
-void set_tc_balance(int v);
-void set_tc_tma(int v, int nb);
-void set_layer_tuning(int v, int conc);
+// setters behind mvb_tune (mvb_api.cu)
 void set_recur_fused(int v);
-void set_spmm_shape(int tx, int chunk);
-void set_spmm_mode(int v);
 void set_mesh_tc(int enable, int c);
-void set_mesh_dbg(int v);
 void set_stream_tc(int v, int sw);
-void set_stream_nt(int v);
 void set_pdl(int v);
-void set_wgrad_perm(int v);
 
 // mesh-resident tensor-core layers (mvb_mesh_tc.cu): 1 = handled / supported, 0 = shape not covered, < 0 = error
 int mesh_tc_fwd_supported(int N, int B, int Fin, int Fout, int K, int Lnnz, int n_in, int n_out);
@@ -241,9 +227,5 @@ int launch_layer_finalize(int B, int nw, int nb, const float *dwp, const float *
 // deferred side chains (mvb_api.cu): see lazy_fork / lazy_done / mvb_side_join
 cudaStream_t lazy_fork(cudaStream_t st, int lane = 0);
 void lazy_done(cudaStream_t side, cudaStream_t st);
-
-// fork a per-thread side stream from `st` (NULL: no overlap) / make `st` wait for it again (mvb_api.cu)
-cudaStream_t side_fork(cudaStream_t st);
-void side_join(cudaStream_t side, cudaStream_t st);
 
 }  // namespace mvb

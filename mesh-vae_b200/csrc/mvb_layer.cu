@@ -304,19 +304,11 @@ cheb_layer_bwd_kernel(LayerArgs a, LayerSmem S) {
             const int in = ki % Fin, k = ki / Fin;
             Ws[(k * Fout + o) * Fin + in] = __ldg(a.w + i);
         }
-    // two modes besides "everything": a.dwp == NULL - input gradient only (pass 2), a.out == NULL - weight gradient
-    // only (pass 1).  The launcher runs them as two concurrent kernels: both are chains of short barrier-separated
-    // phases that leave most issue slots idle, and the weight gradient is off the critical path of the backward pass.
-    const bool want_dw = a.dwp != nullptr;
-    if (want_dw) stage_csr_async(sm + S.csr, N, a.Lnnz, a.Lrp, a.Lci, a.Lv, lrp, lce, tid);
+    // a.out == NULL: weight gradient only (pass 1)
+    stage_csr_async(sm + S.csr, N, a.Lnnz, a.Lrp, a.Lci, a.Lv, lrp, lce, tid);
     stage_mesh_rows(G, LDG, a.dy, a.n_out, a.B, b, Fout, 0, lcq, tid);
     for (int v = tid; v < N; v += LY_NT) inv[v] = a.sel ? -1 : v;
-    if (want_dw) {
-        stage_t0(a, sm, S, b, tid, c0, lqf);
-    } else {
-        cp_async_wait_all();
-        __syncthreads();
-    }
+    stage_t0(a, sm, S, b, tid, c0, lqf);
     if (a.sel)
         for (int r = tid; r < a.n_out; r += LY_NT) inv[__ldg(a.sel + r)] = r;
     if (a.relu)                                              // G = dY * [y > 0]
@@ -370,16 +362,14 @@ cheb_layer_bwd_kernel(LayerArgs a, LayerSmem S) {
         }
     };
     float *cur = sm + S.tA, *old = sm + S.tB;
-    if (want_dw) {
-        wgrad(cur, 0);
-        for (int k = 1; k < K; ++k) {
-            recur_step(cur, old, N, lqf, LDT, lrp, lce, k, tid);
-            __syncthreads();
-            wgrad(old, k);
-            float *t = cur; cur = old; old = t;
-        }
+    wgrad(cur, 0);
+    for (int k = 1; k < K; ++k) {
+        recur_step(cur, old, N, lqf, LDT, lrp, lce, k, tid);
+        __syncthreads();
+        wgrad(old, k);
+        float *t = cur; cur = old; old = t;
     }
-    if (want_dw && a.dbp && blockIdx.y == 0 && tid < Fout) {
+    if (a.dbp && blockIdx.y == 0 && tid < Fout) {
         float s = 0.f;
         for (int r = 0; r < a.n_out; ++r) s += G[r * LDG + tid];
         a.dbp[(int64_t)b * Fout + tid] = s;
@@ -503,21 +493,15 @@ layer_finalize_kernel(int B, int nw, int nb, const float *__restrict__ dwp, cons
 static bool pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
 
 // blocks per mesh: as many as keep every SM busy when the batch is small, while a block keeps >= `min_q` quads
-static int pick_splits(int B, int quads, int min_q, int per_sm = 1) {
+// (one block per SM: two feature splits per mesh of the backward pass at 64 meshes.  Sizing it for two blocks per SM - 4
+// splits, kernel capped at 64 registers - measured 157 us against 149 us for the four backward layers of a step: the
+// per-block instruction count does not shrink with the split.  Running the dW and dX halves of the backward layer as two
+// concurrent kernels measured 63 us for the pair against 59 us for the single kernel at level 2: both halves saturate
+// the same shared-memory pipe; profiles/README.md)
+static int pick_splits(int B, int quads, int min_q) {
     int s = 1;
-    while (B * s * 2 <= per_sm * (num_sms() + num_sms() / 2) && quads / (s * 2) >= min_q) s *= 2;
+    while (B * s * 2 <= num_sms() + num_sms() / 2 && quads / (s * 2) >= min_q) s *= 2;
     return s;
-}
-// blocks per SM the backward grid is sized for (tuning: mvb_set_layer_tuning).  1: two feature splits per mesh at 64
-// meshes.  Sizing it for two blocks per SM (4 splits, kernel capped at 64 registers) measured 157 us against 149 us for
-// the four backward layers of a step: the per-block instruction count does not shrink with the split.
-static int g_layer_bwd_per_sm = 1;
-// dW and dX halves of the backward layer as two concurrent kernels: OFF - measured 63 us for the pair against 59 us for
-// the single kernel at level 2 (both halves saturate the same shared-memory pipe; profiles/README.md)
-static int g_layer_bwd_concurrent = 0;
-void set_layer_tuning(int v, int conc) {
-    if (v >= 1 && v <= 4) g_layer_bwd_per_sm = v;
-    g_layer_bwd_concurrent = conc ? 1 : 0;
 }
 
 static int layer_check(int N, int B, int Fin, int Fout, int K, int Lnnz, int n_in, int Unnz, int n_out, bool backward,
@@ -528,7 +512,7 @@ static int layer_check(int N, int B, int Fin, int Fout, int K, int Lnnz, int n_i
     if (!pow2(QF) || !pow2(CQ)) return 0;
     // forward splits the output columns (each split redoes the cheap recurrence), backward the input features
     // (the backward splits redo nothing - the recurrences are per feature column)
-    const int splits = backward ? pick_splits(B, QF, 1, g_layer_bwd_per_sm) : pick_splits(B, CQ, 2);
+    const int splits = backward ? pick_splits(B, QF, 1) : pick_splits(B, CQ, 2);
     const int ql = (backward ? QF : CQ) / splits;                 // local tile-column quads
     if (n_out > LY_MAXT * 4 * (LY_NT / ql)) return 0;
     if (backward && (QF / splits) * CQ > LY_NT) return 0;
@@ -648,29 +632,8 @@ extern "C" int mvb_cheb_layer_bwd(int N, int B, int Fin, int Fout, int K, const 
     }
     cudaStream_t st = (cudaStream_t)stream;
     const int nw = K * Fin * Fout, nb = dbias ? Fout : 0;
-    cudaStream_t side = (dx && g_layer_bwd_concurrent) ? side_fork(st) : nullptr;
-    int rc;
-    if (side) {
-        // weight gradient (pass 1 + ordered sum over the meshes) on the side stream, input gradient (pass 2) on `st`
-        LayerArgs aw = a, ax = a;
-        aw.out = nullptr;
-        ax.dwp = nullptr;
-        ax.dbp = nullptr;
-        cheb_layer_bwd_kernel<<<dim3(B, splits), LY_NT, smem, st>>>(ax, S);
-        rc = check_launch("mvb_cheb_layer_bwd dx");
-        if (!rc) {
-            cheb_layer_bwd_kernel<<<dim3(B, splits), LY_NT, smem, side>>>(aw, S);
-            rc = check_launch("mvb_cheb_layer_bwd dw");
-        }
-        if (!rc) {
-            launch_pdl(layer_finalize_kernel, dim3((nw + nb + 31) / 32), dim3(256), 0, side, B, nw, nb, a.dwp, a.dbp, dweight, dbias);
-            rc = check_launch("mvb_cheb_layer_bwd finalize");
-        }
-        side_join(side, st);          // rejoin on every path: a captured graph must not end forked
-        return rc;
-    }
     cheb_layer_bwd_kernel<<<dim3(B, splits), LY_NT, smem, st>>>(a, S);
-    rc = check_launch("mvb_cheb_layer_bwd");
+    const int rc = check_launch("mvb_cheb_layer_bwd");
     if (rc) return rc;
     return launch_layer_finalize(B, nw, nb, a.dwp, a.dbp, dweight, dbias, st);
 }

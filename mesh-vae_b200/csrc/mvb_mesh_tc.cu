@@ -29,13 +29,10 @@
 
 namespace mvb {
 
-#ifndef MVB_MT_NT
-#define MVB_MT_NT 768
-#endif
 // threads per CTA: the recurrence is a chain of shared-memory latencies, but every step also ends in a block barrier and the
 // gathers share one LSU pipe - same-box A/B of the whole step (scripts/trace_step.py): 1024 threads 923 us, 896: 907, 768: 906-908,
-// 640: 914, 512: 921; every mesh launch is 1-4 us shorter at 768 than at 1024 (-DMVB_MT_NT=... builds a variant for MVB_LIB)
-constexpr int MT_NT = MVB_MT_NT;
+// 640: 914, 512: 921; every mesh launch is 1-4 us shorter at 768 than at 1024
+constexpr int MT_NT = 768;
 constexpr int MT_NC = MT_NT - 32;    // ... of which the last warp only issues the MMAs (and so never delays a step)
 constexpr int MT_ISSUER = MT_NC;     // thread that issues tcgen05.mma / tcgen05.commit
 
@@ -49,8 +46,6 @@ struct MeshTcArgs {
     int relu;
     float *out;
     int C;                                                        // CTAs per mesh
-    int dbg;                                                      // probe bits (mvb_tune mesh_dbg): 1 no MMAs, 2 no recurrence, 4 no epilogue
-    unsigned long long *prof;                                     // debug: phase time stamps of CTA 0 (mvb_debug_mesh_prof), else NULL
     int tiles;                                                    // ceil(N / 128)
     int tmem_cols;
     // shared-memory offsets (bytes from the 1024-aligned base)
@@ -109,14 +104,6 @@ __device__ __forceinline__ void sts_f(uint32_t a, float v) { asm volatile("st.sh
 // Swizzled byte offset of 16-byte chunk q of row r: r*RB + ((q ^ x(r)) << 4) with x(r) = the row bits the UMMA swizzle
 // mode XORs in.  As r*RB has no bits below 5 + log2(WL/8), this is (r*RB | x(r) << 4) ^ (q << 4): the row part is
 // precomputed per operator entry (row_code), the quad part per thread.
-__device__ __forceinline__ void prof_stamp(unsigned long long *prof, int slot) {
-    if (prof && blockIdx.x == 0 && threadIdx.x == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        prof[slot] = t;
-    }
-}
-
 template <int WL>
 __device__ __forceinline__ uint32_t row_code(int r) {
     constexpr int RB = WL * 4;
@@ -275,7 +262,6 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
     uint64_t *bar = reinterpret_cast<uint64_t *>(smg + a.o_bar);
     uint32_t *slot = reinterpret_cast<uint32_t *>(bar + 2);            // bar[0]: commits of even steps (all steps without lo2), bar[1]: odd
 
-    prof_stamp(a.prof, 0);
     pdl_trigger();
     if (warp == 0) tmem_alloc(slot, (uint32_t)a.tmem_cols);
     if (tid == 0) {
@@ -283,9 +269,7 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
         mbar_init(bar + 1, 1);
         fence_barrier_init();
     }
-    prof_stamp(a.prof, 1);
     stage_operator<WL>(a, rows, ce, tid);
-    prof_stamp(a.prof, 2);
     // ---- B operands: Bt_k[n][kd] = W_k[c*WL + kd][n], K-major, swizzled like the planes, hi / lo ----
     for (int i = tid; i < K * WL * Fout; i += MT_NT) {
         const int n = i % Fout, kk = i / Fout;
@@ -300,7 +284,6 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
     if (a.sel) {
         for (int v = tid; v < N; v += MT_NT) sts_i(inv + 4u * v, -1);
     }
-    prof_stamp(a.prof, 3);
     pdl_wait();          // everything above reads only the operator and the weights; x is the previous kernel's output
     // ---- T_0 into plane A (+ its lo part) ----
     const int64_t xrow = (int64_t)a.B * Fin;               // floats between consecutive vertices of one mesh
@@ -347,19 +330,16 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
             }
         }
     }
-    prof_stamp(a.prof, 4);
     fence_proxy_async();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    prof_stamp(a.prof, 5);
     if (a.sel) {
         for (int r = tid; r < a.n_out; r += MT_NT) sts_i(inv + 4u * (uint32_t)__ldg(a.sel + r), r);
     }
     const uint32_t tmem_base = *slot;
     const uint32_t idesc = make_idesc(128, Fout, 0, 0);
-    const bool mma_on = !(a.dbg & 1);
-    if (tid == MT_ISSUER && mma_on) {
+    if (tid == MT_ISSUER) {
         issue_step_mmas<WL>(a, tmem_base, pa, plo, bhi, blo, 0, Fout, idesc);
         umma_commit(bar);
     }
@@ -371,32 +351,25 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
         const uint32_t lo_k = (lo2 && (k & 1)) ? plo2 : plo;
         uint64_t *bar_w = lo2 ? bar + (k & 1) : bar;
         const uint32_t par_w = lo2 ? (uint32_t)(((k >> 1) + 1) & 1) : (uint32_t)((k - 1) & 1);
-        recur_step<WL>(cur, old, lo_k, rows, ce, (a.dbg & 2) ? 0 : N, k, bar_w, par_w, mma_on && !(lo2 && k < 2), tid, nullptr, 0);
-        prof_stamp(a.prof, 4 + 2 * k);
+        recur_step<WL>(cur, old, lo_k, rows, ce, N, k, bar_w, par_w, !(lo2 && k < 2), tid, nullptr, 0);
         fence_proxy_async();
         tc_fence_before();
         __syncthreads();
-        prof_stamp(a.prof, 5 + 2 * k);
-        if (tid == MT_ISSUER && mma_on) {
+        if (tid == MT_ISSUER) {
             tc_fence_after();
             issue_step_mmas<WL>(a, tmem_base, old, lo_k, bhi, blo, k, Fout, idesc);
             umma_commit(lo2 ? bar + (k & 1) : bar);
         }
         const uint32_t t = cur; cur = old; old = t;
     }
-    prof_stamp(a.prof, 20);
-    if (mma_on) {          // the last commit (tcgen05.commit tracks every MMA issued before it)
-        const int kl = K - 1;
-        mbar_wait(lo2 ? bar + (kl & 1) : bar, lo2 ? (uint32_t)((kl >> 1) & 1) : (uint32_t)(kl & 1));
-    }
+    const int kl = K - 1;          // the last commit (tcgen05.commit tracks every MMA issued before it)
+    mbar_wait(lo2 ? bar + (kl & 1) : bar, lo2 ? (uint32_t)((kl >> 1) & 1) : (uint32_t)(kl & 1));
     tc_fence_after();
-    prof_stamp(a.prof, 21);
 
     // ---- epilogue: TMEM -> registers -> bias / ReLU -> the rows D keeps ----
     const int quarter = warp & 3, group = warp >> 2;            // a warp reads TMEM lanes [32 (warp % 4), +32)
     constexpr int NG = MT_NT / 128;
-    if (a.dbg & 4) {
-    } else if (a.C == 1) {
+    if (a.C == 1) {
         for (int t = group; t < a.tiles; t += NG) {
             const int row = t * 128 + quarter * 32 + lane;
             const int ro = (row < N) ? (a.sel ? lds_i(inv + 4u * row) : row) : -1;
@@ -424,7 +397,6 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
         const int H = Fout >> 1, HQ = H >> 2;
         const uint32_t theirs = pb;
         cluster_sync_all();                      // the partner's MMAs no longer read its planes
-        prof_stamp(a.prof, 16);
         const uint32_t theirs_remote = map_to_cta(theirs, (uint32_t)(c ^ 1));
         const int ps = (c ^ 1) * H;              // first column of the partner's half
         for (int t = group; t < a.tiles; t += NG) {
@@ -443,9 +415,7 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
                 }
             }
         }
-        prof_stamp(a.prof, 17);
         cluster_sync_all();                      // both halves are in place
-        prof_stamp(a.prof, 18);
         for (int t = group; t < a.tiles; t += NG) {
             const int row = t * 128 + quarter * 32 + lane;
             const int ro = (row < N) ? (a.sel ? lds_i(inv + 4u * row) : row) : -1;
@@ -470,11 +440,9 @@ cheb_mesh_tc_fwd_kernel(const MeshTcArgs a) {
             }
         }
     }
-    prof_stamp(a.prof, 22);
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)a.tmem_cols);
-    prof_stamp(a.prof, 23);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -701,9 +669,6 @@ cheb_mesh_tc_bwd_kernel(const MeshTcBwdArgs g) {
 // ---------------------------------------------------------------------------------------------
 static int g_mesh_tc = 1;            // 0: the FFMA mesh-resident kernels of mvb_layer.cu (A/B runs)
 static int g_mesh_tc_c = 0;          // 0: automatic cluster size, 1 / 2: forced
-static int g_mesh_dbg = 0;           // probe bits for timing attribution (results are then WRONG): see MeshTcArgs::dbg
-void set_mesh_dbg(int v) { g_mesh_dbg = v; }
-static unsigned long long *g_mesh_prof = nullptr;
 void set_mesh_tc(int enable, int c) { g_mesh_tc = enable ? 1 : 0; g_mesh_tc_c = (c == 1 || c == 2) ? c : 0; }
 
 static int pow2_cols_m(int n) {
@@ -818,8 +783,6 @@ int launch_mesh_tc_fwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lr
     a.n_in = n_in; a.Urp = Urp; a.Uci = Uci; a.Uv = Uv;
     a.n_out = n_out; a.sel = sel;
     a.x = x; a.w = w; a.bias = bias; a.relu = relu; a.out = y;
-    a.dbg = g_mesh_dbg;
-    a.prof = g_mesh_prof;
     const int c = pick_mesh_c(a, Fin, Fout);
     if (!c) return 0;
     int rc;
@@ -967,7 +930,3 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
 }
 
 }  // namespace mvb
-
-// debug hook (scripts/mesh_tc_probe.py; not in include/mvb.h): 24 uint64 %globaltimer stamps of CTA 0 of the next
-// tensor-core mesh forward launches are written to `buf` (device memory); NULL switches it off
-extern "C" void mvb_debug_mesh_prof(void *buf) { mvb::g_mesh_prof = reinterpret_cast<unsigned long long *>(buf); }

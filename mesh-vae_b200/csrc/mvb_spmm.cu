@@ -309,11 +309,9 @@ cheb_recur_bwd_kernel(int N, int K, const int32_t *__restrict__ g_rowptr, const 
     }
 }
 
-static int g_recur_fused = 1, g_recur_threads = 1024;
-void set_recur_fused(int v) {          // 0 = off, 1 = on, >= 64: on with that many threads per block (tuning runs)
-    g_recur_fused = v != 0;
-    if (v >= 64 && v <= 1024) g_recur_threads = v & ~31;
-}
+static int g_recur_fused = 1;
+void set_recur_fused(int v) { g_recur_fused = v != 0; }
+constexpr int RECUR_NT = 1024;         // threads per block of the fused recurrences
 
 static bool recur_shape(int N, int nnz, int64_t ncols, const void *a, const void *b, int *cs4, size_t *smem, int *nnz_smem) {
     if (!g_recur_fused || N < 1 || ncols % 4 != 0 || !aligned16(a) || !aligned16(b)) return false;
@@ -352,11 +350,11 @@ int launch_cheb_recur_fwd(int N, int nnz, int K, const int32_t *rowptr, const in
     if (cs4 == 2) {
         if (smem_optin(cheb_recur_fwd_kernel<2>, 200 * 1024, optin2, "cheb_recur_fwd_kernel")) e = cudaErrorInvalidValue;
         if (e == cudaSuccess)
-            launch_pdl(cheb_recur_fwd_kernel<2>, dim3(grid), dim3(g_recur_threads), smem, st, N, K, rowptr, colidx, vals, (const float4 *)x, (float4 *)basis, nc4, nnz_smem);
+            launch_pdl(cheb_recur_fwd_kernel<2>, dim3(grid), dim3(RECUR_NT), smem, st, N, K, rowptr, colidx, vals, (const float4 *)x, (float4 *)basis, nc4, nnz_smem);
     } else {
         if (smem_optin(cheb_recur_fwd_kernel<1>, 200 * 1024, optin1, "cheb_recur_fwd_kernel")) e = cudaErrorInvalidValue;
         if (e == cudaSuccess)
-            launch_pdl(cheb_recur_fwd_kernel<1>, dim3(grid), dim3(g_recur_threads), smem, st, N, K, rowptr, colidx, vals, (const float4 *)x, (float4 *)basis, nc4, nnz_smem);
+            launch_pdl(cheb_recur_fwd_kernel<1>, dim3(grid), dim3(RECUR_NT), smem, st, N, K, rowptr, colidx, vals, (const float4 *)x, (float4 *)basis, nc4, nnz_smem);
     }
     if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_recur_fwd: %s", cudaGetErrorString(e));
     int rc = check_launch("mvb cheb_recur_fwd");
@@ -375,21 +373,17 @@ int launch_cheb_recur_bwd(int N, int nnz, int K, const int32_t *rowptr_t, const 
     if (cs4 == 2) {
         if (smem_optin(cheb_recur_bwd_kernel<2>, 200 * 1024, optin2, "cheb_recur_bwd_kernel")) e = cudaErrorInvalidValue;
         if (e == cudaSuccess)
-            cheb_recur_bwd_kernel<2><<<grid, g_recur_threads, smem, st>>>(N, K, rowptr_t, colidx_t, vals_t, (const float4 *)P, (float4 *)dx, nc4, nnz_smem);
+            cheb_recur_bwd_kernel<2><<<grid, RECUR_NT, smem, st>>>(N, K, rowptr_t, colidx_t, vals_t, (const float4 *)P, (float4 *)dx, nc4, nnz_smem);
     } else {
         if (smem_optin(cheb_recur_bwd_kernel<1>, 200 * 1024, optin1, "cheb_recur_bwd_kernel")) e = cudaErrorInvalidValue;
         if (e == cudaSuccess)
-            cheb_recur_bwd_kernel<1><<<grid, g_recur_threads, smem, st>>>(N, K, rowptr_t, colidx_t, vals_t, (const float4 *)P, (float4 *)dx, nc4, nnz_smem);
+            cheb_recur_bwd_kernel<1><<<grid, RECUR_NT, smem, st>>>(N, K, rowptr_t, colidx_t, vals_t, (const float4 *)P, (float4 *)dx, nc4, nnz_smem);
     }
     if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_recur_bwd: %s", cudaGetErrorString(e));
     int rc = check_launch("mvb cheb_recur_bwd");
     return rc ? rc : 1;
 }
 
-static int g_spmm_tx = 0, g_spmm_chunk = 0;      // 0 = automatic; set through mvb_set_spmm_shape for tuning runs
-void set_spmm_shape(int tx, int chunk) { g_spmm_tx = tx; g_spmm_chunk = chunk; }
-static int g_spmm_mode = 0;   // 0 = automatic block size, 1/2/3 = force 256/512/1024-thread blocks (tuning runs)
-void set_spmm_mode(int v) { g_spmm_mode = v; }
 int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t *colidx, const float *vals,
                 const float *x, float *y, const float *z, const float *w, float alpha, float beta,
                 int64_t ncols, cudaStream_t st) {
@@ -410,11 +404,9 @@ int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t
         // The grid is ONE WAVE: exactly as many blocks as the GPU holds at once, each with an equal share of
         // the rows.  The kernel is latency-bound, so a trailing partial wave costs as much as a full one:
         // at 64 meshes the 64-row chunks gave 632 blocks = 2.13 waves and 17.3 us, 296 blocks of 136 rows
-        // give 14.7 us (0.54 -> 0.64 of the HBM peak; scripts/spmm_ab.py, profiles/README.md).
-        int tx = g_spmm_tx, chunk = g_spmm_chunk;
-        int nthreads = (g_spmm_mode == 2) ? 512 : (g_spmm_mode == 3 ? 1024 : 256);
-        if (g_spmm_mode == 0 && tx <= 0 && chunk <= 0 && nc4 >= 32) {
-            tx = 32;
+        // give 14.7 us (0.54 -> 0.64 of the HBM peak; profiles/README.md).
+        int tx = 32, chunk = 0, nthreads = 256;
+        if (nc4 >= 32) {
             const int gx1 = (nc4 + tx - 1) / tx;
             for (nthreads = 1024; nthreads >= 256; nthreads >>= 1) {
                 const int gy1 = num_sms() * (2048 / nthreads) / gx1;
@@ -426,12 +418,10 @@ int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t
                 nthreads = 256;
                 chunk = 0;
             }
-        }
-        if (tx <= 0) {
-            tx = (nc4 >= 512) ? 32 : 16;
+        } else {                             // narrow planes: 256-thread blocks of at most 16 column quads, 32-row chunks
+            tx = 16;
             while (tx > nc4 && tx > 1) tx >>= 1;
         }
-        if (tx > 256) tx = 256;
         const dim3 block(tx, nthreads / tx);
         if (chunk <= 0) chunk = 32;
         if (chunk < (int)block.y) chunk = block.y;

@@ -30,7 +30,7 @@
 
 namespace mvb {
 
-constexpr int ST_NT_MAX = 1024;        // threads per CTA (template parameter NT: 1024 / 768 / 544); the last warp issues the MMAs
+constexpr int ST_NT_MAX = 1024;        // threads per CTA (template parameter NT; 768 / 544 measured slower); the last warp issues the MMAs
 constexpr int ST_NS = 4;               // stages of the operand ring (one 128-pair tile each: 8 KB hi + 8 KB lo)
 constexpr int ST_STAGE = 16384;
 constexpr int ST_ECAP = 4096;          // staged operator entries per CTA
@@ -404,12 +404,10 @@ static int g_stream_tc = 0;            // opt-in (mvb_tune stream_tc=1): at 64 m
                                        // kernels it replaces (fwd 103 vs 108 us, bwd 122 vs 122 us in the captured step) but holds every SM, so
                                        // the deferred weight-gradient chains no longer overlap it: 944 vs 911 us per step (profiles/README.md)
 static int g_stream_sw = 16;           // meshes per slab (mvb_tune stream_tc=enable,sw; 0: the decomposition with the least work per CTA)
-static int g_stream_nt = 1024;         // threads per CTA (mvb_tune stream_nt=1024 / 768 / 544)
 void set_stream_tc(int v, int sw) {
     g_stream_tc = v ? 1 : 0;
     if (sw == 0 || sw == 8 || sw == 16) g_stream_sw = sw;
 }
-void set_stream_nt(int v) { g_stream_nt = v; }
 
 static size_t al256s(size_t v) { return (v + 255) / 256 * 256; }
 
@@ -479,7 +477,7 @@ size_t stream_tc_bwd_workspace_bytes(int N, int B, int K, int has_up) {
 }
 
 template <bool BWD, int NT, int SW>
-static int launch_stream_nt(const StreamArgs &a, const StreamPlan &pl, cudaStream_t st) {
+static int launch_stream_kernel(const StreamArgs &a, const StreamPlan &pl, cudaStream_t st) {
     static DevFlags optin;
     int rc = smem_optin(cheb_stream_tc_kernel<BWD, NT, SW>, 227 * 1024, optin, "cheb_stream_tc");
     if (rc) return rc;
@@ -494,8 +492,8 @@ static int launch_stream_t(const StreamArgs &a, const StreamPlan &pl, cudaStream
         cudaGetLastError();
         return set_err(MVB_ECUDA, "cheb_stream_tc: memset: %s", cudaGetErrorString(e));
     }
-    if (pl.SW == 16) return g_stream_nt == 768 ? launch_stream_nt<BWD, 768, 16>(a, pl, st) : launch_stream_nt<BWD, 1024, 16>(a, pl, st);
-    return g_stream_nt == 768 ? launch_stream_nt<BWD, 768, 8>(a, pl, st) : launch_stream_nt<BWD, 1024, 8>(a, pl, st);
+    if (pl.SW == 16) return launch_stream_kernel<BWD, ST_NT_MAX, 16>(a, pl, st);
+    return launch_stream_kernel<BWD, ST_NT_MAX, 8>(a, pl, st);
 }
 
 // returns 1 = launched, 0 = shape not covered, < 0 = error

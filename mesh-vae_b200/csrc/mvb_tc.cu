@@ -18,23 +18,13 @@
 // Operands are staged global -> registers -> shared directly into the canonical SWIZZLE_64B / SWIZZLE_128B layouts the UMMA
 // shared-memory descriptors expect: a tile row is 64 B (Fin = 16) or 128 B (Fin = 32) and its
 // 16-byte chunk index is XORed with address bits [7,9) / [7,10), which also makes the staging
-// stores bank-conflict free.  A TMA-fed variant of the row GEMM exists (tc_rowgemm_tma_kernel below: the raw fp32 tile
-// loaded by cp.async.bulk.tensor IS the hi operand, only lo is computed) - measured slower than the register path
-// (it needs a block barrier per plane instead of per plane pair), opt-in.
-#include <stdlib.h>
-#include <cuda.h>
+// stores bank-conflict free.
 #include "mvb_internal.cuh"
 #include "mvb_tcgen05.cuh"
 
 namespace mvb {
 
 static int g_tc_enabled = 1;
-static int g_tc_pg6 = 2;           // planes staged at a time by the 6-plane forward contraction (tuning: 1, 2, 3, 6)
-void set_tc_pg6(int v) { if (v == 1 || v == 2 || v == 3 || v == 6) g_tc_pg6 = v; }
-static int g_tc_cap = 4;           // resident CTAs per SM the row-GEMM grid is sized for (tuning: 1..4)
-void set_tc_cap(int v) { if (v >= 1 && v <= 4) g_tc_cap = v; }
-static int g_tc_balance = 0;       // row-GEMM grid = tiles / rounds instead of all block slots (tuning)
-void set_tc_balance(int v) { g_tc_balance = v ? 1 : 0; }
 void set_tc_enabled(int v) { g_tc_enabled = v; }
 int tc_enabled() { return g_tc_enabled; }
 
@@ -54,8 +44,8 @@ struct TcRowArgs {
     float *out;
     int tmem_cols;
     int tile_w;                   // floats per staged tile row (16 or 32)
-    int tile_planes;              // number of staged tiles (= in_planes when planar, 1 when packed)
-    const int32_t *row_sel;       // optional input-row selection (ContractArgs), planar layouts only
+    int tile_planes;              // number of staged tiles (= in_planes, 1 for 4-wide planes)
+    const int32_t *row_sel;       // optional input-row selection (ContractArgs)
     int sel_group;
     int64_t plane_rows;           // rows of one input plane (== rows without a selection)
 };
@@ -67,7 +57,7 @@ __device__ __forceinline__ int64_t sel_row(const int32_t *row_sel, int group, in
 }
 
 // B operand: Bt[n][kd] (n = output column, kd = logical K index p*in_w + i), K-major, swizzled like A,
-// hi/lo split.  kd maps to (tile plane, column) = (kd / tile_w, kd % tile_w) - for the packed layout
+// hi/lo split.  kd maps to (tile plane, column) = (kd / tile_w, kd % tile_w) - for 4-wide planes
 // there is a single tile plane.  Loads are issued four at a time (the weights are L2/L1 resident).
 __device__ __forceinline__ void stage_b_operand(const TcRowArgs &a, char *Bhi, char *Blo, int b_plane, int row_bytes,
                                                 int tid, int nthreads) {
@@ -172,24 +162,21 @@ __device__ __forceinline__ void row_epilogue(const TcRowArgs &a, uint32_t tmem_b
 //              the forward contraction staged at once only ONE 128-thread CTA fitted per SM and the
 //              kernel ran at 2.7 TB/s (profiles/README.md).
 // W = 4      : all NP planes share one tile row (PG = NP).
-// W = 0      : packed layout for narrow planes (Fin = 3, Fout = 3 ...): the K*Fin <= 32 logical
-//              columns of a row are packed into one tile row, staged with scalar accesses.
 template <int W, int NP, int PG>
 __global__ void __launch_bounds__(128)
 tc_rowgemm_kernel(TcRowArgs a) {
     extern __shared__ __align__(1024) char smem_raw[];
     char *smem = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    constexpr bool PACKED = (W == 0);
     constexpr bool ONE_TILE = (W == 4);              // 4-wide planes: all NP planes share one tile row
-    constexpr int Q4 = PACKED ? 1 : W / 4;
-    constexpr int NPR = PACKED ? 1 : PG;             // planes prefetched into registers (one group)
-    constexpr int NPL = (PACKED || ONE_TILE) ? 1 : PG;   // staged A tiles
-    constexpr int NPB = (PACKED || ONE_TILE) ? 1 : NP;   // staged B tiles (all planes, once)
-    constexpr int NG = (PACKED || ONE_TILE) ? 1 : NP / PG;
-    static_assert(PACKED || ONE_TILE || NP % PG == 0, "plane groups must divide the plane count");
+    constexpr int Q4 = W / 4;
+    constexpr int NPR = PG;                          // planes prefetched into registers (one group)
+    constexpr int NPL = ONE_TILE ? 1 : PG;           // staged A tiles
+    constexpr int NPB = ONE_TILE ? 1 : NP;           // staged B tiles (all planes, once)
+    constexpr int NG = ONE_TILE ? 1 : NP / PG;
+    static_assert(ONE_TILE || NP % PG == 0, "plane groups must divide the plane count");
     constexpr int NV = NPR * Q4;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int wt = (PACKED || ONE_TILE) ? a.tile_w : W;
+    const int wt = ONE_TILE ? a.tile_w : W;
     const int row_bytes = wt * 4;
     const int R = 128;
     const int a_plane = R * row_bytes;
@@ -207,7 +194,7 @@ tc_rowgemm_kernel(TcRowArgs a) {
         mbar_init(bar, 1);
         fence_barrier_init();
     }
-    if (PACKED || ONE_TILE) {   // padding columns of the packed tiles must be finite zeros in A and B
+    if (ONE_TILE) {             // padding columns of the shared tile row must be finite zeros in A and B
         for (int i = tid; i < (2 * a_plane + 2 * b_plane) / 16; i += blockDim.x)
             reinterpret_cast<float4 *>(Ahi)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         __syncthreads();
@@ -221,7 +208,7 @@ tc_rowgemm_kernel(TcRowArgs a) {
     const uint32_t idesc = make_idesc(128, a.nn16, 0, 0);
     const uint32_t layout_type = (row_bytes == 128) ? 2u : 4u;
     const uint32_t sbo = 8u * row_bytes;
-    const int kslices = (PACKED || ONE_TILE) ? (a.in_planes * a.in_w + 7) / 8 : W / 8;
+    const int kslices = ONE_TILE ? (a.in_planes * a.in_w + 7) / 8 : W / 8;
     const int row = warp * 32 + lane;                 // D row (TMEM lane) this thread reads back
     uint32_t phase = 0;
     const int64_t ntiles = (a.rows + R - 1) / R;
@@ -229,20 +216,20 @@ tc_rowgemm_kernel(TcRowArgs a) {
     float4 pre[NV];
     float4 prem[Q4];
     // tile-invariant part of a thread's pieces (row within the tile, swizzled shared-memory offset): computed once
-    int srow[Q4 > 0 ? Q4 : 1];
-    uint32_t soff[Q4 > 0 ? Q4 : 1];
+    int srow[Q4];
+    uint32_t soff[Q4];
 #pragma unroll
     for (int j = 0; j < Q4; ++j) {
         const int i = j * 128 + tid;
-        srow[j] = i / (Q4 > 0 ? Q4 : 1);
+        srow[j] = i / Q4;
         soff[j] = swz_off(srow[j], i - srow[j] * Q4, row_bytes);
     }
-    // global -> registers for plane group g of the tile starting at row0 (planar layout)
+    // global -> registers for plane group g of the tile starting at row0
     auto prefetch = [&](int64_t row0, int g) {
         const int nr = (int)((a.rows - row0) < R ? (a.rows - row0) : R);
 #pragma unroll
         if (a.row_sel) {          // selected rows: the pieces of a tile row stay contiguous, the rows are gathered
-            int64_t src[Q4 > 0 ? Q4 : 1];
+            int64_t src[Q4];
 #pragma unroll
             for (int j = 0; j < Q4; ++j) src[j] = (srow[j] < nr) ? sel_row(a.row_sel, a.sel_group, row0 + srow[j]) : 0;
 #pragma unroll
@@ -296,54 +283,14 @@ tc_rowgemm_kernel(TcRowArgs a) {
             }
         }
     };
-    // packed layout: scalar staging straight to shared memory; the (plane, row, feature) index space
-    // of the tile is flattened so that every thread has 8 independent coalesced loads in flight
-    auto stage_packed = [&](int64_t row0, int nr) {
-        const int per_plane = R * a.in_w;
-        const int total = a.in_planes * per_plane;
-        for (int base = 0; base < total; base += 8 * 128) {
-            float v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int i = base + u * 128 + tid;
-                v[u] = 0.f;
-                if (i < total) {
-                    const int p = i / per_plane, e = i - p * per_plane;
-                    if (e < nr * a.in_w) {
-                        const float *src = (p == 0 ? a.in0 : a.in_rest + (int64_t)(p - 1) * a.rows * a.in_w) + row0 * a.in_w;
-                        v[u] = __ldg(src + e);
-                        if (p == 0 && a.mask) v[u] = __ldg(a.mask + row0 * a.in_w + e) > 0.f ? v[u] : 0.f;
-                    }
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int i = base + u * 128 + tid;
-                if (i < total) {
-                    const int p = i / per_plane, e = i - p * per_plane;
-                    const int r = e / a.in_w, f = e - r * a.in_w;
-                    float h, l;
-                    split_tf32(v[u], h, l);
-                    const int col = p * a.in_w + f;
-                    const uint32_t off = swz_off(r, col >> 2, row_bytes) + (uint32_t)((col & 3) << 2);
-                    *reinterpret_cast<float *>(Ahi + off) = h;
-                    *reinterpret_cast<float *>(Alo + off) = l;
-                }
-            }
-        }
-    };
-
     int64_t t = blockIdx.x;
-    if (!PACKED && t < ntiles) prefetch(t * R, 0);
+    if (t < ntiles) prefetch(t * R, 0);
     for (; t < ntiles; t += gridDim.x) {
         const int64_t row0 = t * R;
         const int nr = (int)((a.rows - row0) < R ? (a.rows - row0) : R);
 #pragma unroll
         for (int g = 0; g < NG; ++g) {
-            if (PACKED)
-                stage_packed(row0, nr);
-            else
-                commit(g);
+            commit(g);
             fence_proxy_async();
             tc_fence_before();
             __syncthreads();
@@ -354,10 +301,8 @@ tc_rowgemm_kernel(TcRowArgs a) {
                 umma_commit(bar);
             }
             // the next group's rows are in flight during the MMAs (and, for the last group, the epilogue)
-            if (!PACKED) {
-                if (g + 1 < NG) prefetch(row0, g + 1);
-                else if (t + gridDim.x < ntiles) prefetch((t + gridDim.x) * R, 0);
-            }
+            if (g + 1 < NG) prefetch(row0, g + 1);
+            else if (t + gridDim.x < ntiles) prefetch((t + gridDim.x) * R, 0);
             mbar_wait(bar, phase);
             phase ^= 1;
             tc_fence_after();
@@ -367,194 +312,6 @@ tc_rowgemm_kernel(TcRowArgs a) {
     }
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)a.tmem_cols);
-}
-
-// ---------------------------------------------------------------------------------------------
-// Row GEMM with TMA-fed operands (16-wide planes, no mask / row selection): kind::tf32 reads only the upper 19 bits of an
-// operand, so the RAW fp32 tile is the `hi` operand as it stands - cp.async.bulk.tensor writes it straight into the K-major
-// SWIZZLE_64B UMMA layout (the TMA swizzle mode and the descriptor's swizzle mode are the same XOR), no register pass; only
-// lo = x - trunc(x) is computed, shared memory to shared memory.  One plane (128 rows x 64 bytes = 8 KB) per iteration:
-//   ring of NB hi tiles filled by TMA NB-1 iterations ahead (mbarrier complete_tx), two lo tiles; per iteration
-//   wait(full) -> convert -> barrier -> one thread issues the 6 MMAs of the plane and commits to the lo tile's mbarrier ->
-//   the tile freed by the PREVIOUS iteration's MMAs is refilled; the accumulator stays in TMEM across the planes of a row tile.
-// ---------------------------------------------------------------------------------------------
-struct TcTmaMaps {
-    CUtensorMap m0;       // plane 0: [rows][16]
-    CUtensorMap m1;       // planes 1..NP-1, contiguous: [(NP-1) * rows][16]
-};
-
-__device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap *map, int c0, int c1, uint64_t *bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(smem_dst),
-                 "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-
-template <int NB>
-__global__ void __launch_bounds__(128)
-tc_rowgemm_tma_kernel(TcRowArgs a, const __grid_constant__ TcTmaMaps maps) {
-    extern __shared__ __align__(1024) char smem_raw[];
-    char *smem = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int NP = a.in_planes;
-    constexpr int R = 128, A_TILE = R * 64;
-    const int b_plane = a.nn16 * 64;
-    char *Ahi = smem;                                   // [NB][8 KB]
-    char *Alo = Ahi + NB * A_TILE;                      // [2][8 KB]
-    char *Bhi = Alo + 2 * A_TILE;                       // [NP][b_plane]
-    char *Blo = Bhi + NP * b_plane;
-    uint64_t *full = reinterpret_cast<uint64_t *>(Blo + NP * b_plane);      // [NB]
-    uint64_t *mbar = full + NB;                                            // [2]: MMAs that read lo tile b (and their hi tile) are done
-    uint32_t *slot = reinterpret_cast<uint32_t *>(mbar + 2);
-
-    pdl_trigger();
-    if (warp == 0) tmem_alloc(slot, (uint32_t)a.tmem_cols);
-    if (tid == 0) {
-        for (int i = 0; i < NB; ++i) mbar_init(full + i, 1);
-        mbar_init(mbar, 1);
-        mbar_init(mbar + 1, 1);
-        fence_barrier_init();
-    }
-    stage_b_operand(a, Bhi, Blo, b_plane, 64, tid, blockDim.x);          // weights: no kernel of the step writes them
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    pdl_wait();          // the planes are the previous kernels' output
-    const uint32_t tmem_base = *slot;
-    const uint32_t idesc = make_idesc(128, a.nn16, 0, 0);
-    const int64_t ntiles = (a.rows + R - 1) / R;
-    const int64_t my_tiles = ((int64_t)blockIdx.x < ntiles) ? (ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-    const int64_t n_iters = my_tiles * NP;
-    const int row = warp * 32 + lane;                   // D row (TMEM lane) this thread reads back
-
-    // iteration it = (tile it / NP of this CTA, plane it % NP)
-    auto issue_load = [&](int64_t it) {
-        const int p = (int)(it % NP);
-        const int64_t row0 = ((int64_t)blockIdx.x + (it / NP) * gridDim.x) * R;
-        uint64_t *fb = full + (it % NB);
-        mbar_expect_tx(fb, (uint32_t)A_TILE);
-        if (p == 0) tma_load_2d(smem_u32(Ahi + (it % NB) * A_TILE), &maps.m0, 0, (int)row0, fb);
-        else tma_load_2d(smem_u32(Ahi + (it % NB) * A_TILE), &maps.m1, 0, (int)((int64_t)(p - 1) * a.rows + row0), fb);
-    };
-    if (tid == 0)
-        for (int64_t it = 0; it < NB - 1 && it < n_iters; ++it) issue_load(it);
-
-    // this thread's four pieces of a tile (row, 16-byte chunk): swizzled offsets, tile-invariant
-    uint32_t soff[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int i = j * 128 + tid;
-        soff[j] = swz_off(i >> 2, i & 3, 64);
-    }
-    for (int64_t it = 0; it < n_iters; ++it) {
-        const int p = (int)(it % NP), lb = (int)(it & 1), hb = (int)(it % NB);
-        if (it >= 2) mbar_wait(mbar + lb, (uint32_t)(((it - 2) >> 1) & 1));        // the MMAs of iteration it - 2 have read lo tile lb
-        mbar_wait(full + hb, (uint32_t)((it / NB) & 1));                           // the raw tile has landed
-        const char *hi = Ahi + hb * A_TILE;
-        char *lo = Alo + lb * A_TILE;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const float4 v = *reinterpret_cast<const float4 *>(hi + soff[j]);
-            float4 h, l;
-            split4(v, h, l);
-            *reinterpret_cast<float4 *>(lo + soff[j]) = l;
-        }
-        fence_proxy_async();
-        tc_fence_before();
-        __syncthreads();
-        if (tid == 0) {
-            tc_fence_after();
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                const uint64_t ah = make_desc(smem_u32(hi) + j * 32, 16, 512, 4u), al = make_desc(smem_u32(lo) + j * 32, 16, 512, 4u);
-                const uint64_t bh = make_desc(smem_u32(Bhi + p * b_plane) + j * 32, 16, 512, 4u);
-                const uint64_t bl = make_desc(smem_u32(Blo + p * b_plane) + j * 32, 16, 512, 4u);
-                umma_tf32(tmem_base, al, bh, idesc, (p > 0 || j > 0) ? 1u : 0u);      // small terms first
-                umma_tf32(tmem_base, ah, bl, idesc, 1u);
-                umma_tf32(tmem_base, ah, bh, idesc, 1u);
-            }
-            umma_commit(mbar + lb);
-            // refill the hi tile that the PREVIOUS iteration's MMAs have finished with (iteration it + NB - 1)
-            const int64_t nx = it + NB - 1;
-            if (nx < n_iters) {
-                if (it >= 1) mbar_wait(mbar + (lb ^ 1), (uint32_t)(((it - 1) >> 1) & 1));
-                issue_load(nx);
-            }
-        }
-        if (p == NP - 1) {       // the row tile is complete: every MMA issued so far is covered by this commit
-            mbar_wait(mbar + lb, (uint32_t)((it >> 1) & 1));
-            tc_fence_after();
-            const int64_t row0 = ((int64_t)blockIdx.x + (it / NP) * gridDim.x) * R;
-            const int nr = (int)((a.rows - row0) < R ? (a.rows - row0) : R);
-            row_epilogue(a, tmem_base, warp, row, nr, row0);
-            tc_fence_before();   // order this tile's TMEM reads before the barrier that precedes the next MMA
-        }
-    }
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)a.tmem_cols);
-}
-
-static int g_tc_tma = 0;            // mvb_tune tc_tma=0/1[,hi tiles in the ring: 3 or 4].  Off by default: same-box A/B of the step (bench.py,
-                                    // two passes): register-staged kernel 0.8920 / 0.8918 ms, TMA-fed 0.9049 / 0.9054 ms (ring of 3, four CTAs per SM),
-                                    // 0.9066 / 0.9068 ms (ring of 4, three CTAs per SM); results identical (same products, same order)
-static int g_tc_tma_nb = 4;
-void set_tc_tma(int v, int nb) {
-    g_tc_tma = v ? 1 : 0;
-    if (nb == 3 || nb == 4) g_tc_tma_nb = nb;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-    static EncodeTiledFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-        else
-            cudaGetLastError();
-    }
-    return fn;
-}
-static bool make_plane_map(CUtensorMap *m, const float *base, int64_t nrows) {
-    EncodeTiledFn fn = encode_tiled_fn();
-    if (!fn) return false;
-    const cuuint64_t gdim[2] = {16, (cuuint64_t)nrows};
-    const cuuint64_t gstride[1] = {64};
-    const cuuint32_t box[2] = {16, 128};
-    const cuuint32_t estride[2] = {1, 1};
-    return fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float *>(base), gdim, gstride, box, estride, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// 1 = launched, 0 = not covered
-static int launch_rowgemm_tma(const TcRowArgs &t, cudaStream_t st) {
-    if (!g_tc_tma || t.in_w != 16 || t.in_planes < 2 || t.in_planes > 8 || t.mask || t.row_sel || t.w_fold > 1) return 0;
-    if (t.rows < 128 * 64 || (int64_t)t.in_planes * t.rows >= ((int64_t)1 << 31)) return 0;
-    TcTmaMaps maps;
-    if (!make_plane_map(&maps.m0, t.in0, t.rows) || !make_plane_map(&maps.m1, t.in_rest, (int64_t)(t.in_planes - 1) * t.rows)) return 0;
-    const int NB = g_tc_tma_nb;
-    const size_t smem = 1024 + (size_t)(NB + 2) * 8192 + 2 * (size_t)t.in_planes * t.nn16 * 64 + (NB + 2) * 8 + 16;
-    static DevFlags optin3, optin4;
-    if (NB == 3 ? smem_optin(tc_rowgemm_tma_kernel<3>, 200 * 1024, optin3, "tc_rowgemm_tma") : smem_optin(tc_rowgemm_tma_kernel<4>, 200 * 1024, optin4, "tc_rowgemm_tma")) return 0;
-    int per_sm = (int)((220 * 1024) / smem);
-    if (per_sm > 512 / t.tmem_cols) per_sm = 512 / t.tmem_cols;
-    if (per_sm > 6) per_sm = 6;
-    if (per_sm < 1) per_sm = 1;
-    const int64_t ntiles = (t.rows + 127) / 128;
-    int64_t grid = (int64_t)num_sms() * per_sm;
-    if (grid > ntiles) grid = ntiles;
-    if (NB == 3) launch_pdl(tc_rowgemm_tma_kernel<3>, dim3((unsigned)grid), dim3(128), smem, st, t, maps);
-    else launch_pdl(tc_rowgemm_tma_kernel<4>, dim3((unsigned)grid), dim3(128), smem, st, t, maps);
-    const int rc = check_launch("mvb tc_rowgemm_tma");
-    return rc ? rc : 1;
 }
 
 static int pow2_cols(int n) {
@@ -585,14 +342,8 @@ int launch_contract_tc(const ContractArgs &a, cudaStream_t st) {
     if (nn16 > 256 || a.rows < 128) return 0;
     const bool planar = (w == 16 && a.in_planes <= 6) || (w == 32 && a.in_planes <= 3) || (w == 4 && a.in_planes <= 8);
     const bool vec_ok = aligned16(a.in0) && (a.in_planes == 1 || aligned16(a.in_rest)) && (!a.mask || aligned16(a.mask));
-    // the scalar-staged packed layout (narrow planes, Fin = 3 / Fout = 3) is functional but its index
-    // arithmetic makes it slower than the FFMA kernel: opt-in only (MVB_TC_PACKED=1) until those layers
-    // are padded to 4-wide planes
-    static const bool allow_packed = getenv("MVB_TC_PACKED") != nullptr;
-    const bool packed = allow_packed && !(planar && vec_ok) && Kd <= 32;
-    if (!(planar && vec_ok) && !packed) return 0;
-    if (!aligned16(a.out)) return 0;
-    if (a.row_sel && (packed || a.mask || a.sel_group < 1)) return 0;
+    if (!(planar && vec_ok) || !aligned16(a.out)) return 0;
+    if (a.row_sel && (a.mask || a.sel_group < 1)) return 0;
     TcRowArgs t;
     t.row_sel = a.row_sel;
     t.sel_group = a.sel_group;
@@ -613,16 +364,11 @@ int launch_contract_tc(const ContractArgs &a, cudaStream_t st) {
     t.out_w = a.out_w;
     t.out = a.out;
     t.tmem_cols = pow2_cols(nn16);
-    t.tile_w = (packed || w == 4) ? (Kd <= 16 ? 16 : 32) : w;
-    t.tile_planes = (packed || w == 4) ? 1 : a.in_planes;
-    if (!packed && w == 16) {          // TMA-fed variant (mvb_tune tc_tma=1)
-        const int rt = launch_rowgemm_tma(t, st);
-        if (rt != 0) return rt;
-    }
-    // plane groups (A tiles staged at a time): 3 of 6 / 2 of 4 planes for 16-wide planes, 1 of 2-3 for 32-wide
+    t.tile_w = (w == 4) ? (Kd <= 16 ? 16 : 32) : w;
+    t.tile_planes = (w == 4) ? 1 : a.in_planes;
+    // plane groups (A tiles staged at a time): 2 of 4-6 planes for 16-wide planes, 1 of 2-3 for 32-wide
     int pg = t.tile_planes;
-    if (w == 16 && a.in_planes == 6) pg = g_tc_pg6;
-    else if (w == 16 && a.in_planes == 4) pg = 2;
+    if (w == 16 && (a.in_planes == 4 || a.in_planes == 6)) pg = 2;
     else if (w == 32 && a.in_planes >= 2) pg = 1;
     const size_t smem = 1024 + (size_t)pg * (2 * 128 * t.tile_w * 4) + (size_t)t.tile_planes * (2 * nn16 * t.tile_w * 4) + 64;
     if (smem > 200 * 1024) return 0;
@@ -630,18 +376,12 @@ int launch_contract_tc(const ContractArgs &a, cudaStream_t st) {
     // CTAs per SM: shared memory and TMEM (512 columns) permitting
     int per_sm = (int)((220 * 1024) / smem);
     if (per_sm > 512 / t.tmem_cols) per_sm = 512 / t.tmem_cols;
-    if (per_sm > g_tc_cap) per_sm = g_tc_cap;
+    if (per_sm > 4) per_sm = 4;
     if (per_sm < 1) per_sm = 1;
     int64_t grid = (int64_t)num_sms() * per_sm;
     if (grid > ntiles) grid = ntiles;
-    if (g_tc_balance && grid > 0) {          // every block the same number of tiles
-        const int64_t rounds = (ntiles + grid - 1) / grid;
-        grid = (ntiles + rounds - 1) / rounds;
-    }
     int rc;
-    if (packed) {
-        rc = launch_rowgemm_t<0, 1>(t, (unsigned)grid, smem, st);
-    } else if (w == 4) {
+    if (w == 4) {
         switch (a.in_planes) {
             case 1: rc = launch_rowgemm_t<4, 1>(t, (unsigned)grid, smem, st); break;
             case 2: rc = launch_rowgemm_t<4, 2>(t, (unsigned)grid, smem, st); break;
@@ -659,12 +399,7 @@ int launch_contract_tc(const ContractArgs &a, cudaStream_t st) {
             case 3: rc = launch_rowgemm_t<16, 3>(t, (unsigned)grid, smem, st); break;
             case 4: rc = launch_rowgemm_t<16, 4, 2>(t, (unsigned)grid, smem, st); break;
             case 5: rc = launch_rowgemm_t<16, 5>(t, (unsigned)grid, smem, st); break;
-            default:
-                if (pg == 6) rc = launch_rowgemm_t<16, 6, 6>(t, (unsigned)grid, smem, st);
-                else if (pg == 2) rc = launch_rowgemm_t<16, 6, 2>(t, (unsigned)grid, smem, st);
-                else if (pg == 1) rc = launch_rowgemm_t<16, 6, 1>(t, (unsigned)grid, smem, st);
-                else rc = launch_rowgemm_t<16, 6, 3>(t, (unsigned)grid, smem, st);
-                break;
+            default: rc = launch_rowgemm_t<16, 6, 2>(t, (unsigned)grid, smem, st); break;
         }
     } else {
         switch (a.in_planes) {
@@ -700,7 +435,6 @@ struct TcWgradArgs {
     const int32_t *row_sel;        // optional selection of the T rows (WgradArgs); dy / mask are dense over the selected rows
     int sel_group;
     int64_t plane_rows;
-    int perm;                      // conflict-free lane order for the 16-wide staging stores (mvb_tune wgrad_perm)
 };
 
 // byte offset of logical (row r, feature column col) in a BASE32B tile made of 32-column blocks of blk bytes
@@ -709,8 +443,7 @@ __device__ __forceinline__ uint32_t b32_off(int r, int col, int blk) {
     return (uint32_t)(b * blk + r * 128 + (((c >> 1) ^ (r & 3)) << 5) + ((c & 1) << 4) + ((col & 3) << 2));
 }
 
-// NPF > 0: planes of width 4*Q4 floats (4, 16 or 32), Fout % 4 == 0: vector staging with register prefetch;
-// NPF == 0: generic scalar staging
+// NPF planes of width 4*Q4 floats (4, 16 or 32), Fout % 4 == 0: vector staging with register prefetch
 constexpr int WG_NT = 256;      // 8 warps: all of them stage tiles, warps 0-3 own the TMEM lanes of the epilogue (ncu: the
                                 // 128-thread version was paced by its own instruction stream at 8 warps per SM)
 template <int NPF, int Q4>
@@ -718,9 +451,7 @@ __global__ void __launch_bounds__(WG_NT)
 tc_wgrad_kernel(TcWgradArgs a) {
     extern __shared__ __align__(1024) char smem_raw[];
     char *smem = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    constexpr bool FAST = NPF > 0;
-    constexpr int NPV = FAST ? NPF : 1;
-    constexpr int W = 4 * Q4;                          // plane width (FAST only)
+    constexpr int W = 4 * Q4;                          // plane width
     constexpr int LPT = (64 * Q4 + WG_NT - 1) / WG_NT; // float4 loads per thread per plane per 64-row tile
     constexpr int DJ = 512 / WG_NT;                    // dY pieces per thread (up to 64 rows x 8 quads)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -756,46 +487,42 @@ tc_wgrad_kernel(TcWgradArgs a) {
     // N = 32 yields A.[B_hi | B_lo]; two MMAs per K step (A_hi, A_lo) instead of three give all four hi/lo products, the
     // epilogue adds the two column halves.  These MMAs cost the same whatever N is (the M = 128 operand is streamed from
     // shared memory per instruction), and their count paces the kernel.
-    const bool nstack = FAST && a.n16 == 16;
+    const bool nstack = a.n16 == 16;
     const uint32_t idesc = make_idesc(128, nstack ? 32 : a.n16, 1, 1);
     const int64_t ntiles = (a.rows + R - 1) / R;
-    const int dq4 = a.n_out >> 2;                      // float4 chunks per dY row (FAST only)
+    const int dq4 = a.n_out >> 2;                      // float4 chunks per dY row
 
     // register prefetch DEPTH tiles ahead.  Depth 3 for the narrow planes (10 KB per tile) measured no faster than depth 1
     // (43.3 vs 42.7 us): the kernel is paced by the MMA instruction stream, not by memory latency - see N-stacking below
     constexpr int DEPTH = 1;
-    float4 pre[DEPTH][LPT * NPV];
+    float4 pre[DEPTH][LPT * NPF];
     float4 pred[DEPTH][DJ], prem[DEPTH][DJ];
     // everything about a thread's pieces of a tile that does not depend on the tile - row, shared-memory offsets,
     // validity - is computed once: the per-tile code is then loads, the hi/lo split and stores (ncu: 11.2 M warp
     // instructions for 4998 narrow tiles before, two integer divisions and a swizzle computation per piece per tile)
-    // 16-wide planes (4 quads per row): a warp's 32 pieces are 8 rows x 4 quads.  In row-major lane order the 8 lanes
+    // 16-wide planes (4 quads per row): a warp's 32 pieces are 8 rows x 4 quads.  In this row-major lane order the 8 lanes
     // of a quarter warp (2 rows x 4 quads) hit only TWO of the four 32-byte units of the BASE32B swizzle - every 16-byte
-    // store is a 2-way bank conflict (ncu r02b: 47 % of the shared wavefronts of tc_wgrad<6,4>).  With a.perm the lane order
-    // (quad & 1, row & 3, quad >> 1, row >> 2) gives each quarter warp 4 rows x one 32-byte unit: all four units, no conflict;
-    // the global loads of the warp still cover the same contiguous 512 bytes.
-    auto perm16 = [](int i) {
-        const int l = i & 31;
-        return (i & ~31) | ((((l >> 4) & 1) * 4 + ((l >> 1) & 3)) << 2) | (((l >> 3) & 1) * 2 + (l & 1));
-    };
+    // store is a 2-way bank conflict (ncu r02b: 47 % of the shared wavefronts of tc_wgrad<6,4>).  A conflict-free lane
+    // order measured no faster (bench.py, 0.9209 / 0.9389 against 0.9181 / 0.9182 ms per step): the stores do not pace
+    // the kernel.
     int trow[LPT];                       // row of T piece j within the tile, -1 = no piece
     int tidx[LPT];                       // its quad index inside the tile (row * Q4 + quad)
-    uint32_t toff[NPV][LPT];
+    uint32_t toff[NPF][LPT];
 #pragma unroll
     for (int j = 0; j < LPT; ++j) {
-        const int i = (Q4 == 4 && a.perm) ? perm16(j * WG_NT + tid) : j * WG_NT + tid;
+        const int i = j * WG_NT + tid;
         tidx[j] = i;
-        trow[j] = (FAST && i < 64 * Q4) ? i / Q4 : -1;
+        trow[j] = (i < 64 * Q4) ? i / Q4 : -1;
 #pragma unroll
-        for (int p = 0; p < NPV; ++p) toff[p][j] = trow[j] >= 0 ? b32_off(trow[j], p * W + (i - trow[j] * Q4) * 4, blk) : 0u;
+        for (int p = 0; p < NPF; ++p) toff[p][j] = trow[j] >= 0 ? b32_off(trow[j], p * W + (i - trow[j] * Q4) * 4, blk) : 0u;
     }
     int drow[DJ], didx[DJ];
     uint32_t doff[DJ], doff_lo[DJ];
 #pragma unroll
     for (int j = 0; j < DJ; ++j) {
-        const int i = (dq4 == 4 && a.perm) ? perm16(j * WG_NT + tid) : j * WG_NT + tid;
+        const int i = j * WG_NT + tid;
         didx[j] = i;
-        drow[j] = (FAST && i < R * dq4) ? i / dq4 : -1;
+        drow[j] = (i < R * dq4) ? i / dq4 : -1;
         const int q = drow[j] >= 0 ? i - drow[j] * dq4 : 0;
         doff[j] = drow[j] >= 0 ? b32_off(drow[j], q * 4, blk) : 0u;
         doff_lo[j] = drow[j] >= 0 ? b32_off(drow[j], 16 + q * 4, blk) : 0u;       // N-stacked position of the lo part
@@ -807,7 +534,7 @@ tc_wgrad_kernel(TcWgradArgs a) {
 #pragma unroll
             for (int j = 0; j < LPT; ++j) src[j] = (trow[j] >= 0 && trow[j] < nr) ? sel_row(a.row_sel, a.sel_group, row0 + trow[j]) : 0;
 #pragma unroll
-            for (int p = 0; p < NPV; ++p) {
+            for (int p = 0; p < NPF; ++p) {
                 const float4 *b4 = reinterpret_cast<const float4 *>(p == 0 ? a.in0 : a.in_rest + (int64_t)(p - 1) * a.plane_rows * W);
 #pragma unroll
                 for (int j = 0; j < LPT; ++j) {
@@ -817,7 +544,7 @@ tc_wgrad_kernel(TcWgradArgs a) {
             }
         } else {
 #pragma unroll
-        for (int p = 0; p < NPV; ++p) {
+        for (int p = 0; p < NPF; ++p) {
             const float4 *s4 = reinterpret_cast<const float4 *>((p == 0 ? a.in0 : a.in_rest + (int64_t)(p - 1) * a.rows * W) + row0 * W);
 #pragma unroll
             for (int j = 0; j < LPT; ++j)
@@ -835,7 +562,7 @@ tc_wgrad_kernel(TcWgradArgs a) {
     };
     auto commit = [&](const int d) {
 #pragma unroll
-        for (int p = 0; p < NPV; ++p) {
+        for (int p = 0; p < NPF; ++p) {
 #pragma unroll
             for (int j = 0; j < LPT; ++j) {
                 if (trow[j] >= 0) {
@@ -866,74 +593,21 @@ tc_wgrad_kernel(TcWgradArgs a) {
             }
         }
     };
-    // generic staging (narrow planes such as Fin = 3, or Fout = 3): flattened index space, 8 independent
-    // coalesced scalar loads in flight per thread
-    auto stage_generic = [&](int64_t row0, int nr) {
-        const int per_plane = R * a.in_w;
-        const int t_total = a.in_planes * per_plane;
-        const int total = t_total + R * a.n_out;          // T planes, then the dY tile
-        for (int base = 0; base < total; base += 8 * WG_NT) {
-            float v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int i = base + u * WG_NT + tid;
-                v[u] = 0.f;
-                if (i < t_total) {
-                    const int p = i / per_plane, e = i - p * per_plane;
-                    if (e < nr * a.in_w)
-                        v[u] = __ldg((p == 0 ? a.in0 : a.in_rest + (int64_t)(p - 1) * a.rows * a.in_w) + row0 * a.in_w + e);
-                } else if (i < total) {
-                    const int e = i - t_total;
-                    if (e < nr * a.n_out) {
-                        v[u] = __ldg(a.dy + row0 * a.n_out + e);
-                        if (a.mask) v[u] = __ldg(a.mask + row0 * a.n_out + e) > 0.f ? v[u] : 0.f;
-                    }
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int i = base + u * WG_NT + tid;
-                float h, l;
-                split_tf32(v[u], h, l);
-                if (i < t_total) {
-                    const int p = i / per_plane, e = i - p * per_plane;
-                    const int r = e / a.in_w, f = e - r * a.in_w;
-                    const uint32_t off = b32_off(r, p * a.in_w + f, blk);
-                    *reinterpret_cast<float *>(Thi + off) = h;
-                    *reinterpret_cast<float *>(Tlo + off) = l;
-                } else if (i < total) {
-                    const int e = i - t_total;
-                    const int r = e / a.n_out, f = e - r * a.n_out;
-                    const uint32_t off = b32_off(r, f, blk);
-                    *reinterpret_cast<float *>(Dhi + off) = h;
-                    *reinterpret_cast<float *>(Dlo + off) = l;
-                }
-            }
-        }
-    };
-
     uint32_t acc = 0, phase = 0;
     bool pending = false;
     int64_t t = blockIdx.x;
-    if (FAST) {
 #pragma unroll
-        for (int d = 0; d < DEPTH; ++d)
-            if (t + (int64_t)d * gridDim.x < ntiles) prefetch(d, (t + (int64_t)d * gridDim.x) * R);
-    }
+    for (int d = 0; d < DEPTH; ++d)
+        if (t + (int64_t)d * gridDim.x < ntiles) prefetch(d, (t + (int64_t)d * gridDim.x) * R);
     while (t < ntiles) {
 #pragma unroll
         for (int d = 0; d < DEPTH; ++d) {          // static register slots: the tile loop is unrolled DEPTH times
             if (t >= ntiles) continue;
-            const int64_t row0 = t * R;
-            const int nr = (int)((a.rows - row0) < R ? (a.rows - row0) : R);
             if (pending) {   // the previous tile's MMAs must have finished reading shared memory
                 mbar_wait(bar, phase);
                 phase ^= 1;
             }
-            if (FAST)
-                commit(d);
-            else
-                stage_generic(row0, nr);
+            commit(d);
             fence_proxy_async();
             tc_fence_before();
             __syncthreads();
@@ -953,7 +627,7 @@ tc_wgrad_kernel(TcWgradArgs a) {
             }
             pending = true;
             const int64_t nx = t + (int64_t)DEPTH * gridDim.x;
-            if (FAST && nx < ntiles) prefetch(d, nx * R);     // overlaps this and the next DEPTH-1 tiles
+            if (nx < ntiles) prefetch(d, nx * R);     // overlaps this and the next DEPTH-1 tiles
             t += gridDim.x;
         }
     }
@@ -996,10 +670,6 @@ static int launch_wgrad_t(const TcWgradArgs &t, unsigned grid, size_t smem, cuda
     return check_launch("mvb tc_wgrad");
 }
 
-static int g_wgrad_perm = 0;        // measured (bench.py, same box, 2 x 300 steps each): 0.9181 / 0.9182 ms per step off, 0.9209 / 0.9389 on - the
-                                    // stores are not what paces the kernel; kept as a tuning hook
-void set_wgrad_perm(int v) { g_wgrad_perm = v ? 1 : 0; }
-
 // returns 1 if taken, 0 if unsupported, < 0 on error.  Partial layout matches the FFMA wgrad kernel.
 int launch_wgrad_tc(const WgradArgs &a, int has_bias, int M4, int N4, int *nparts, cudaStream_t st) {
     if (!g_tc_enabled) return 0;
@@ -1008,9 +678,7 @@ int launch_wgrad_tc(const WgradArgs &a, int has_bias, int M4, int N4, int *npart
     const bool fast = ((a.in_w == 16 && a.in_planes <= 6) || (a.in_w == 4 && a.in_planes <= 8) || (a.in_w == 32 && a.in_planes <= 3)) &&
                       (a.n_out % 4 == 0) && aligned16(a.in0) &&
                       (a.in_planes == 1 || aligned16(a.in_rest)) && aligned16(a.dy) && (!a.mask || aligned16(a.mask));
-    static const bool allow_generic = getenv("MVB_TC_PACKED") != nullptr;
-    if (!fast && !allow_generic) return 0;
-    if (a.row_sel && (!fast || a.sel_group < 1)) return 0;
+    if (!fast || (a.row_sel && a.sel_group < 1)) return 0;
     TcWgradArgs t;
     t.row_sel = a.row_sel;
     t.sel_group = a.sel_group;
@@ -1029,17 +697,13 @@ int launch_wgrad_tc(const WgradArgs &a, int has_bias, int M4, int N4, int *npart
     t.N4 = N4;
     t.partials = a.partials;
     t.tmem_cols = 32;
-    t.perm = g_wgrad_perm;
     const size_t smem = 1024 + 10 * 64 * 128 + 64;
     const int64_t ntiles = (a.rows + 63) / 64;
-    int64_t grid = a.background > 0 ? (int64_t)num_sms() / a.background : (int64_t)num_sms() * 2;
-    if (grid < 1) grid = 1;
+    int64_t grid = (int64_t)num_sms() * 2;
     if (grid > ntiles) grid = ntiles;
     if ((size_t)grid * M4 * N4 * sizeof(float) > a.partial_bytes) return set_err(MVB_EWORKSPACE, "tc_wgrad: workspace too small");
     int rc;
-    if (!fast) {
-        rc = launch_wgrad_t<0, 1>(t, (unsigned)grid, smem, st);
-    } else if (a.in_w == 32) {
+    if (a.in_w == 32) {
         switch (a.in_planes) {
             case 1: rc = launch_wgrad_t<1, 8>(t, (unsigned)grid, smem, st); break;
             case 2: rc = launch_wgrad_t<2, 8>(t, (unsigned)grid, smem, st); break;

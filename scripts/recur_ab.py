@@ -1,4 +1,5 @@
-"""A/B the fused coarse-level recurrence kernel (thread count) on the level-1 operator, L2-warm and cold."""
+"""A/B the fused coarse-level recurrence kernel against the step-by-step SpMM launches on the level-1 / 2 operators, L2-warm and
+cold."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -16,8 +17,8 @@ for lvl, B, F in [(1, 64, 16), (1, 64, 32), (2, 64, 16), (1, 256, 16)]:
     x = torch.randn(n, B, F, device=dev)
     w = torch.randn(6, F, 16, device=dev) * 0.1
     ref = None
-    for nt in (0, 256, 512, 768, 1024):
-        L.tune(f"fused_recurrence={nt}")
+    for fused in (0, 1):
+        L.tune(f"fused_recurrence={fused}")
         basis = torch.empty(5, n, B, F, device=dev); y = torch.empty(n, B, 16, device=dev)
         ms = {}
         for cold in (True, False):
@@ -32,5 +33,5 @@ for lvl, B, F in [(1, 64, 16), (1, 64, 32), (2, 64, 16), (1, 256, 16)]:
                 if i >= 3: t.append(s.elapsed_time(e))
             ms[cold] = sum(t) / len(t) * 1e3
         if ref is None: ref = basis.clone()
-        print(f"lvl{lvl} B{B} F{F} threads={nt:4d} ({L.lib.mvb_launch_count()-c0} launches): recurrence+contraction cold {ms[True]:6.1f} us  warm {ms[False]:6.1f} us  identical={torch.equal(basis, ref)}")
+        print(f"lvl{lvl} B{B} F{F} fused={fused} ({L.lib.mvb_launch_count()-c0} launches): recurrence+contraction cold {ms[True]:6.1f} us  warm {ms[False]:6.1f} us  identical={torch.equal(basis, ref)}")
 L.tune(f"fused_recurrence={1}")

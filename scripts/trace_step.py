@@ -24,7 +24,7 @@ if world > 1:
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 dev = torch.device("cuda", local)
 mvb, net, A, nn_ = bench.build_model(dev)
-# tuning hooks for A/B runs: MVB_TUNE="tc_balance=1;tc_tuning=2,3;mesh_tc=0" (include/mvb.h: mvb_tune)
+# switches for A/B runs: MVB_TUNE="fused_recurrence=0;mesh_tc=0" (include/mvb.h: mvb_tune)
 if os.environ.get("MVB_TUNE"):
     mvb._lib.tune(os.environ["MVB_TUNE"])
 from meshvae_b200.engine import TrainEngine  # noqa: E402

@@ -28,6 +28,21 @@ def test_library_exports_every_header_symbol():
     assert _lib.lib.mvb_sm_arch() == 100
 
 
+def test_tune_takes_only_the_implementation_switches():
+    """mvb_tune only sets host-side switches (no GPU needed).  The kernel variants and tuning knobs that were measured and
+    not adopted are gone: their keys are rejected like any unknown key, so none of them comes back unnoticed."""
+    retired = ["tc_tma", "wgrad_perm", "background_div", "tc_tuning", "tc_balance", "layer_tuning", "spmm_shape",
+               "spmm_mode", "stream_nt", "conv_lanes", "overlap", "mesh_dbg"]
+    try:
+        for key in retired:
+            with pytest.raises(_lib.MvbError, match="unknown key"):
+                _lib.tune(f"{key}=1")
+        for spec in ("mesh_tc=1,2", "fused_recurrence=0", "stream_tc=1,8", "pdl=0", "defer_wgrad=1"):
+            _lib.tune(spec)
+    finally:
+        _lib.tune("mesh_tc=1,0;fused_recurrence=1;stream_tc=0,16;pdl=1;defer_wgrad=0")
+
+
 def test_only_sm100a_code_is_embedded():
     import subprocess
     out = subprocess.run(["/usr/local/cuda/bin/cuobjdump", "--list-elf", mvb.build.LIB], capture_output=True, text=True)

@@ -206,27 +206,3 @@ def test_unsupported_levels_fall_back(mvb, ops):
     y = Fn.cheb_layer(x, w, None, l_op, None, None, relu=True)                       # composition path
     assert torch.equal(y, Fn.cheb_conv(x, w, None, l_op, True))
 
-
-def test_tma_fed_contraction_is_bit_identical(mvb, ops):
-    """mvb_tune tc_tma=1: the level-0 contraction with its operand tiles loaded by TMA (cp.async.bulk.tensor, SWIZZLE_64B: the raw
-    fp32 tile is the hi operand of the 3xTF32 scheme) forms the same products in the same order as the register-staged kernel"""
-    A, D, U, nn_ = ops
-    Fn = mvb.functional
-    dev = torch.device("cuda:0")
-    n = nn_[0]
-    ei, norm = O.cheb_norm(A[0]._indices(), n)
-    l_op = mvb.operators.from_edges(ei.to(dev), norm.to(dev), n, dev)
-    outs = []
-    for ring in (0, 3, 4):
-        mvb._lib.tune(f"tc_tma={1 if ring else 0},{ring or 4}")
-        try:
-            x = _rand(n, 64, 16, seed=11).to(dev).requires_grad_()
-            w = _rand(6, 16, 16, seed=12, scale=0.1).to(dev).requires_grad_()
-            b = _rand(16, seed=13, scale=0.1).to(dev).requires_grad_()
-            y = Fn.cheb_conv(x, w, b, l_op, True)
-            y.backward(_rand(n, 64, 16, seed=14).to(dev))
-            outs.append((y.detach().clone(), x.grad.clone(), w.grad.clone()))
-        finally:
-            mvb._lib.tune("tc_tma=0,4")
-    for o in outs[1:]:
-        assert all(torch.equal(p, q) for p, q in zip(outs[0], o))
