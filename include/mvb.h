@@ -279,7 +279,7 @@ int mvb_dp_reduce_adam(int world, int rank, int channel, int64_t offset, int64_t
  * mvb_cheb_sel_bwd: dW / db of such a layer when its input needs NO gradient (the first encoder layer: the basis form
  * dW_k = T_k^T G, db = 1^T G, G = dy_sel * [y_sel > 0] reduced over the selected rows only - G is zero elsewhere).
  * mvb_cheb_sel_supported: 1 for the plane widths of the tensor-core kernels (Fin 4 / 16 / 32, Fout % 4 == 0, <= 32), else 0 -
- * the caller then composes mvb_cheb_fwd + mvb_pool_fwd. */
+ * the caller then composes mvb_cheb_fwd + mvb_pool_fwd.  sel[n_sel]: distinct conv rows (see mvb_cheb_layer_fwd). */
 int mvb_cheb_sel_supported(int N, int B, int Fin, int Fout, int K, int n_sel);
 int mvb_cheb_sel_fwd(int N, int B, int Fin, int Fout, int K, int nnz, const int32_t *rowptr, const int32_t *colidx,
                      const float *vals, const float *x, const float *weight, const float *bias, int relu, int n_sel,
@@ -297,7 +297,9 @@ int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const float *x, con
  * epilogue (only the rows that D keeps are contracted and written).
  *   x [n_in,B,Fin] (n_in == N unless U [N x n_in] is given), y [n_out,B,Fout] (n_out == N unless
  *   sel[n_out] is given: output row r is conv row sel[r] - D is such a selection,
- *   mesh_operations.py:72-85: one 1.0 per row).
+ *   mesh_operations.py:72-85: one 1.0 per row).  The entries of sel must be distinct (the kernels invert the map); a D
+ *   that selects a vertex twice is a plain sparse product: mvb_pool_* after the convolution.  The same holds for the sel
+ *   of mvb_cheb_sel_*.
  * Two implementations behind the same entry points: the tensor-core mesh kernels (csrc/mvb_mesh_tc.cu: 16 / 32-wide
  *   features, up to 1280 vertices - levels 1-3 of the template; a cluster of 1-2 CTAs per mesh keeps the basis planes
  *   in shared memory in the UMMA operand layout and contracts them with tcgen05.mma into TMEM accumulators) and the

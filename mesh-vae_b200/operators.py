@@ -44,8 +44,10 @@ class MeshOperator:
         up = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(self.device)  # noqa: E731
         self.rowptr, self.colidx, self.vals = up(rp), up(ci), up(v)
         self.rowptr_t, self.colidx_t, self.vals_t = up(rpt), up(cit), up(vt)
-        # one nonzero per row with value 1 (the D matrices, mesh_operations.py:72-85): pure row selection
-        self.is_selection = bool(self.nnz == n_rows and np.all(np.diff(rp) == 1) and np.all(v == 1.0))
+        # one nonzero per row with value 1 at distinct columns (the D matrices, mesh_operations.py:72-85): pure row
+        # selection.  The fused kernels invert it (inv[sel[r]] = r), so a column selected twice must take the SpMM path
+        self.is_selection = bool(self.nnz == n_rows and np.all(np.diff(rp) == 1) and np.all(v == 1.0)
+                                 and np.unique(ci).shape[0] == self.nnz)
         # square operators: rows >= n_active are empty and no entry references a column >= n_active
         # (the coarse operator applied to a finer tensor, models/cheb_VAE.py:288) -> closed-form rows
         self.n_active = self.n_rows
