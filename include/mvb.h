@@ -57,9 +57,13 @@ int mvb_set_tensor_cores(int enable);
  * implementations tested against each other; pdl and defer_wgrad change only how kernels are launched and joined.  The
  * mvb Python package applies the environment variable MVB_TUNE through this call when it is imported. */
 int mvb_tune(const char *spec);
-/* Deferred side chains: with mvb_tune("defer_wgrad=1") the weight-gradient reductions of mvb_cheb_layer_bwd run on an
- * internal per-device side stream (as does the weight-gradient branch of mvb_cheb_bwd) and are NOT joined into the
- * caller's stream before the call returns - they then overlap the following layers' backward kernels.  The caller must
+/* Deferred side chains: with mvb_tune("defer_wgrad=1") the weight-gradient work of these calls runs on an internal
+ * per-device side stream and is NOT joined into the caller's stream before the call returns - it then overlaps the
+ * following layers' backward kernels:
+ *   lane 0: mvb_cheb_bwd in the adjoint form (mvb_cheb_bwd_uses_basis == 0), mvb_cheb_layer_bwd when its tensor-core
+ *           kernel runs, mvb_cheb_stream_bwd;
+ *   lane 1: mvb_linear_bwd with dx (its dW / db tiles run as a launch of their own).
+ * No other call defers.  The caller must
  * (1) keep every buffer of the call (workspace, x, dweight, dbias) alive and untouched until it has called
  * mvb_side_join(stream), which makes `stream` wait for the pending chain, and (2) call it before reading any gradient
  * and before a stream capture ends.  Default off: every call joins before it returns. */

@@ -94,10 +94,10 @@ class cheb_VAE(nn.Module):
             u_op = None if up is None else operators.from_sparse(up, x.device)
             d_op = None if down is None else operators.from_sparse(down, x.device)
             fin, fout = conv.weight.shape[1], conv.weight.shape[2]
-            if fin % 4 == 0 and fout % 4 == 0 and Fn.cheb_layer_supported(l_op.n_rows, x.shape[0], fin, fout, conv.weight.shape[0],
-                                                                           l_op, u_op, d_op):
-                y = Fn.cheb_layer(Fn.to_vertex_major(x), conv.weight, conv.bias, l_op, u_op, d_op, relu=True)
-                return Fn.from_vertex_major(y)
+            if fin % 4 == 0 and fout % 4 == 0:
+                y = Fn.cheb_layer_fused(Fn.to_vertex_major(x), conv.weight, conv.bias, l_op, u_op, d_op, relu=True)
+                if y is not None:
+                    return Fn.from_vertex_major(y)
             if u_op is None and fout % 4 == 0:
                 # level 0 (too large for a mesh-resident kernel): conv + ReLU + row selection, only the rows D keeps are
                 # contracted / reduced over (first encoder layer: its input needs no gradient)

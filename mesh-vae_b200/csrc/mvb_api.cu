@@ -4,6 +4,7 @@
 #include <stdarg.h>
 #include <stdlib.h>
 #include <atomic>
+#include <mutex>
 #include <vector>
 #include "mvb_internal.cuh"
 
@@ -51,8 +52,6 @@ void set_pdl(int v) { g_pdl = v ? 1 : 0; }
 extern "C" int mvb_version(void) { return MVB_VERSION; }
 extern "C" int mvb_sm_arch(void) { return 100; }
 extern "C" const char *mvb_last_error(void) { return err_buf(); }
-
-namespace mvb { long long launch_count(); }
 extern "C" int64_t mvb_launch_count(void) { return (int64_t)mvb::launch_count(); }
 
 
@@ -130,10 +129,6 @@ extern "C" int mvb_pool_bwd(int n_in_rows, int n_out_rows, const int32_t *rowptr
 // sum_k c_k W_k; only the first n_active vertices (a contiguous prefix in the vertex-major layout)
 // run the SpMM recurrence.  This is what makes the reference's output layer - the 20-vertex
 // operator applied to the 4998-vertex mesh, models/cheb_VAE.py:288 - a streaming pass.
-static void fill_contract(ContractArgs &a) {
-    memset(&a, 0, sizeof(a));
-}
-
 extern "C" int mvb_cheb_fwd(int N, int B, int Fin, int Fout, int K, int n_active, int nnz,
                             const int32_t *rowptr, const int32_t *colidx, const float *vals,
                             const float *x, const float *weight, const float *bias, int relu,
@@ -142,23 +137,11 @@ extern "C" int mvb_cheb_fwd(int N, int B, int Fin, int Fout, int K, int n_active
     MVB_REQUIRE(n_active >= 0 && n_active <= N, "cheb_fwd: n_active=%d outside [0,%d]", n_active, N);
     MVB_REQUIRE(x && weight && y && (K == 1 || n_active == 0 || (basis && rowptr)), "cheb_fwd: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t ncols = (int64_t)B * Fin;
-    const int64_t plane = (int64_t)n_active * ncols;
-    int rc;
     if (n_active > 0) {
         // recurrence: T_1 = L x ; T_k = 2 L T_{k-1} - T_{k-2}     (nn/conv.py:564, 568-569)
-        // one fused launch when the level fits shared memory, else one SpMM launch per step
-        rc = (K > 1) ? launch_cheb_recur_fwd(n_active, nnz, K, rowptr, colidx, vals, x, basis, ncols, st) : 1;
-        if (rc < 0) return rc;
-        for (int k = 1; k < K && rc == 0; ++k) {
-            float *tk = basis + (int64_t)(k - 1) * plane;
-            const float *tkm1 = (k == 1) ? x : basis + (int64_t)(k - 2) * plane;
-            const float *tkm2 = (k == 1) ? nullptr : (k == 2 ? x : basis + (int64_t)(k - 3) * plane);
-            int rc2 = launch_spmm(n_active, n_active, rowptr, colidx, vals, tkm1, tk, tkm2, nullptr, k == 1 ? 1.f : 2.f, -1.f, ncols, st);
-            if (rc2) return rc2;
-        }
-        ContractArgs a;
-        fill_contract(a);
+        int rc = launch_cheb_recurrence(n_active, nnz, K, rowptr, colidx, vals, x, basis, (int64_t)B * Fin, st);
+        if (rc) return rc;
+        ContractArgs a{};
         a.rows = (int64_t)n_active * B;
         a.in_planes = K;
         a.in_w = Fin;
@@ -175,29 +158,10 @@ extern "C" int mvb_cheb_fwd(int N, int B, int Fin, int Fout, int K, int n_active
     }
     if (n_active < N) {
         const int64_t off = (int64_t)n_active * B;
-        rc = launch_fold_fwd((int64_t)(N - n_active) * B, K, Fin, Fout, x + off * Fin, weight, bias, relu, y + off * Fout, st);
-        if (rc < 0) return rc;
-        if (rc == 1) return MVB_OK;
-        ContractArgs a;
-        fill_contract(a);
-        a.rows = (int64_t)(N - n_active) * B;
-        a.in_planes = 1;
-        a.in_w = Fin;
-        a.in0 = x + off * Fin;
-        a.wmat = weight;
-        a.w_fold = K;
-        a.bias = bias;
-        a.relu = relu;
-        a.out_planes = 1;
-        a.out_w = Fout;
-        a.out = y + off * Fout;
-        rc = launch_contract(a, st);
-        if (rc) return rc;
+        return launch_fold_fwd((int64_t)(N - n_active) * B, K, Fin, Fout, x + off * Fin, weight, bias, relu, y + off * Fout, st);
     }
     return MVB_OK;
 }
-
-static inline size_t align_up_c(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // ---------------------------------------------------------------------------------------------
 // Chebyshev convolution followed by a row selection (the encoder loop body at the levels that do not fit a
@@ -225,19 +189,9 @@ extern "C" int mvb_cheb_sel_fwd(int N, int B, int Fin, int Fout, int K, int nnz,
                 Fout, K, n_sel);
     MVB_REQUIRE(x && weight && y_sel && sel && (K == 1 || (basis && rowptr)), "cheb_sel_fwd: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t ncols = (int64_t)B * Fin;
-    const int64_t plane = (int64_t)N * ncols;
-    int rc = (K > 1) ? launch_cheb_recur_fwd(N, nnz, K, rowptr, colidx, vals, x, basis, ncols, st) : 1;
-    if (rc < 0) return rc;
-    for (int k = 1; k < K && rc == 0; ++k) {
-        float *tk = basis + (int64_t)(k - 1) * plane;
-        const float *tkm1 = (k == 1) ? x : basis + (int64_t)(k - 2) * plane;
-        const float *tkm2 = (k == 1) ? nullptr : (k == 2 ? x : basis + (int64_t)(k - 3) * plane);
-        int rc2 = launch_spmm(N, N, rowptr, colidx, vals, tkm1, tk, tkm2, nullptr, k == 1 ? 1.f : 2.f, -1.f, ncols, st);
-        if (rc2) return rc2;
-    }
-    ContractArgs a;
-    fill_contract(a);
+    int rc = launch_cheb_recurrence(N, nnz, K, rowptr, colidx, vals, x, basis, (int64_t)B * Fin, st);
+    if (rc) return rc;
+    ContractArgs a{};
     a.rows = (int64_t)n_sel * B;
     a.in_planes = K;
     a.in_w = Fin;
@@ -258,8 +212,13 @@ extern "C" int mvb_cheb_sel_fwd(int N, int B, int Fin, int Fout, int K, int nnz,
     return MVB_OK;
 }
 
+// workspace of mvb_cheb_sel_bwd: the weight-gradient partials
+static float *cheb_sel_bwd_ws(WsCarve &c, int Fin, int Fout, int K) { return c.take<float>(wgrad_partial_bytes(K * Fin, Fout)); }
+
 extern "C" size_t mvb_cheb_sel_bwd_workspace_bytes(int Fin, int Fout, int K) {
-    return align_up_c(wgrad_partial_bytes(K * Fin, Fout), 256);
+    WsCarve c;
+    cheb_sel_bwd_ws(c, Fin, Fout, K);
+    return c.off;
 }
 
 extern "C" int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const float *x, const float *basis,
@@ -267,11 +226,12 @@ extern "C" int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const fl
                                 float *dbias, void *workspace, size_t workspace_bytes, void *stream) {
     MVB_REQUIRE(sel_shape_ok(N, B, Fin, Fout, K, n_sel), "cheb_sel_bwd: shape not supported");
     MVB_REQUIRE(x && dy_sel && sel && dweight && workspace && (K == 1 || basis), "cheb_sel_bwd: null pointer");
-    const size_t need = mvb_cheb_sel_bwd_workspace_bytes(Fin, Fout, K);
-    if (workspace_bytes < need) return set_err(MVB_EWORKSPACE, "cheb_sel_bwd: workspace %zu < %zu", workspace_bytes, need);
+    WsCarve c{reinterpret_cast<char *>(workspace)};
+    WgradArgs wa{};
+    wa.partials = cheb_sel_bwd_ws(c, Fin, Fout, K);
+    wa.partial_bytes = c.off;
+    if (workspace_bytes < c.off) return set_err(MVB_EWORKSPACE, "cheb_sel_bwd: workspace %zu < %zu", workspace_bytes, c.off);
     cudaStream_t st = (cudaStream_t)stream;
-    WgradArgs wa;
-    memset(&wa, 0, sizeof(wa));
     wa.rows = (int64_t)n_sel * B;
     wa.in_planes = K;
     wa.in_w = Fin;
@@ -280,8 +240,6 @@ extern "C" int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const fl
     wa.dy = dy_sel;
     wa.mask = y_sel_for_relu;
     wa.n_out = Fout;
-    wa.partials = reinterpret_cast<float *>(workspace);
-    wa.partial_bytes = need;
     wa.row_sel = sel;
     wa.sel_group = B;
     wa.plane_rows = (int64_t)N * B;
@@ -291,22 +249,31 @@ extern "C" int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const fl
     return launch_wgrad_finalize(wa.partials, nA, m4A, nullptr, 0, 0, Fin, K * Fin, Fout, dweight, dbias, st);
 }
 
-static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-// per-host-thread side stream + fork/join events for intra-call concurrency
-struct SideStream {
+// ---------------------------------------------------------------------------------------------
+// Side chains (SideChain, mvb_internal.cuh).  A non-deferred chain that runs beside the caller's stream (the
+// weight-gradient branch of mvb_cheb_bwd) uses the calling thread's own side stream and is joined before the call
+// returns: the two branches overlap, and in a captured CUDA graph they become parallel branches.
+// Deferred chains: the weight-gradient reduction of a layer (10-20 us) is not on the critical path of the backward pass:
+// nothing reads dW / db before the optimizer.  In deferred mode (mvb_tune "defer_wgrad=1", switched on by the step
+// engine around its backward pass) such a chain is forked onto a per-device lane stream (the chains of successive layers
+// queue up there, each started by an event on the caller's stream once its producer kernel has been enqueued) and
+// joined back only by mvb_side_join - so they fill the idle SMs / memory bandwidth under the following layers'
+// latency-bound kernels; in a captured CUDA graph they form a parallel branch.
+// The deferred state is per device and process-wide (autograd runs backward functions on its own thread).
+// ---------------------------------------------------------------------------------------------
+namespace mvb {
+struct SideLane {
     cudaStream_t stream = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
-    bool ok = false;
+    bool tried = false, ok = false, pending = false;
 };
-static SideStream *side_stream() {
-    static thread_local SideStream s;
-    static thread_local bool tried = false;
-    if (!tried) {
-        tried = true;
-        // creation is not a stream operation: legal while another stream is capturing only in relaxed
-        // mode, so it is done during the (uncaptured) warm-up calls; if it fails we simply do not fork
-        if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess &&
+
+// Creation is not a stream operation: legal while another stream is capturing only in relaxed mode, so it happens
+// during the (uncaptured) warm-up calls; when it fails the lane is never used and the chain runs on the caller's stream.
+static SideLane *open_lane(SideLane &s, int priority) {
+    if (!s.tried) {
+        s.tried = true;
+        if (cudaStreamCreateWithPriority(&s.stream, cudaStreamNonBlocking, priority) == cudaSuccess &&
             cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming) == cudaSuccess &&
             cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) == cudaSuccess)
             s.ok = true;
@@ -316,57 +283,19 @@ static SideStream *side_stream() {
     return s.ok ? &s : nullptr;
 }
 
-// Two algebraically equal forms of the backward pass (L acts on vertices, W on features: they commute):
-//   basis form  : dW_k = T_k(L x)^T G,  dX = sum_k T_k(L^T) (G W_k^T)      - needs the forward basis T_k,
-//                 K planes P_k = G W_k^T and a reverse recurrence on Fin-wide planes;
-//   adjoint form: S_k = T_k(L^T) G,  dW_k = x^T S_k,  dX = sum_k S_k W_k^T - the FORWARD kernels run on G
-//                 (recurrence on Fout-wide planes, one contraction), nothing saved by the forward pass.
-// Plane traffic is ~(32 Fin + 2 Fout) vs ~(27 Fout + 2 Fin) plane-widths: the adjoint form is used when
-// the input gradient is wanted and Fout <= 1.2 Fin (every 16->16 layer of the reference model; the
-// first encoder layer, which needs no dX, keeps the basis form: its basis is only 3-4 columns wide).
-static bool adjoint_form(int Fin, int Fout, int need_dx) { return need_dx && 25 * Fout <= 30 * Fin && Fout % 4 == 0; }
-
-// fork the per-thread side stream from `st` (NULL when the fork fails)
-static SideStream *fork_side(cudaStream_t st) {
-    SideStream *side = side_stream();
-    if (!side) return nullptr;
-    if (cudaEventRecord(side->fork, st) != cudaSuccess || cudaStreamWaitEvent(side->stream, side->fork, 0) != cudaSuccess) {
+// make the lane wait for what `st` has enqueued so far
+static bool fork_lane(SideLane *s, cudaStream_t st) {
+    if (!s) return false;
+    if (cudaEventRecord(s->fork, st) != cudaSuccess || cudaStreamWaitEvent(s->stream, s->fork, 0) != cudaSuccess) {
         cudaGetLastError();
-        return nullptr;
+        return false;
     }
-    return side;
+    return true;
 }
-struct JoinGuard {   // the side stream must rejoin on every exit path (a captured graph must not end forked)
-    SideStream *s;
-    cudaStream_t main;
-    ~JoinGuard() {
-        if (s) {
-            cudaEventRecord(s->join, s->stream);
-            cudaStreamWaitEvent(main, s->join, 0);
-        }
-    }
-};
 
-// ---------------------------------------------------------------------------------------------
-// Deferred side chains.  The weight-gradient reduction of a mesh-resident layer (tc_wgrad + finalize kernels, 10-20 us)
-// is not on the critical path of the backward pass: nothing reads dW / db before the optimizer.  In deferred mode
-// (mvb_tune "defer_wgrad=1", switched on by the step engine around its backward pass) such a chain is forked onto a
-// per-device side stream (the chains of successive layers queue up there, each started by an event on the caller's
-// stream once its producer kernel has been enqueued) and joined back only by mvb_side_join - so they fill the idle
-// SMs / memory bandwidth under the following layers' latency-bound kernels; in a captured CUDA graph they form a
-// parallel branch.  Off (default): the chain is joined before the call returns.
-// The state is per device and process-wide (autograd runs backward functions on its own thread).
-// ---------------------------------------------------------------------------------------------
-#include <mutex>
-namespace mvb {
-struct LazySide {
-    cudaStream_t stream = nullptr;
-    cudaEvent_t fork = nullptr, join = nullptr;
-    bool tried = false, ok = false, pending = false;
-};
 constexpr int LAZY_SLOTS = 4;       // slot 1 = lane 1 (dense-layer weight gradients); slots 0, 2, 3 = lane 0 (convolution weight gradients:
                                     // successive chains go round robin over CONV_LANES of them, so that chains can overlap each other)
-static LazySide g_lazy[64][LAZY_SLOTS];
+static SideLane g_lazy[64][LAZY_SLOTS];
 constexpr int CONV_LANES = 3;       // same-box A/B (bench.py, 300 steps, second pass): 1 lane 0.9197 ms per step, 2: 0.9152, 3: 0.9116,
                                     // 4: 0.9109, 5: 0.9111, 7: 0.9109 - the chains queued behind each other in the tail of the
                                     // backward pass (the last layers' reductions) now run side by side
@@ -376,70 +305,70 @@ static std::mutex g_lazy_mu;
 static int g_defer_wgrad = 0;
 void set_defer_wgrad(int v) { g_defer_wgrad = v ? 1 : 0; }
 
-static LazySide *lazy_side(int slot) {
+static SideLane *lazy_side(int slot) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    LazySide &s = g_lazy[dev][slot & (LAZY_SLOTS - 1)];
-    if (!s.tried) {
-        s.tried = true;
-        // LOWEST priority: when a chain and a kernel of the caller's stream are ready together (the input-gradient
-        // contraction next to the weight-gradient reduction of the same layer), the block scheduler serves the caller's
-        // kernel first - the chain takes what is left (a captured graph keeps the priority as a kernel-node attribute)
-        int least = 0, greatest = 0;
-        if (cudaDeviceGetStreamPriorityRange(&least, &greatest) != cudaSuccess) { least = 0; cudaGetLastError(); }
-        if (cudaStreamCreateWithPriority(&s.stream, cudaStreamNonBlocking, least) == cudaSuccess &&
-            cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming) == cudaSuccess &&
-            cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) == cudaSuccess)
-            s.ok = true;
-        else
-            cudaGetLastError();
+    // LOWEST priority: when a chain and a kernel of the caller's stream are ready together (the input-gradient
+    // contraction next to the weight-gradient reduction of the same layer), the block scheduler serves the caller's
+    // kernel first - the chain takes what is left (a captured graph keeps the priority as a kernel-node attribute)
+    int least = 0, greatest = 0;
+    SideLane &s = g_lazy[dev][slot & (LAZY_SLOTS - 1)];
+    if (!s.tried && cudaDeviceGetStreamPriorityRange(&least, &greatest) != cudaSuccess) {
+        least = 0;
+        cudaGetLastError();
     }
-    return s.ok ? &s : nullptr;
+    return open_lane(s, least);
 }
 
 // make `st` wait for a pending chain (if any)
-static void lazy_join_locked(LazySide *s, cudaStream_t st) {
+static void lazy_join_locked(SideLane *s, cudaStream_t st) {
     if (s && s->pending) {
         cudaStreamWaitEvent(st, s->join, 0);
         s->pending = false;
     }
 }
 
-// Call AFTER the producer kernel of the chain has been enqueued on `st`.  Makes the side stream wait for that point of
-// `st`; returns the stream to enqueue the chain on, or NULL (not deferred / unavailable): run it on `st`.
-cudaStream_t lazy_fork(cudaStream_t st, int lane) {
-    if (!g_defer_wgrad) return nullptr;
-    std::lock_guard<std::mutex> lk(g_lazy_mu);
-    int slot = 1;
-    if (lane == 0) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-        slot = kConvSlot[g_conv_next[dev]];
-        g_conv_next[dev] = (g_conv_next[dev] + 1) % CONV_LANES;
+SideChain::SideChain(cudaStream_t st, int lane, bool local) : st_(st), stream_(st) {
+    if (lane >= 0 && g_defer_wgrad) {
+        std::lock_guard<std::mutex> lk(g_lazy_mu);
+        int slot = 1;
+        if (lane == 0) {
+            int dev = 0;
+            if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
+            slot = kConvSlot[g_conv_next[dev]];
+            g_conv_next[dev] = (g_conv_next[dev] + 1) % CONV_LANES;
+        }
+        SideLane *s = lazy_side(slot);
+        if (fork_lane(s, st)) {
+            lane_ = s;
+            stream_ = s->stream;
+            deferred_ = true;
+            return;
+        }
     }
-    LazySide *s = lazy_side(slot);
-    if (!s) return nullptr;
-    if (cudaEventRecord(s->fork, st) != cudaSuccess || cudaStreamWaitEvent(s->stream, s->fork, 0) != cudaSuccess) {
-        cudaGetLastError();
-        return nullptr;
+    if (local) {
+        static thread_local SideLane t_side;
+        SideLane *s = open_lane(t_side, 0);
+        if (fork_lane(s, st)) {
+            lane_ = s;
+            stream_ = s->stream;
+        }
     }
-    return s->stream;
 }
 
-// the chain has been enqueued on `side`: record its end (the side stream is in order: the latest record covers every
-// earlier chain); joined by mvb_side_join
-void lazy_done(cudaStream_t side, cudaStream_t st) {
-    if (!side) return;
-    std::lock_guard<std::mutex> lk(g_lazy_mu);
-    LazySide *s = nullptr;
-    for (int slot = 0; slot < LAZY_SLOTS; ++slot) {
-        LazySide *c = lazy_side(slot);
-        if (c && c->stream == side) { s = c; break; }
+// deferred: record the chain's end (a lane is in order: the latest record covers every earlier chain) for mvb_side_join;
+// local: join into the caller's stream now
+SideChain::~SideChain() {
+    if (!lane_) return;
+    if (deferred_) {
+        std::lock_guard<std::mutex> lk(g_lazy_mu);
+        cudaEventRecord(lane_->join, lane_->stream);
+        lane_->pending = true;
+        if (!g_defer_wgrad) lazy_join_locked(lane_, st_);
+    } else {
+        cudaEventRecord(lane_->join, lane_->stream);
+        cudaStreamWaitEvent(st_, lane_->join, 0);
     }
-    if (!s) return;
-    cudaEventRecord(s->join, s->stream);
-    s->pending = true;
-    if (!g_defer_wgrad) lazy_join_locked(s, st);
 }
 }  // namespace mvb
 
@@ -461,21 +390,63 @@ extern "C" int mvb_side_join_lane(void *stream, int lane) {
     return MVB_OK;
 }
 
+// Two algebraically equal forms of the backward pass (L acts on vertices, W on features: they commute):
+//   basis form  : dW_k = T_k(L x)^T G,  dX = sum_k T_k(L^T) (G W_k^T)      - needs the forward basis T_k,
+//                 K planes P_k = G W_k^T and a reverse recurrence on Fin-wide planes;
+//   adjoint form: S_k = T_k(L^T) G,  dW_k = x^T S_k,  dX = sum_k S_k W_k^T - the FORWARD kernels run on G
+//                 (recurrence on Fout-wide planes, one contraction), nothing saved by the forward pass.
+// Plane traffic is ~(32 Fin + 2 Fout) vs ~(27 Fout + 2 Fin) plane-widths: the adjoint form is used when
+// the input gradient is wanted and Fout <= 1.2 Fin (every 16->16 layer of the reference model; the
+// first encoder layer, which needs no dX, keeps the basis form: its basis is only 3-4 columns wide).
+static bool adjoint_form(int Fin, int Fout, int need_dx) { return need_dx && 25 * Fout <= 30 * Fin && Fout % 4 == 0; }
+
+// workspace of the basis form: weight-gradient partials of the active prefix and of the empty rows, then (with dX)
+// the K planes P_k = dY W_k^T
+struct ChebBwdBasisWs {
+    float *partA, *partB, *P;
+    size_t partA_bytes, partB_bytes;
+};
+static ChebBwdBasisWs cheb_bwd_basis_ws(WsCarve &c, int N, int B, int Fin, int Fout, int K, int n_active, int need_dx) {
+    ChebBwdBasisWs w{};
+    w.partA_bytes = align_up(wgrad_partial_bytes(K * Fin, Fout), 256);
+    w.partA = c.take<float>(w.partA_bytes);
+    if (n_active < N) {
+        w.partB_bytes = align_up(wgrad_partial_bytes(Fin, Fout), 256);
+        w.partB = c.take<float>(w.partB_bytes);
+    }
+    if (need_dx) w.P = c.take<float>((size_t)K * n_active * B * Fin * sizeof(float));
+    return w;
+}
+
+// workspace of the adjoint form: weight-gradient partials (active prefix, empty rows), the column-sum partials of db,
+// G = dY * [y > 0] and S_1..S_{K-1}
+struct ChebBwdAdjointWs {
+    float *partA, *partB, *colpart, *G, *S;
+    size_t partA_bytes, partB_bytes;
+};
+static ChebBwdAdjointWs cheb_bwd_adjoint_ws(WsCarve &c, int N, int B, int Fin, int Fout, int K, int n_active) {
+    ChebBwdAdjointWs w{};
+    w.partA_bytes = align_up(wgrad_partial_bytes(K * Fout, Fin), 256);
+    w.partA = c.take<float>(w.partA_bytes);
+    if (n_active < N) {
+        w.partB_bytes = align_up(wgrad_partial_bytes(Fin, Fout), 256);
+        w.partB = c.take<float>(w.partB_bytes);
+    }
+    w.colpart = c.take<float>((size_t)mask_colsum_blocks((int64_t)N * B) * Fout * sizeof(float));
+    w.G = c.take<float>((size_t)N * B * Fout * sizeof(float));
+    w.S = c.take<float>((size_t)(K > 1 ? K - 1 : 0) * n_active * B * Fout * sizeof(float));
+    return w;
+}
+
 extern "C" int mvb_cheb_bwd_uses_basis(int Fin, int Fout, int need_dx) { return adjoint_form(Fin, Fout, need_dx) ? 0 : 1; }
 
 extern "C" size_t mvb_cheb_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int n_active, int need_dx) {
-    if (adjoint_form(Fin, Fout, need_dx)) {
-        size_t bytes = align_up(wgrad_partial_bytes(K * Fout, Fin), 256);
-        if (n_active < N) bytes += align_up(wgrad_partial_bytes(Fin, Fout), 256);
-        bytes += align_up((size_t)mask_colsum_blocks((int64_t)N * B) * Fout * sizeof(float), 256);
-        bytes += align_up((size_t)N * B * Fout * sizeof(float), 256);                       // G
-        bytes += align_up((size_t)(K > 1 ? K - 1 : 0) * n_active * B * Fout * sizeof(float), 256);   // S_1..S_{K-1}
-        return bytes;
-    }
-    size_t bytes = align_up(wgrad_partial_bytes(K * Fin, Fout), 256);
-    if (n_active < N) bytes += align_up(wgrad_partial_bytes(Fin, Fout), 256);
-    if (need_dx) bytes += align_up((size_t)K * n_active * B * Fin * sizeof(float), 256);
-    return bytes;
+    WsCarve c;
+    if (adjoint_form(Fin, Fout, need_dx))
+        cheb_bwd_adjoint_ws(c, N, B, Fin, Fout, K, n_active);
+    else
+        cheb_bwd_basis_ws(c, N, B, Fin, Fout, K, n_active, need_dx);
+    return c.off;
 }
 
 static int cheb_bwd_adjoint(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, const int32_t *rowptr_t,
@@ -505,28 +476,19 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
     }
     const int64_t rows_act = (int64_t)n_active * B;
     const int64_t rows_in = (int64_t)(N - n_active) * B;
-    const int64_t ncols = (int64_t)B * Fin;
-    const int64_t plane = (int64_t)n_active * ncols;
-    char *ws = reinterpret_cast<char *>(workspace);
-    const size_t partA_bytes = align_up(wgrad_partial_bytes(K * Fin, Fout), 256);
-    const size_t partB_bytes = (n_active < N) ? align_up(wgrad_partial_bytes(Fin, Fout), 256) : 0;
-    float *partA = reinterpret_cast<float *>(ws);
-    float *partB = reinterpret_cast<float *>(ws + partA_bytes);
-    float *P = reinterpret_cast<float *>(ws + partA_bytes + partB_bytes);
+    WsCarve c{reinterpret_cast<char *>(workspace)};
+    const ChebBwdBasisWs w = cheb_bwd_basis_ws(c, N, B, Fin, Fout, K, n_active, dx != nullptr);
     const int has_bias = dbias != nullptr;
     int rc, nA = 0, m4A = 0, nB = 0, m4B = 0;
 
     // The weight-gradient branch (partials + ordered finalize) and the input-gradient branch
     // (P_k, reverse recurrence) are independent: fork the former onto a side stream so that the two
     // overlap (and become parallel branches of a captured CUDA graph), join before returning.
-    cudaStream_t wst = st;
-    SideStream *side = dx ? fork_side(st) : nullptr;
-    if (side) wst = side->stream;
-    JoinGuard join_guard{side, st};
+    SideChain side(st, -1, dx != nullptr);
+    const cudaStream_t wst = side.stream();
 
     // dW_k = T_k^T dY, db = 1^T dY over the active prefix ...
-    WgradArgs wa;
-    memset(&wa, 0, sizeof(wa));
+    WgradArgs wa{};
     wa.rows = rows_act;
     wa.in_planes = K;
     wa.in_w = Fin;
@@ -535,14 +497,13 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
     wa.dy = dy;
     wa.mask = y_for_relu;
     wa.n_out = Fout;
-    wa.partials = partA;
-    wa.partial_bytes = partA_bytes;
+    wa.partials = w.partA;
+    wa.partial_bytes = w.partA_bytes;
     rc = launch_wgrad_partials(wa, has_bias, &nA, &m4A, wst);
     if (rc) return rc;
     // ... plus S = x^T dY over the empty rows (dW_k += c_k S)
     if (rows_in > 0) {
-        WgradArgs wb;
-        memset(&wb, 0, sizeof(wb));
+        WgradArgs wb{};
         wb.rows = rows_in;
         wb.in_planes = 1;
         wb.in_w = Fin;
@@ -550,18 +511,17 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
         wb.dy = dy + rows_act * Fout;
         wb.mask = y_for_relu ? y_for_relu + rows_act * Fout : nullptr;
         wb.n_out = Fout;
-        wb.partials = partB;
-        wb.partial_bytes = partB_bytes;
+        wb.partials = w.partB;
+        wb.partial_bytes = w.partB_bytes;
         rc = launch_wgrad_partials(wb, has_bias, &nB, &m4B, wst);
         if (rc) return rc;
     }
-    rc = launch_wgrad_finalize(partA, nA, m4A, partB, nB, m4B, Fin, K * Fin, Fout, dweight, dbias, wst);
+    rc = launch_wgrad_finalize(w.partA, nA, m4A, w.partB, nB, m4B, Fin, K * Fin, Fout, dweight, dbias, wst);
     if (rc || !dx) return rc;
 
     if (rows_act > 0) {
         // P_k = dY W_k^T for all k in one pass (plane k of the workspace)
-        ContractArgs a;
-        fill_contract(a);
+        ContractArgs a{};
         a.rows = rows_act;
         a.in_planes = 1;
         a.in_w = Fout;
@@ -571,30 +531,16 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
         a.w_transposed = 1;
         a.out_planes = K;
         a.out_w = Fin;
-        a.out = P;
+        a.out = w.P;
         rc = launch_contract(a, st);
         if (rc) return rc;
-        // reverse recurrence, in place on the P planes (G_k overwrites P_k):
-        //   G_{K-1} = P_{K-1};  G_k = P_k + 2 L^T G_{k+1} - G_{k+2}  (k >= 1);  dX = P_0 + L^T G_1 - G_2
-        int fused = (K > 1) ? launch_cheb_recur_bwd(n_active, nnz, K, rowptr_t, colidx_t, vals_t, P, dx, ncols, st) : 0;
-        if (fused < 0) return fused;
-        for (int k = K - 2; k >= 0 && fused == 0; --k) {
-            float *pk = P + (int64_t)k * plane;
-            const float *gk1 = P + (int64_t)(k + 1) * plane;
-            const float *gk2 = (k + 2 <= K - 1) ? P + (int64_t)(k + 2) * plane : nullptr;
-            float *dst = (k == 0) ? dx : pk;
-            rc = launch_spmm(n_active, n_active, rowptr_t, colidx_t, vals_t, gk1, dst, gk2, pk, k == 0 ? 1.f : 2.f, -1.f, ncols, st);
-            if (rc) return rc;
-        }
-        if (K == 1) {
-            cudaError_t e = cudaMemcpyAsync(dx, P, (size_t)plane * sizeof(float), cudaMemcpyDeviceToDevice, st);
-            if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_bwd: memcpy: %s", cudaGetErrorString(e));
-        }
+        // reverse recurrence, in place on the P planes: dX = sum_k T_k(L^T) P_k
+        rc = launch_cheb_recurrence_bwd(n_active, nnz, K, rowptr_t, colidx_t, vals_t, w.P, dx, (int64_t)B * Fin, st);
+        if (rc) return rc;
     }
     if (rows_in > 0) {
         // empty rows: dX = dY (sum_k c_k W_k)^T
-        ContractArgs a;
-        fill_contract(a);
+        ContractArgs a{};
         a.rows = rows_in;
         a.in_planes = 1;
         a.in_w = Fout;
@@ -617,56 +563,31 @@ static int cheb_bwd_adjoint(int N, int B, int Fin, int Fout, int K, int n_active
                             const float *y_for_relu, const float *dy, float *dx, float *dweight, float *dbias, char *ws,
                             cudaStream_t st) {
     const int64_t rows_act = (int64_t)n_active * B, rows_in = (int64_t)(N - n_active) * B, rows_all = (int64_t)N * B;
-    const int64_t ncols = (int64_t)B * Fout;
-    const int64_t plane = (int64_t)n_active * ncols;
-    const size_t partA_bytes = align_up(wgrad_partial_bytes(K * Fout, Fin), 256);
-    const size_t partB_bytes = (n_active < N) ? align_up(wgrad_partial_bytes(Fin, Fout), 256) : 0;
-    const size_t col_bytes = align_up((size_t)mask_colsum_blocks(rows_all) * Fout * sizeof(float), 256);
-    const size_t g_bytes = align_up((size_t)rows_all * Fout * sizeof(float), 256);
-    float *partA = reinterpret_cast<float *>(ws);
-    float *partB = reinterpret_cast<float *>(ws + partA_bytes);
-    float *colpart = reinterpret_cast<float *>(ws + partA_bytes + partB_bytes);
-    float *Gbuf = reinterpret_cast<float *>(ws + partA_bytes + partB_bytes + col_bytes);
-    float *S = reinterpret_cast<float *>(ws + partA_bytes + partB_bytes + col_bytes + g_bytes);
+    WsCarve c{ws};
+    const ChebBwdAdjointWs w = cheb_bwd_adjoint_ws(c, N, B, Fin, Fout, K, n_active);
     // G = dY * [y > 0] over ALL rows, db = column sums of G
-    const float *G = y_for_relu ? Gbuf : dy;
-    int rc = launch_mask_colsum(rows_all, Fout, dy, y_for_relu, y_for_relu ? Gbuf : nullptr, dbias, colpart, st);
+    const float *G = y_for_relu ? w.G : dy;
+    int rc = launch_mask_colsum(rows_all, Fout, dy, y_for_relu, y_for_relu ? w.G : nullptr, dbias, w.colpart, st);
     if (rc) return rc;
     // S_k = T_k(L^T) G on the active prefix: the forward recurrence kernels with CSR(L^T)
-    if (n_active > 0 && K > 1) {
-        rc = launch_cheb_recur_fwd(n_active, nnz, K, rowptr_t, colidx_t, vals_t, G, S, ncols, st);
-        if (rc < 0) return rc;
-        for (int k = 1; k < K && rc == 0; ++k) {
-            float *sk = S + (int64_t)(k - 1) * plane;
-            const float *skm1 = (k == 1) ? G : S + (int64_t)(k - 2) * plane;
-            const float *skm2 = (k == 1) ? nullptr : (k == 2 ? G : S + (int64_t)(k - 3) * plane);
-            int rc2 = launch_spmm(n_active, n_active, rowptr_t, colidx_t, vals_t, skm1, sk, skm2, nullptr, k == 1 ? 1.f : 2.f, -1.f, ncols, st);
-            if (rc2) return rc2;
-        }
+    if (n_active > 0) {
+        rc = launch_cheb_recurrence(n_active, nnz, K, rowptr_t, colidx_t, vals_t, G, w.S, (int64_t)B * Fout, st);
+        if (rc) return rc;
     }
     // weight-gradient branch on a side stream, input-gradient contraction on the main stream.  Deferred mode (step
     // engine): the branch is joined lazily - nothing reads dW before the optimizer - so the contraction that the next
     // layer waits for no longer shares the memory system with it; otherwise forked and joined within this call.
-    cudaStream_t wst = st;
-    cudaStream_t lazy = lazy_fork(st);
-    SideStream *side = lazy ? nullptr : fork_side(st);
-    if (lazy) wst = lazy;
-    else if (side) wst = side->stream;
-    JoinGuard join_guard{side, st};
-    struct LazyGuard {
-        cudaStream_t s, main;
-        ~LazyGuard() { lazy_done(s, main); }
-    } lazy_guard{lazy, st};
+    SideChain side(st, 0, true);
+    const cudaStream_t wst = side.stream();
     // the input-gradient contraction is launched FIRST (the next layer waits for it; in deferred mode the
     // weight-gradient chain behind it then only takes the block slots it leaves free)
     if (rows_act > 0) {      // dX = sum_k S_k W_k^T
-        ContractArgs a;
-        fill_contract(a);
+        ContractArgs a{};
         a.rows = rows_act;
         a.in_planes = K;
         a.in_w = Fout;
         a.in0 = G;
-        a.in_rest = S;
+        a.in_rest = w.S;
         a.wmat = weight;
         a.w_transposed = 2;
         a.out_planes = 1;
@@ -677,61 +598,28 @@ static int cheb_bwd_adjoint(int N, int B, int Fin, int Fout, int K, int n_active
     }
     if (rows_in > 0) {       // empty rows: dX = G (sum_k c_k W_k)^T
         rc = launch_fold_dx(rows_in, K, Fin, Fout, G + rows_act * Fout, weight, dx + rows_act * Fin, st);
-        if (rc < 0) return rc;
-        if (rc == 0) {
-        ContractArgs a;
-        fill_contract(a);
-        a.rows = rows_in;
-        a.in_planes = 1;
-        a.in_w = Fout;
-        a.in0 = G + rows_act * Fout;
-        a.wmat = weight;
-        a.w_transposed = 1;
-        a.w_fold = K;
-        a.out_planes = 1;
-        a.out_w = Fin;
-        a.out = dx + rows_act * Fin;
-        rc = launch_contract(a, st);
         if (rc) return rc;
-        }
     }
     int nA = 0, m4A = 0, nB = 0, m4B = 0;
     if (rows_act > 0) {      // A = [S_0|..|S_{K-1}]^T x   ([K*Fout, Fin]; dW_k[i][o] = A[k*Fout + o][i])
-        WgradArgs wa;
-        memset(&wa, 0, sizeof(wa));
+        WgradArgs wa{};
         wa.rows = rows_act;
         wa.in_planes = K;
         wa.in_w = Fout;
         wa.in0 = G;
-        wa.in_rest = S;
+        wa.in_rest = w.S;
         wa.dy = x;
         wa.n_out = Fin;
-        wa.partials = partA;
-        wa.partial_bytes = partA_bytes;
+        wa.partials = w.partA;
+        wa.partial_bytes = w.partA_bytes;
         rc = launch_wgrad_partials(wa, 0, &nA, &m4A, wst);
         if (rc) return rc;
     }
     if (rows_in > 0) {       // empty rows of the operator: S = x^T G, dW_k += cos(k pi/2) S
-        rc = launch_fold_wgrad(rows_in, Fin, Fout, x + rows_act * Fin, G + rows_act * Fout, partB, partB_bytes, &nB, &m4B, wst);
-        if (rc < 0) return rc;
-    }
-    if (rows_in > 0 && nB == 0) {
-        WgradArgs wb;
-        memset(&wb, 0, sizeof(wb));
-        wb.rows = rows_in;
-        wb.in_planes = 1;
-        wb.in_w = Fin;
-        wb.in0 = x + rows_act * Fin;
-        wb.dy = G + rows_act * Fout;
-        wb.n_out = Fout;
-        wb.partials = partB;
-        wb.partial_bytes = partB_bytes;
-        rc = launch_wgrad_partials(wb, 0, &nB, &m4B, wst);
+        rc = launch_fold_wgrad(rows_in, Fin, Fout, x + rows_act * Fin, G + rows_act * Fout, w.partB, w.partB_bytes, &nB, &m4B, wst);
         if (rc) return rc;
     }
-    rc = launch_wgrad_finalize(partA, nA, m4A, partB, nB, m4B, Fin, K * Fin, Fout, dweight, nullptr, wst, 1);
-    if (rc) return rc;
-    return MVB_OK;
+    return launch_wgrad_finalize(w.partA, nA, m4A, w.partB, nB, m4B, Fin, K * Fin, Fout, dweight, nullptr, wst, 1);
 }
 
 // Make `stream` wait for the LATEST record of `event` at execution time.  With cudaEventWaitExternal the call is

@@ -666,37 +666,73 @@ static int fold_grid(int64_t threads) {
     return (int)(g > cap ? cap : (g < 1 ? 1 : g));
 }
 
-// 1 = handled, 0 = shape not covered (caller uses the generic kernels), < 0 = error
 int launch_fold_fwd(int64_t rows, int K, int Fin, int Fout, const float *x, const float *w, const float *bias, int relu,
                     float *out, cudaStream_t st) {
-    if (!fold_ok(K, Fin, Fout, x, out, bias)) return 0;
-    launch_pdl(fold_rows_fwd_kernel, dim3(fold_grid(rows * (Fout / 4))), dim3(256), (size_t)Fin * Fout * 4, st, rows, K, Fin, Fout, x, w, bias, relu, out);
-    const int rc = check_launch("mvb fold_rows_fwd");
-    return rc ? rc : 1;
+    if (fold_ok(K, Fin, Fout, x, out, bias)) {
+        launch_pdl(fold_rows_fwd_kernel, dim3(fold_grid(rows * (Fout / 4))), dim3(256), (size_t)Fin * Fout * 4, st, rows, K, Fin, Fout, x, w, bias, relu, out);
+        return check_launch("mvb fold_rows_fwd");
+    }
+    ContractArgs a{};
+    a.rows = rows;
+    a.in_planes = 1;
+    a.in_w = Fin;
+    a.in0 = x;
+    a.wmat = w;
+    a.w_fold = K;
+    a.bias = bias;
+    a.relu = relu;
+    a.out_planes = 1;
+    a.out_w = Fout;
+    a.out = out;
+    return launch_contract(a, st);
 }
 int launch_fold_dx(int64_t rows, int K, int Fin, int Fout, const float *g, const float *w, float *dx, cudaStream_t st) {
-    if (!fold_ok(K, Fin, Fout, g, dx, nullptr)) return 0;
-    launch_pdl(fold_rows_dx_kernel, dim3(fold_grid(rows * (Fin / 4))), dim3(256), (size_t)Fin * Fout * 4, st, rows, K, Fin, Fout, g, w, dx);
-    const int rc = check_launch("mvb fold_rows_dx");
-    return rc ? rc : 1;
+    if (fold_ok(K, Fin, Fout, g, dx, nullptr)) {
+        launch_pdl(fold_rows_dx_kernel, dim3(fold_grid(rows * (Fin / 4))), dim3(256), (size_t)Fin * Fout * 4, st, rows, K, Fin, Fout, g, w, dx);
+        return check_launch("mvb fold_rows_dx");
+    }
+    ContractArgs a{};
+    a.rows = rows;
+    a.in_planes = 1;
+    a.in_w = Fout;
+    a.in0 = g;
+    a.wmat = w;
+    a.w_transposed = 1;
+    a.w_fold = K;
+    a.out_planes = 1;
+    a.out_w = Fin;
+    a.out = dx;
+    return launch_contract(a, st);
 }
-// partials: at least wgrad_partial_bytes(Fin, Fout); *nparts blocks of [Fin][Fout] are written, *m4 = Fin
+// partials: at least wgrad_partial_bytes(Fin, Fout); *nparts blocks of [*m4][Fout] are written
 int launch_fold_wgrad(int64_t rows, int Fin, int Fout, const float *x, const float *g, float *partials, size_t partial_bytes,
                       int *nparts, int *m4, cudaStream_t st) {
-    if (!fold_ok(1, Fin, Fout, x, g, partials)) return 0;
-    const int nblk = (Fin / 4) * (Fout / 4);
-    const int lanes = 256 / nblk;
-    int64_t grid = (rows + (int64_t)lanes * 16 - 1) / ((int64_t)lanes * 16);      // >= 16 rows per lane
-    const int64_t cap = (int64_t)num_sms() * 2;
-    if (grid > cap) grid = cap;
-    if (grid < 1) grid = 1;
-    if ((size_t)grid * Fin * Fout * sizeof(float) > partial_bytes) return 0;
-    launch_pdl(fold_rows_wgrad_kernel, dim3((unsigned)grid), dim3(256), (size_t)lanes * nblk * 16 * 4, st, rows, Fin, Fout, x, g, partials);
-    const int rc = check_launch("mvb fold_rows_wgrad");
-    if (rc) return rc;
-    *nparts = (int)grid;
-    *m4 = Fin;
-    return 1;
+    if (fold_ok(1, Fin, Fout, x, g, partials)) {
+        const int nblk = (Fin / 4) * (Fout / 4);
+        const int lanes = 256 / nblk;
+        int64_t grid = (rows + (int64_t)lanes * 16 - 1) / ((int64_t)lanes * 16);      // >= 16 rows per lane
+        const int64_t cap = (int64_t)num_sms() * 2;
+        if (grid > cap) grid = cap;
+        if (grid < 1) grid = 1;
+        if ((size_t)grid * Fin * Fout * sizeof(float) <= partial_bytes) {
+            launch_pdl(fold_rows_wgrad_kernel, dim3((unsigned)grid), dim3(256), (size_t)lanes * nblk * 16 * 4, st, rows, Fin, Fout, x, g, partials);
+            const int rc = check_launch("mvb fold_rows_wgrad");
+            if (rc) return rc;
+            *nparts = (int)grid;
+            *m4 = Fin;
+            return MVB_OK;
+        }
+    }
+    WgradArgs a{};
+    a.rows = rows;
+    a.in_planes = 1;
+    a.in_w = Fin;
+    a.in0 = x;
+    a.dy = g;
+    a.n_out = Fout;
+    a.partials = partials;
+    a.partial_bytes = partial_bytes;
+    return launch_wgrad_partials(a, 0, nparts, m4, st);
 }
 
 // phase 2: dweight [M, n_out] (M = K*fin), dbias [n_out] or null.  a_transposed: see the kernel.

@@ -543,14 +543,6 @@ vae_heads_bwd_kernel(int B, int H, int Z, int C, const float *__restrict__ h, co
 
 using namespace mvb;
 
-static bool al16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
-template <typename KernelT>
-static int ensure_smem(KernelT kernel, size_t bytes, DevFlags *granted, const char *what) {
-    if (bytes <= 48 * 1024) return MVB_OK;
-    return smem_optin(kernel, bytes, *granted, what);
-}
-
 extern "C" int mvb_linear_fwd(int M, int K, int N, const float *x, int x_vm_f, const float *W, const float *bias,
                               int relu, float p_drop, uint64_t seed, const int64_t *offset_dev, int64_t offset_host,
                               float *y, int y_vm_f, void *stream) {
@@ -560,10 +552,10 @@ extern "C" int mvb_linear_fwd(int M, int K, int N, const float *x, int x_vm_f, c
     MVB_REQUIRE((int64_t)M * N < (1LL << 32), "linear_fwd: M*N exceeds the dropout counter range");
     const int K4 = (K + 3) & ~3;
     const int KC = K4 < 640 ? K4 : 640;
-    const bool vec = (K % 4 == 0) && (x_vm_f == 0 || x_vm_f % 4 == 0) && al16(x) && al16(W);
+    const bool vec = (K % 4 == 0) && (x_vm_f == 0 || x_vm_f % 4 == 0) && aligned16(x) && aligned16(W);
     const size_t smem = (size_t)(LF_TM + LF_TN) * (KC + 4) * sizeof(float);
     static DevFlags granted4, granted1;
-    int rc = vec ? ensure_smem(linear_fwd_kernel<4>, smem, &granted4, "linear_fwd") : ensure_smem(linear_fwd_kernel<1>, smem, &granted1, "linear_fwd");
+    int rc = vec ? smem_optin(linear_fwd_kernel<4>, smem, granted4, "linear_fwd") : smem_optin(linear_fwd_kernel<1>, smem, granted1, "linear_fwd");
     if (rc) return rc;
     dim3 grid((N + LF_TN - 1) / LF_TN, (M + LF_TM - 1) / LF_TM);
     if (vec)
@@ -588,14 +580,14 @@ extern "C" int mvb_linear_bwd(int M, int K, int N, const float *x, int x_vm_f, c
     const size_t smA = (size_t)3 * 64 * BW_LA * sizeof(float);
     const size_t smB = (size_t)(2 * BW_TMB * (nc_b + 4) + nc_b * BW_TKX) * sizeof(float);
     const size_t smem = nB ? (smA > smB ? smA : smB) : smA;
-    const bool vn = (N % 4 == 0) && (y_vm_f == 0 || y_vm_f % 4 == 0) && al16(gy) && (!relu || al16(y));
-    const bool vk = (K % 4 == 0) && (x_vm_f == 0 || x_vm_f % 4 == 0) && al16(x) && al16(W);
+    const bool vn = (N % 4 == 0) && (y_vm_f == 0 || y_vm_f % 4 == 0) && aligned16(gy) && (!relu || aligned16(y));
+    const bool vk = (K % 4 == 0) && (x_vm_f == 0 || x_vm_f % 4 == 0) && aligned16(x) && aligned16(W);
     static DevFlags granted[4];
     const float scale = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
     int rc;
 #define MVB_LBWD(VN_, VK_, SLOT)                                                                                             \
     do {                                                                                                                     \
-        rc = ensure_smem(linear_bwd_kernel<VN_, VK_>, smem, &granted[SLOT], "linear_bwd");                                   \
+        rc = smem_optin(linear_bwd_kernel<VN_, VK_>, smem, granted[SLOT], "linear_bwd");                                     \
         if (rc) return rc;                                                                                                   \
         launch_pdl(linear_bwd_kernel<VN_, VK_>, dim3(nA + nB), dim3(256), smem, (cudaStream_t)stream, M, K, N, x, x_vm_f, W, y, gy, y_vm_f, relu, \
                                                                                   scale, dx, dW, db, nA, k_tiles, nc_b);     \
@@ -603,26 +595,24 @@ extern "C" int mvb_linear_bwd(int M, int K, int N, const float *x, int x_vm_f, c
     // Deferred mode (step engine, mvb_tune "defer_wgrad=1"): the input-gradient tiles (role B) are what the backward
     // pass waits for - they are launched alone on the caller's stream, and the weight / bias gradient tiles (role A) go
     // to the deferred side chain (joined by mvb_side_join before the optimizer).  Otherwise one launch with both roles.
-    cudaStream_t lazy = (dx && nB) ? lazy_fork((cudaStream_t)stream, 1) : nullptr;
+    SideChain side((cudaStream_t)stream, (dx && nB) ? 1 : -1, false);
 #define MVB_LBWD_SPLIT(VN_, VK_, SLOT)                                                                                        \
     do {                                                                                                                     \
-        rc = ensure_smem(linear_bwd_kernel<VN_, VK_>, smem, &granted[SLOT], "linear_bwd");                                   \
-        if (rc) break;                                                                                                       \
+        rc = smem_optin(linear_bwd_kernel<VN_, VK_>, smem, granted[SLOT], "linear_bwd");                                     \
+        if (rc) return rc;                                                                                                   \
         launch_pdl(linear_bwd_kernel<VN_, VK_>, dim3(nB), dim3(256), smem, (cudaStream_t)stream, M, K, N, x, x_vm_f, W, y, gy, y_vm_f, relu,      \
                                                                              scale, dx, dW, db, 0, k_tiles, nc_b);           \
         rc = check_launch("mvb_linear_bwd dx");                                                                              \
-        if (rc) break;                                                                                                       \
-        launch_pdl(linear_bwd_kernel<VN_, VK_>, dim3(nA), dim3(256), smem, lazy, M, K, N, x, x_vm_f, W, y, gy, y_vm_f, relu, scale, nullptr, dW,  \
-                                                             db, nA, k_tiles, nc_b);                                         \
-        rc = check_launch("mvb_linear_bwd dW");                                                                              \
+        if (rc) return rc;                                                                                                   \
+        launch_pdl(linear_bwd_kernel<VN_, VK_>, dim3(nA), dim3(256), smem, side.stream(), M, K, N, x, x_vm_f, W, y, gy, y_vm_f, relu, scale,     \
+                                                             nullptr, dW, db, nA, k_tiles, nc_b);                            \
+        return check_launch("mvb_linear_bwd dW");                                                                            \
     } while (0)
-    if (lazy) {
+    if (side.deferred()) {
         if (vn && vk) MVB_LBWD_SPLIT(4, 4, 0);
         else if (vn) MVB_LBWD_SPLIT(4, 1, 1);
         else if (vk) MVB_LBWD_SPLIT(1, 4, 2);
         else MVB_LBWD_SPLIT(1, 1, 3);
-        lazy_done(lazy, (cudaStream_t)stream);
-        return rc;
     }
 #undef MVB_LBWD_SPLIT
     if (vn && vk) MVB_LBWD(4, 4, 0);
@@ -645,7 +635,7 @@ extern "C" int mvb_vae_heads_fwd(int B, int H, int Z, int C, const float *h, con
     const size_t smem = (size_t)(2 * (C + H) + (C + 2 * Z) * (C + H + 1)) * sizeof(float);
     MVB_REQUIRE(smem <= 220 * 1024, "vae_heads_fwd: H=%d too large", H);
     static DevFlags granted;
-    int rc = ensure_smem(vae_heads_fwd_kernel, smem, &granted, "vae_heads_fwd");
+    int rc = smem_optin(vae_heads_fwd_kernel, smem, granted, "vae_heads_fwd");
     if (rc) return rc;
     launch_pdl(vae_heads_fwd_kernel, dim3(B), dim3(256), smem, (cudaStream_t)stream, B, H, Z, C, h, y_onehot, eps, Wc, bc, Wm, bm, Wv, bv, p_drop,
                                                                   seed, offset_dev, offset_host, y_hat, mu, logvar, z, zcat);
@@ -667,7 +657,7 @@ extern "C" int mvb_vae_heads_bwd(int B, int H, int Z, int C, const float *h, con
     const size_t smem = smA > smB ? smA : smB;
     MVB_REQUIRE(smem <= 220 * 1024, "vae_heads_bwd: batch %d / H=%d too large for one pass", B, H);
     static DevFlags granted;
-    int rc = ensure_smem(vae_heads_bwd_kernel, smem, &granted, "vae_heads_bwd");
+    int rc = smem_optin(vae_heads_bwd_kernel, smem, granted, "vae_heads_bwd");
     if (rc) return rc;
     const int nbg = (B + HB_ROWS - 1) / HB_ROWS;
     const int ntile = (C + H + 1 + 31) / 32;

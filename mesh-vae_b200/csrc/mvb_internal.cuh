@@ -13,6 +13,23 @@ char *err_buf();
 int set_err(int code, const char *fmt, ...);
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Bump carver over a caller's workspace: every piece starts at an `align`-aligned offset and spans a whole number of
+// `align` units.  One function per entry point describes its workspace with it: the *_workspace_bytes query runs that
+// function with base == nullptr (it only measures, every pointer is NULL) and the launch runs it on the caller's buffer,
+// so the two cannot disagree.
+struct WsCarve {
+    char *base = nullptr;
+    size_t off = 0;
+    template <class T>
+    T *take(size_t bytes, size_t align = 256) {
+        off = align_up(off, align);
+        T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
+        off += align_up(bytes, align);
+        return p;
+    }
+};
 
 #define MVB_REQUIRE(cond, ...)                          \
     do {                                                \
@@ -49,6 +66,7 @@ struct DevFlags {
 };
 template <typename KernelT>
 inline int smem_optin(KernelT kernel, size_t bytes, DevFlags &f, const char *what) {
+    if (bytes <= 48 * 1024) return MVB_OK;          // the default limit: no opt-in needed
     const int d = device_slot();
     if (bytes <= f.granted[d]) return MVB_OK;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
@@ -72,8 +90,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // launch with the programmatic-serialization attribute (kernels that begin with pdl_trigger() / pdl_wait())
 template <typename... KArgs, typename... Args>
 inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
+    cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
@@ -132,11 +149,14 @@ int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t
                 const float *x, float *y, const float *z, const float *w, float alpha, float beta,
                 int64_t ncols, cudaStream_t st);
 
-// fused multi-step recurrences for N that fits shared memory: 1 = handled, 0 = use the step kernels
-int launch_cheb_recur_fwd(int N, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
-                          const float *x, float *basis, int64_t ncols, cudaStream_t st);
-int launch_cheb_recur_bwd(int N, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
-                          const float *P, float *dx, int64_t ncols, cudaStream_t st);
+// Chebyshev recurrence T_1 = L t0, T_k = 2 L T_{k-1} - T_{k-2} (k < K) into planes[k-1] (n * ncols floats each): one
+// fused launch when the level fits shared memory, else one SpMM launch per step.
+int launch_cheb_recurrence(int n, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
+                           const float *t0, float *planes, int64_t ncols, cudaStream_t st);
+// its reverse: in place on the K planes P (G_k overwrites P_k), G_{K-1} = P_{K-1}, G_k = P_k + 2 L^T G_{k+1} - G_{k+2}
+// (k >= 1), dx = P_0 + L^T G_1 - G_2 (dx = P_0 when K == 1); CSR(L^T) in rowptr_t / colidx_t / vals_t
+int launch_cheb_recurrence_bwd(int n, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
+                               float *P, float *dx, int64_t ncols, cudaStream_t st);
 
 // Generic small-matrix contraction over the rows of vertex-major activations:
 //   out[p_out][row][j] = act( sum_{p_in,i} in[p_in][row][i] * Wm[p_in*in_w + i][p_out*out_w + j] + bias )
@@ -191,7 +211,8 @@ int mask_colsum_blocks(int64_t rows);
 int launch_mask_colsum(int64_t rows, int ncol, const float *dy, const float *y, float *g, float *db, float *part,
                        cudaStream_t st);
 
-// narrow closed-form rows (operator rows without entries): 1 = handled, 0 = shape not covered, < 0 = error
+// closed-form rows (operator rows without entries): narrow FFMA kernels where they cover the shape, else the generic
+// contraction / weight-gradient kernels with w_fold = K
 int launch_fold_fwd(int64_t rows, int K, int Fin, int Fout, const float *x, const float *w, const float *bias, int relu,
                     float *out, cudaStream_t st);
 int launch_fold_dx(int64_t rows, int K, int Fin, int Fout, const float *g, const float *w, float *dx, cudaStream_t st);
@@ -224,8 +245,28 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
 // ordered sum over the meshes of per-mesh partials (mvb_layer.cu): dw[j] = sum_b dwp[b][j], db likewise
 int launch_layer_finalize(int B, int nw, int nb, const float *dwp, const float *dbp, float *dw, float *db, cudaStream_t st);
 
-// deferred side chains (mvb_api.cu): see lazy_fork / lazy_done / mvb_side_join
-cudaStream_t lazy_fork(cudaStream_t st, int lane = 0);
-void lazy_done(cudaStream_t side, cudaStream_t st);
+// A side chain: kernels that need what the caller's stream `st` has enqueued so far - construct the guard after the
+// chain's producer kernel - but that nothing later on `st` reads before the call returns (weight gradients).  stream()
+// is where to enqueue the chain:
+//   - while mvb_tune "defer_wgrad=1" is on and lane >= 0: a deferred lane (mvb_api.cu; lane 0 = convolution weight
+//     gradients, lane 1 = dense-layer weight gradients).  The destructor records the chain's end; mvb_side_join joins it.
+//   - otherwise, with `local`: the calling thread's side stream.  The destructor joins it into `st`.
+//   - otherwise (or when no side stream can be had): `st` itself.
+// The destructor runs on every exit path: a captured graph must not end forked.
+struct SideLane;
+class SideChain {
+  public:
+    SideChain(cudaStream_t st, int lane, bool local);
+    ~SideChain();
+    SideChain(const SideChain &) = delete;
+    SideChain &operator=(const SideChain &) = delete;
+    cudaStream_t stream() const { return stream_; }
+    bool deferred() const { return deferred_; }
+
+  private:
+    cudaStream_t st_, stream_;
+    SideLane *lane_ = nullptr;
+    bool deferred_ = false;
+};
 
 }  // namespace mvb

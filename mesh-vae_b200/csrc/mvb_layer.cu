@@ -544,13 +544,21 @@ extern "C" int mvb_cheb_layer_supported(int N, int B, int Fin, int Fout, int K, 
     return fwd && bwd;
 }
 
-extern "C" size_t mvb_cheb_layer_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int has_up) {
-    const size_t ffma = ((size_t)B * K * Fin * Fout + (size_t)B * Fout) * sizeof(float);
-    const size_t tc = mesh_tc_bwd_workspace_bytes(N, B, Fin, Fout, K, has_up);
-    return ffma > tc ? ffma : tc;
+// workspace of the FFMA backward kernel: per-mesh dW partials [B][K*Fin*Fout], then per-mesh db partials [B][Fout]
+static float *layer_bwd_ws(WsCarve &c, int B, int Fin, int Fout, int K, float **dbp) {
+    float *dwp = c.take<float>((size_t)B * K * Fin * Fout * sizeof(float), sizeof(float));
+    *dbp = c.take<float>((size_t)B * Fout * sizeof(float), sizeof(float));
+    return dwp;
 }
 
-static bool al16p(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// one buffer serves whichever kernel runs: the tensor-core layer (mesh_tc_bwd_workspace_bytes) or the FFMA one
+extern "C" size_t mvb_cheb_layer_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int has_up) {
+    WsCarve c;
+    float *dbp;
+    layer_bwd_ws(c, B, Fin, Fout, K, &dbp);
+    const size_t tc = mesh_tc_bwd_workspace_bytes(N, B, Fin, Fout, K, has_up);
+    return c.off > tc ? c.off : tc;
+}
 
 extern "C" int mvb_cheb_layer_fwd(int N, int B, int Fin, int Fout, int K, const int32_t *L_rowptr, const int32_t *L_colidx,
                                   const float *L_vals, int L_nnz, int n_in, const int32_t *U_rowptr, const int32_t *U_colidx,
@@ -559,7 +567,7 @@ extern "C" int mvb_cheb_layer_fwd(int N, int B, int Fin, int Fout, int K, const 
     MVB_REQUIRE(L_rowptr && x && weight && y, "cheb_layer_fwd: null pointer");
     MVB_REQUIRE(U_rowptr || n_in == N, "cheb_layer_fwd: n_in=%d != N=%d without an up-sampling operator", n_in, N);
     MVB_REQUIRE(sel || n_out == N, "cheb_layer_fwd: n_out=%d != N=%d without a row selection", n_out, N);
-    if (al16p(x) && al16p(weight) && al16p(y)) {
+    if (aligned16(x) && aligned16(weight) && aligned16(y)) {
         const int tc = launch_mesh_tc_fwd(N, B, Fin, Fout, K, L_rowptr, L_colidx, L_vals, L_nnz, n_in, U_rowptr, U_colidx, U_vals,
                                           n_out, sel, x, weight, bias, relu, y, (cudaStream_t)stream);
         if (tc != 0) return tc < 0 ? tc : MVB_OK;
@@ -568,9 +576,8 @@ extern "C" int mvb_cheb_layer_fwd(int N, int B, int Fin, int Fout, int K, const 
     int splits = 1;
     if (!layer_check(N, B, Fin, Fout, K, L_nnz, n_in, U_rowptr ? U_nnz : 0, n_out, false, &S, &splits))
         return set_err(MVB_EINVAL, "cheb_layer_fwd: shape N=%d Fin=%d Fout=%d K=%d not supported (see mvb_cheb_layer_supported)", N, Fin, Fout, K);
-    if (!al16p(x) || !al16p(weight) || !al16p(y)) return set_err(MVB_EALIGN, "cheb_layer_fwd: x / weight / y must be 16-byte aligned");
-    LayerArgs a;
-    memset(&a, 0, sizeof(a));
+    if (!aligned16(x) || !aligned16(weight) || !aligned16(y)) return set_err(MVB_EALIGN, "cheb_layer_fwd: x / weight / y must be 16-byte aligned");
+    LayerArgs a{};
     a.N = N; a.B = B; a.Fin = Fin; a.Fout = Fout; a.K = K;
     a.Lrp = L_rowptr; a.Lci = L_colidx; a.Lv = L_vals; a.Lnnz = L_nnz;
     a.n_in = n_in; a.Urp = U_rowptr; a.Uci = U_colidx; a.Uv = U_vals; a.Unnz = U_rowptr ? U_nnz : 0;
@@ -598,7 +605,7 @@ extern "C" int mvb_cheb_layer_bwd(int N, int B, int Fin, int Fout, int K, const 
     MVB_REQUIRE(U_rowptr || n_in == N, "cheb_layer_bwd: n_in != N without an up-sampling operator");
     MVB_REQUIRE(!U_rowptr || !dx || Ut_rowptr, "cheb_layer_bwd: dx requested without U^T");
     MVB_REQUIRE(sel || n_out == N, "cheb_layer_bwd: n_out != N without a row selection");
-    if (al16p(x) && al16p(weight) && al16p(dy) && (!y_for_relu || al16p(y_for_relu)) && (!dx || al16p(dx)) && al16p(workspace)) {
+    if (aligned16(x) && aligned16(weight) && aligned16(dy) && (!y_for_relu || aligned16(y_for_relu)) && (!dx || aligned16(dx)) && aligned16(workspace)) {
         const int tc = launch_mesh_tc_bwd(N, B, Fin, Fout, K, Lt_rowptr, Lt_colidx, Lt_vals, L_nnz, n_in, U_rowptr, U_colidx, U_vals,
                                           Ut_rowptr, Ut_colidx, Ut_vals, n_out, sel, x, weight, y_for_relu, dy, dx, dweight, dbias,
                                           workspace, workspace_bytes, (cudaStream_t)stream);
@@ -608,12 +615,13 @@ extern "C" int mvb_cheb_layer_bwd(int N, int B, int Fin, int Fout, int K, const 
     int splits = 1;
     if (!layer_check(N, B, Fin, Fout, K, L_nnz, n_in, U_rowptr ? U_nnz : 0, n_out, true, &S, &splits))
         return set_err(MVB_EINVAL, "cheb_layer_bwd: shape N=%d Fin=%d Fout=%d K=%d not supported", N, Fin, Fout, K);
-    if (!al16p(x) || !al16p(weight) || !al16p(dy) || (y_for_relu && !al16p(y_for_relu)) || (dx && !al16p(dx)))
+    if (!aligned16(x) || !aligned16(weight) || !aligned16(dy) || (y_for_relu && !aligned16(y_for_relu)) || (dx && !aligned16(dx)))
         return set_err(MVB_EALIGN, "cheb_layer_bwd: tensors must be 16-byte aligned");
-    const size_t need = ((size_t)B * K * Fin * Fout + (size_t)B * Fout) * sizeof(float);
-    if (workspace_bytes < need) return set_err(MVB_EWORKSPACE, "cheb_layer_bwd: workspace %zu < %zu", workspace_bytes, need);
-    LayerArgs a;
-    memset(&a, 0, sizeof(a));
+    WsCarve c{reinterpret_cast<char *>(workspace)};
+    float *dbp;
+    float *dwp = layer_bwd_ws(c, B, Fin, Fout, K, &dbp);
+    if (workspace_bytes < c.off) return set_err(MVB_EWORKSPACE, "cheb_layer_bwd: workspace %zu < %zu", workspace_bytes, c.off);
+    LayerArgs a{};
     a.N = N; a.B = B; a.Fin = Fin; a.Fout = Fout; a.K = K;
     a.Lrp = L_rowptr; a.Lci = L_colidx; a.Lv = L_vals; a.Lnnz = L_nnz;
     a.Ltrp = Lt_rowptr; a.Ltci = Lt_colidx; a.Ltv = Lt_vals;
@@ -621,8 +629,8 @@ extern "C" int mvb_cheb_layer_bwd(int N, int B, int Fin, int Fout, int K, const 
     a.Utrp = U_rowptr ? Ut_rowptr : nullptr; a.Utci = Ut_colidx; a.Utv = Ut_vals;
     a.n_out = n_out; a.sel = sel;
     a.x = x; a.w = weight; a.y = y_for_relu; a.dy = dy; a.relu = y_for_relu != nullptr; a.out = dx;
-    a.dwp = reinterpret_cast<float *>(workspace);
-    a.dbp = a.dwp + (size_t)B * K * Fin * Fout;
+    a.dwp = dwp;
+    a.dbp = dbp;
     a.splits = splits;
     static DevFlags optin;
     const size_t smem = (size_t)S.total * 4;

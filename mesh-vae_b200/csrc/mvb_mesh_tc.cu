@@ -722,8 +722,7 @@ static int launch_mesh_fwd_t(const MeshTcArgs &a, cudaStream_t st) {
     static DevFlags optin;
     int rc = smem_optin(cheb_mesh_tc_fwd_kernel<WL>, 227 * 1024, optin, "cheb_mesh_tc_fwd");
     if (rc) return rc;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
+    cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)(a.B * a.C));
     cfg.blockDim = dim3(MT_NT);
     cfg.dynamicSmemBytes = (size_t)a.total + 1024;
@@ -765,8 +764,7 @@ static int pick_mesh_c(MeshTcArgs &a, int width_in, int width_acc) {
 // 1 = the tensor-core mesh kernel covers this layer
 int mesh_tc_fwd_supported(int N, int B, int Fin, int Fout, int K, int Lnnz, int n_in, int n_out) {
     if (!g_mesh_tc || N < 1 || B < 1 || K < 1 || K > 16 || Lnnz < 0) return 0;
-    MeshTcArgs a;
-    memset(&a, 0, sizeof(a));
+    MeshTcArgs a{};
     a.N = N; a.B = B; a.Fin = Fin; a.Fout = Fout; a.K = K; a.Lnnz = Lnnz; a.n_in = n_in; a.n_out = n_out;
     return pick_mesh_c(a, Fin, Fout) ? 1 : 0;
 }
@@ -776,8 +774,7 @@ int launch_mesh_tc_fwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lr
                        int n_in, const int32_t *Urp, const int32_t *Uci, const float *Uv, int n_out, const int32_t *sel,
                        const float *x, const float *w, const float *bias, int relu, float *y, cudaStream_t st) {
     if (!g_mesh_tc || K > 16) return 0;
-    MeshTcArgs a;
-    memset(&a, 0, sizeof(a));
+    MeshTcArgs a{};
     a.N = N; a.B = B; a.Fin = Fin; a.Fout = Fout; a.K = K;
     a.Lrp = Lrp; a.Lci = Lci; a.Lv = Lv; a.Lnnz = Lnnz;
     a.n_in = n_in; a.Urp = Urp; a.Uci = Uci; a.Uv = Uv;
@@ -800,8 +797,7 @@ static int launch_mesh_bwd_t(const MeshTcBwdArgs &g, cudaStream_t st) {
     static DevFlags optin;
     int rc = smem_optin(cheb_mesh_tc_bwd_kernel<WL>, 227 * 1024, optin, "cheb_mesh_tc_bwd");
     if (rc) return rc;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
+    cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)(g.m.B * g.m.C));
     cfg.blockDim = dim3(MT_NT);
     cfg.dynamicSmemBytes = (size_t)g.m.total + 1024;
@@ -847,21 +843,39 @@ static int wgrad_group(int K, int Fout) {
 
 int mesh_tc_bwd_supported(int N, int B, int Fin, int Fout, int K, int Lnnz, int n_in, int n_out, int has_up) {
     if (!g_mesh_tc || N < 1 || B < 1 || K < 1 || K > 16 || Lnnz < 0 || (int64_t)N * B < 256) return 0;
-    MeshTcBwdArgs g;
-    memset(&g, 0, sizeof(g));
+    MeshTcBwdArgs g{};
     g.m.N = N; g.m.B = B; g.m.Fin = Fin; g.m.Fout = Fout; g.m.K = K; g.m.Lnnz = Lnnz; g.m.n_in = n_in; g.m.n_out = n_out;
     return pick_mesh_c_bwd(g, has_up) ? 1 : 0;
 }
 
-static size_t al256(size_t v) { return (v + 255) / 256 * 256; }
+// Workspace of the backward layer: S_0..S_{K-1}, T_0 (with up-sampling), the db partials, then the weight-gradient
+// partials of each plane group.  A launch has at most 16 groups (K <= 16); the size query measures any K.
+struct MeshBwdWs {
+    float *S, *T0, *dbp;
+    float *part[16];
+    size_t part_bytes[16];
+};
+static MeshBwdWs mesh_bwd_ws(WsCarve &c, int N, int B, int Fin, int Fout, int K, int has_up) {
+    MeshBwdWs w{};
+    w.S = c.take<float>((size_t)K * N * B * Fout * sizeof(float));
+    if (has_up) w.T0 = c.take<float>((size_t)N * B * Fin * sizeof(float));
+    w.dbp = c.take<float>((size_t)B * Fout * sizeof(float));
+    const int grp = wgrad_group(K, Fout);
+    for (int g = 0, k0 = 0; k0 < K; ++g, k0 += grp) {
+        const size_t bytes = align_up(wgrad_partial_bytes((K - k0 < grp ? K - k0 : grp) * Fout, Fin), 256);
+        float *p = c.take<float>(bytes);
+        if (g < 16) {
+            w.part[g] = p;
+            w.part_bytes[g] = bytes;
+        }
+    }
+    return w;
+}
 
 size_t mesh_tc_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int has_up) {
-    size_t bytes = al256((size_t)K * N * B * Fout * sizeof(float));              // S_0..S_{K-1}
-    if (has_up) bytes += al256((size_t)N * B * Fin * sizeof(float));             // T_0
-    bytes += al256((size_t)B * Fout * sizeof(float));                            // db partials
-    const int grp = wgrad_group(K, Fout);
-    for (int k0 = 0; k0 < K; k0 += grp) bytes += al256(wgrad_partial_bytes((K - k0 < grp ? K - k0 : grp) * Fout, Fin));
-    return bytes;
+    WsCarve c;
+    mesh_bwd_ws(c, N, B, Fin, Fout, K, has_up);
+    return c.off;
 }
 
 // returns 1 = handled, 0 = shape not covered, < 0 = error.  Lt*: CSR(L^T); U* / Ut*: CSR(U), CSR(U^T) or NULL
@@ -871,8 +885,7 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
                        const float *dy, float *dx, float *dweight, float *dbias, void *workspace, size_t workspace_bytes,
                        cudaStream_t st) {
     if (!g_mesh_tc || K > 16 || (int64_t)N * B < 256) return 0;
-    MeshTcBwdArgs g;
-    memset(&g, 0, sizeof(g));
+    MeshTcBwdArgs g{};
     MeshTcArgs &a = g.m;
     a.N = N; a.B = B; a.Fin = Fin; a.Fout = Fout; a.K = K;
     a.Lrp = Ltrp; a.Lci = Ltci; a.Lv = Ltv; a.Lnnz = Lnnz;
@@ -882,12 +895,12 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
     const int has_up = Urp != nullptr;
     const int c = pick_mesh_c_bwd(g, has_up);
     if (!c) return 0;
-    const size_t need = mesh_tc_bwd_workspace_bytes(N, B, Fin, Fout, K, has_up);
-    if (workspace_bytes < need) return set_err(MVB_EWORKSPACE, "cheb_layer_bwd: workspace %zu < %zu", workspace_bytes, need);
-    char *ws = reinterpret_cast<char *>(workspace);
-    g.S = reinterpret_cast<float *>(ws); ws += al256((size_t)K * N * B * Fout * sizeof(float));
-    if (has_up) { g.T0 = reinterpret_cast<float *>(ws); ws += al256((size_t)N * B * Fin * sizeof(float)); }
-    g.dbp = dbias ? reinterpret_cast<float *>(ws) : nullptr; ws += al256((size_t)B * Fout * sizeof(float));
+    WsCarve carve{reinterpret_cast<char *>(workspace)};
+    const MeshBwdWs ws = mesh_bwd_ws(carve, N, B, Fin, Fout, K, has_up);
+    if (workspace_bytes < carve.off) return set_err(MVB_EWORKSPACE, "cheb_layer_bwd: workspace %zu < %zu", workspace_bytes, carve.off);
+    g.S = ws.S;
+    g.T0 = ws.T0;
+    g.dbp = dbias ? ws.dbp : nullptr;
     g.Utrp = has_up ? Utrp : nullptr; g.Utci = Utci; g.Utv = Utv;
     g.dy = dy; g.y = y_for_relu;
     int rc;
@@ -898,16 +911,18 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
     }
     if (rc) return rc;
     // db and dW off the critical path: on the deferred side chain when the step engine has switched it on
-    cudaStream_t side = lazy_fork(st);
-    cudaStream_t ws_st = side ? side : st;
-    if (dbias) rc = launch_layer_finalize(B, 0, Fout, nullptr, g.dbp, nullptr, dbias, ws_st);
+    SideChain side(st, 0, false);
+    const cudaStream_t ws_st = side.stream();
+    if (dbias) {
+        rc = launch_layer_finalize(B, 0, Fout, nullptr, g.dbp, nullptr, dbias, ws_st);
+        if (rc) return rc;
+    }
     // dW_k[i][o] = sum_rows T_0[row][i] S_k[row][o]: streaming tensor-core reduction over all meshes, plane groups
     const int64_t rows = (int64_t)N * B;
     const int grp = wgrad_group(K, Fout);
-    for (int k0 = 0; k0 < K && !rc; k0 += grp) {
+    for (int gi = 0, k0 = 0; k0 < K; ++gi, k0 += grp) {
         const int np = K - k0 < grp ? K - k0 : grp;
-        WgradArgs wa;
-        memset(&wa, 0, sizeof(wa));
+        WgradArgs wa{};
         wa.rows = rows;
         wa.in_planes = np;
         wa.in_w = Fout;
@@ -915,17 +930,15 @@ int launch_mesh_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt
         wa.in_rest = g.S + (int64_t)(k0 + 1) * rows * Fout;
         wa.dy = has_up ? g.T0 : x;
         wa.n_out = Fin;
-        wa.partials = reinterpret_cast<float *>(ws);
-        wa.partial_bytes = al256(wgrad_partial_bytes(np * Fout, Fin));
-        ws += wa.partial_bytes;
+        wa.partials = ws.part[gi];
+        wa.partial_bytes = ws.part_bytes[gi];
         int nA = 0, m4A = 0;
         rc = launch_wgrad_partials(wa, 0, &nA, &m4A, ws_st);
-        if (!rc)
-            rc = launch_wgrad_finalize(wa.partials, nA, m4A, nullptr, 0, 0, Fin, np * Fin, Fout, dweight + (int64_t)k0 * Fin * Fout, nullptr,
-                                       ws_st, 1);
+        if (rc) return rc;
+        rc = launch_wgrad_finalize(wa.partials, nA, m4A, nullptr, 0, 0, Fin, np * Fin, Fout, dweight + (int64_t)k0 * Fin * Fout, nullptr,
+                                   ws_st, 1);
+        if (rc) return rc;
     }
-    lazy_done(side, st);          // on every path: a captured graph must not end forked
-    if (rc) return rc;
     return 1;
 }
 

@@ -337,8 +337,8 @@ static bool recur_shape(int N, int nnz, int64_t ncols, const void *a, const void
     return true;
 }
 
-// returns 1 = handled, 0 = shape not supported (caller runs the step-by-step SpMM), < 0 = error
-int launch_cheb_recur_fwd(int N, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
+// fused multi-step recurrences: 1 = handled, 0 = shape not supported (use the step kernels), < 0 = error
+static int launch_cheb_recur_fwd(int N, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
                           const float *x, float *basis, int64_t ncols, cudaStream_t st) {
     int cs4, nnz_smem;
     size_t smem;
@@ -361,7 +361,7 @@ int launch_cheb_recur_fwd(int N, int nnz, int K, const int32_t *rowptr, const in
     return rc ? rc : 1;
 }
 
-int launch_cheb_recur_bwd(int N, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
+static int launch_cheb_recur_bwd(int N, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
                           const float *P, float *dx, int64_t ncols, cudaStream_t st) {
     int cs4, nnz_smem;
     size_t smem;
@@ -382,6 +382,43 @@ int launch_cheb_recur_bwd(int N, int nnz, int K, const int32_t *rowptr_t, const 
     if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_recur_bwd: %s", cudaGetErrorString(e));
     int rc = check_launch("mvb cheb_recur_bwd");
     return rc ? rc : 1;
+}
+
+int launch_cheb_recurrence(int n, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
+                           const float *t0, float *planes, int64_t ncols, cudaStream_t st) {
+    if (K < 2) return MVB_OK;
+    const int fused = launch_cheb_recur_fwd(n, nnz, K, rowptr, colidx, vals, t0, planes, ncols, st);
+    if (fused) return fused < 0 ? fused : MVB_OK;
+    const int64_t plane = (int64_t)n * ncols;
+    for (int k = 1; k < K; ++k) {
+        float *tk = planes + (int64_t)(k - 1) * plane;
+        const float *tkm1 = (k == 1) ? t0 : planes + (int64_t)(k - 2) * plane;
+        const float *tkm2 = (k == 1) ? nullptr : (k == 2 ? t0 : planes + (int64_t)(k - 3) * plane);
+        const int rc = launch_spmm(n, n, rowptr, colidx, vals, tkm1, tk, tkm2, nullptr, k == 1 ? 1.f : 2.f, -1.f, ncols, st);
+        if (rc) return rc;
+    }
+    return MVB_OK;
+}
+
+int launch_cheb_recurrence_bwd(int n, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
+                               float *P, float *dx, int64_t ncols, cudaStream_t st) {
+    const int64_t plane = (int64_t)n * ncols;
+    if (K == 1) {
+        const cudaError_t e = cudaMemcpyAsync(dx, P, (size_t)plane * sizeof(float), cudaMemcpyDeviceToDevice, st);
+        if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_bwd: memcpy: %s", cudaGetErrorString(e));
+        return MVB_OK;
+    }
+    const int fused = launch_cheb_recur_bwd(n, nnz, K, rowptr_t, colidx_t, vals_t, P, dx, ncols, st);
+    if (fused) return fused < 0 ? fused : MVB_OK;
+    for (int k = K - 2; k >= 0; --k) {
+        float *pk = P + (int64_t)k * plane;
+        const float *gk1 = P + (int64_t)(k + 1) * plane;
+        const float *gk2 = (k + 2 <= K - 1) ? P + (int64_t)(k + 2) * plane : nullptr;
+        float *dst = (k == 0) ? dx : pk;
+        const int rc = launch_spmm(n, n, rowptr_t, colidx_t, vals_t, gk1, dst, gk2, pk, k == 0 ? 1.f : 2.f, -1.f, ncols, st);
+        if (rc) return rc;
+    }
+    return MVB_OK;
 }
 
 int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t *colidx, const float *vals,

@@ -409,8 +409,6 @@ void set_stream_tc(int v, int sw) {
     if (sw == 0 || sw == 8 || sw == 16) g_stream_sw = sw;
 }
 
-static size_t al256s(size_t v) { return (v + 255) / 256 * 256; }
-
 struct StreamPlan {
     int grid, SW, RP, nslabs, tiles_per_cta;
     size_t smem;
@@ -464,16 +462,33 @@ int stream_tc_supported(int N, int B, int Fin, int Fout, int K, int n_in, int ha
     return stream_plan(N, B, Fin, Fout, K, n_in, has_up, n_out, true, &pl) ? 1 : 0;
 }
 
-size_t stream_tc_fwd_workspace_bytes(int N, int B) { return 256 + 3 * (size_t)N * B * 16 * sizeof(float); }      // planes: multiples of 64 bytes
-
-size_t stream_tc_bwd_workspace_bytes(int N, int B, int K, int has_up) {
-    const size_t plane = (size_t)N * B * 16 * sizeof(float);       // a multiple of 64 bytes
-    size_t bytes = 256 + (size_t)K * plane;                        // S_0..S_{K-1} (contiguous: [K][N][B][16])
-    if (has_up) bytes += 2 * plane;                                // T_0, dT_0
-    bytes = al256s(bytes);
-    bytes += al256s((size_t)num_sms() * 16 * sizeof(float));       // db partials
-    bytes += al256s(wgrad_partial_bytes(K * 16, 16));
-    return bytes;
+// Workspaces: a 256-byte block of tile counters, then the [N][B][16] planes (multiples of 64 bytes, packed without
+// padding).  Forward: three planes.  Backward: S_0..S_{K-1}, with up-sampling T_0 and dT_0, then the db partials and
+// the weight-gradient partials.
+struct StreamWs {
+    unsigned int *ctr;
+    float *planes, *T0, *dT0, *dbp, *part;
+    size_t part_bytes;
+};
+static StreamWs stream_fwd_ws(WsCarve &c, int N, int B) {
+    StreamWs w{};
+    w.ctr = c.take<unsigned int>(256);
+    w.planes = c.take<float>(3 * (size_t)N * B * 16 * sizeof(float), 64);
+    return w;
+}
+static StreamWs stream_bwd_ws(WsCarve &c, int N, int B, int K, int has_up) {
+    const size_t plane = (size_t)N * B * 16 * sizeof(float);
+    StreamWs w{};
+    w.ctr = c.take<unsigned int>(256);
+    w.planes = c.take<float>((size_t)K * plane, 64);
+    if (has_up) {
+        w.T0 = c.take<float>(plane, 64);
+        w.dT0 = c.take<float>(plane, 64);
+    }
+    w.dbp = c.take<float>((size_t)num_sms() * 16 * sizeof(float));
+    w.part_bytes = align_up(wgrad_partial_bytes(K * 16, 16), 256);
+    w.part = c.take<float>(w.part_bytes);
+    return w;
 }
 
 template <bool BWD, int NT, int SW>
@@ -502,17 +517,16 @@ int launch_stream_tc_fwd(int N, int B, int Fin, int Fout, int K, const int32_t *
                          const float *w, const float *bias, int relu, float *y, void *workspace, size_t workspace_bytes, cudaStream_t st) {
     StreamPlan pl;
     if (sel || !stream_plan(N, B, Fin, Fout, K, n_in, Urp != nullptr, n_out, false, &pl)) return 0;
-    if (workspace_bytes < stream_tc_fwd_workspace_bytes(N, B))
-        return set_err(MVB_EWORKSPACE, "cheb_stream_fwd: workspace %zu < %zu", workspace_bytes, stream_tc_fwd_workspace_bytes(N, B));
-    StreamArgs a;
-    memset(&a, 0, sizeof(a));
+    WsCarve c{reinterpret_cast<char *>(workspace)};
+    const StreamWs ws = stream_fwd_ws(c, N, B);
+    if (workspace_bytes < c.off) return set_err(MVB_EWORKSPACE, "cheb_stream_fwd: workspace %zu < %zu", workspace_bytes, c.off);
+    StreamArgs a{};
     a.N = N; a.B = B; a.K = K; a.Nacc = Fout;
     a.Lrp = Lrp; a.Lci = Lci; a.Lv = Lv;
     a.n_in = n_in; a.Urp = Urp; a.Uci = Uci; a.Uv = Uv;
     a.x = x; a.w = w; a.bias = bias; a.relu = relu; a.out = y;
-    char *ws = reinterpret_cast<char *>(workspace);
-    a.ctr = reinterpret_cast<unsigned int *>(ws);
-    a.planes = reinterpret_cast<float *>(ws + 256);
+    a.ctr = ws.ctr;
+    a.planes = ws.planes;
     a.SW = pl.SW; a.RP = pl.RP; a.nslabs = pl.nslabs; a.tiles_per_cta = pl.tiles_per_cta;
     a.pairs = (int64_t)N * B;
     const int rc = launch_stream_t<false>(a, pl, st);
@@ -527,51 +541,46 @@ int launch_stream_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *
     StreamPlan pl;
     const int has_up = Urp != nullptr;
     if (sel || !stream_plan(N, B, Fin, Fout, K, n_in, has_up, n_out, true, &pl)) return 0;
-    const size_t need = stream_tc_bwd_workspace_bytes(N, B, K, has_up);
-    if (workspace_bytes < need) return set_err(MVB_EWORKSPACE, "cheb_stream_bwd: workspace %zu < %zu", workspace_bytes, need);
-    const size_t plane = (size_t)N * B * 16 * sizeof(float);
-    StreamArgs a;
-    memset(&a, 0, sizeof(a));
+    WsCarve c{reinterpret_cast<char *>(workspace)};
+    const StreamWs ws = stream_bwd_ws(c, N, B, K, has_up);
+    if (workspace_bytes < c.off) return set_err(MVB_EWORKSPACE, "cheb_stream_bwd: workspace %zu < %zu", workspace_bytes, c.off);
+    StreamArgs a{};
     a.N = N; a.B = B; a.K = K; a.Nacc = Fin;
     a.Lrp = Ltrp; a.Lci = Ltci; a.Lv = Ltv;
     a.n_in = n_in; a.Urp = Urp; a.Uci = Uci; a.Uv = Uv;
     a.Utrp = (has_up && dx) ? Utrp : nullptr; a.Utci = Utci; a.Utv = Utv;
     a.x = x; a.w = w; a.out = dx;
     a.dy = dy; a.y = y_for_relu;
-    char *ws = reinterpret_cast<char *>(workspace);
-    a.ctr = reinterpret_cast<unsigned int *>(ws); ws += 256;
-    a.planes = reinterpret_cast<float *>(ws); ws += (size_t)K * plane;
-    if (has_up) {
-        a.T0 = reinterpret_cast<float *>(ws); ws += plane;
-        a.dT0 = reinterpret_cast<float *>(ws); ws += plane;
-    }
-    ws = reinterpret_cast<char *>(workspace) + al256s((size_t)(ws - reinterpret_cast<char *>(workspace)));
-    a.dbp = dbias ? reinterpret_cast<float *>(ws) : nullptr; ws += al256s((size_t)num_sms() * 16 * sizeof(float));
+    a.ctr = ws.ctr;
+    a.planes = ws.planes;
+    a.T0 = ws.T0;
+    a.dT0 = ws.dT0;
+    a.dbp = dbias ? ws.dbp : nullptr;
     a.SW = pl.SW; a.RP = pl.RP; a.nslabs = pl.nslabs; a.tiles_per_cta = pl.tiles_per_cta;
     a.pairs = (int64_t)N * B;
     int rc = launch_stream_t<true>(a, pl, st);
     if (rc) return rc;
     // db and dW off the critical path (deferred side chain when the step engine has switched it on)
-    cudaStream_t side = lazy_fork(st);
-    cudaStream_t ws_st = side ? side : st;
-    if (dbias) rc = launch_layer_finalize(pl.grid, 0, 16, nullptr, a.dbp, nullptr, dbias, ws_st);
-    if (!rc) {
-        WgradArgs wa;
-        memset(&wa, 0, sizeof(wa));
-        wa.rows = (int64_t)N * B;
-        wa.in_planes = K;
-        wa.in_w = 16;
-        wa.in0 = a.planes;
-        wa.in_rest = a.planes + (int64_t)N * B * 16;
-        wa.dy = has_up ? a.T0 : x;
-        wa.n_out = Fin;
-        wa.partials = reinterpret_cast<float *>(ws);
-        wa.partial_bytes = al256s(wgrad_partial_bytes(K * 16, 16));
-        int nA = 0, m4A = 0;
-        rc = launch_wgrad_partials(wa, 0, &nA, &m4A, ws_st);
-        if (!rc) rc = launch_wgrad_finalize(wa.partials, nA, m4A, nullptr, 0, 0, Fin, K * Fin, Fout, dweight, nullptr, ws_st, 1);
+    SideChain side(st, 0, false);
+    const cudaStream_t ws_st = side.stream();
+    if (dbias) {
+        rc = launch_layer_finalize(pl.grid, 0, 16, nullptr, a.dbp, nullptr, dbias, ws_st);
+        if (rc) return rc;
     }
-    lazy_done(side, st);
+    WgradArgs wa{};
+    wa.rows = (int64_t)N * B;
+    wa.in_planes = K;
+    wa.in_w = 16;
+    wa.in0 = a.planes;
+    wa.in_rest = a.planes + (int64_t)N * B * 16;
+    wa.dy = has_up ? a.T0 : x;
+    wa.n_out = Fin;
+    wa.partials = ws.part;
+    wa.partial_bytes = ws.part_bytes;
+    int nA = 0, m4A = 0;
+    rc = launch_wgrad_partials(wa, 0, &nA, &m4A, ws_st);
+    if (rc) return rc;
+    rc = launch_wgrad_finalize(wa.partials, nA, m4A, nullptr, 0, 0, Fin, K * Fin, Fout, dweight, nullptr, ws_st, 1);
     if (rc) return rc;
     return 1;
 }
@@ -581,15 +590,15 @@ int launch_stream_tc_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *
 // ---------------------------------------------------------------------------------------------
 // C ABI (include/mvb.h)
 // ---------------------------------------------------------------------------------------------
-static bool st_al16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 extern "C" int mvb_cheb_stream_supported(int N, int B, int Fin, int Fout, int K, int n_in, int has_up, int n_out) {
     return mvb::stream_tc_supported(N, B, Fin, Fout, K, n_in, has_up, n_out);
 }
 
 extern "C" size_t mvb_cheb_stream_fwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int has_up) {
     (void)Fin; (void)Fout; (void)K; (void)has_up;
-    return mvb::stream_tc_fwd_workspace_bytes(N, B);
+    mvb::WsCarve c;
+    mvb::stream_fwd_ws(c, N, B);
+    return c.off;
 }
 
 extern "C" int mvb_cheb_stream_fwd(int N, int B, int Fin, int Fout, int K, const int32_t *L_rowptr, const int32_t *L_colidx,
@@ -599,7 +608,7 @@ extern "C" int mvb_cheb_stream_fwd(int N, int B, int Fin, int Fout, int K, const
     (void)L_nnz; (void)U_nnz;
     MVB_REQUIRE(L_rowptr && L_colidx && L_vals && x && weight && y && workspace, "cheb_stream_fwd: null pointer");
     MVB_REQUIRE(U_rowptr || n_in == N, "cheb_stream_fwd: n_in=%d != N=%d without an up-sampling operator", n_in, N);
-    if (!st_al16(x) || !st_al16(y) || !st_al16(workspace)) return mvb::set_err(MVB_EALIGN, "cheb_stream_fwd: x / y / workspace must be 16-byte aligned");
+    if (!mvb::aligned16(x) || !mvb::aligned16(y) || !mvb::aligned16(workspace)) return mvb::set_err(MVB_EALIGN, "cheb_stream_fwd: x / y / workspace must be 16-byte aligned");
     const int rc = mvb::launch_stream_tc_fwd(N, B, Fin, Fout, K, L_rowptr, L_colidx, L_vals, n_in, U_rowptr, U_colidx, U_vals, N, nullptr, x,
                                              weight, bias, relu, y, workspace, workspace_bytes, (cudaStream_t)stream);
     if (rc < 0) return rc;
@@ -609,7 +618,9 @@ extern "C" int mvb_cheb_stream_fwd(int N, int B, int Fin, int Fout, int K, const
 
 extern "C" size_t mvb_cheb_stream_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int has_up) {
     (void)Fin; (void)Fout;
-    return mvb::stream_tc_bwd_workspace_bytes(N, B, K, has_up);
+    mvb::WsCarve c;
+    mvb::stream_bwd_ws(c, N, B, K, has_up);
+    return c.off;
 }
 
 extern "C" int mvb_cheb_stream_bwd(int N, int B, int Fin, int Fout, int K, const int32_t *Lt_rowptr, const int32_t *Lt_colidx,
@@ -621,7 +632,7 @@ extern "C" int mvb_cheb_stream_bwd(int N, int B, int Fin, int Fout, int K, const
     MVB_REQUIRE(Lt_rowptr && Lt_colidx && Lt_vals && x && weight && dy && dweight && workspace, "cheb_stream_bwd: null pointer");
     MVB_REQUIRE(U_rowptr || n_in == N, "cheb_stream_bwd: n_in != N without an up-sampling operator");
     MVB_REQUIRE(!U_rowptr || !dx || Ut_rowptr, "cheb_stream_bwd: dx requested without U^T");
-    if (!st_al16(x) || !st_al16(dy) || (y_for_relu && !st_al16(y_for_relu)) || (dx && !st_al16(dx)) || !st_al16(workspace))
+    if (!mvb::aligned16(x) || !mvb::aligned16(dy) || (y_for_relu && !mvb::aligned16(y_for_relu)) || (dx && !mvb::aligned16(dx)) || !mvb::aligned16(workspace))
         return mvb::set_err(MVB_EALIGN, "cheb_stream_bwd: tensors must be 16-byte aligned");
     const int rc = mvb::launch_stream_tc_bwd(N, B, Fin, Fout, K, Lt_rowptr, Lt_colidx, Lt_vals, n_in, U_rowptr, U_colidx, U_vals, Ut_rowptr,
                                              Ut_colidx, Ut_vals, N, nullptr, x, weight, y_for_relu, dy, dx, dweight, dbias, workspace,

@@ -28,12 +28,32 @@ def _sink(t):
     return None if t is None else getattr(t, "_mvb_grad_sink", None)
 
 
-def _grad_out(sink, like):
-    return sink if sink is not None else torch.empty_like(like)
+def _grad_outs(sinks, w, n_bias):
+    """(dw, db) for a backward kernel to write: the Parameters' gradient sinks where installed, else new tensors;
+    db is None when n_bias is None (no bias)"""
+    sw, sb = sinks
+    dw = sw if sw is not None else torch.empty_like(w)
+    if n_bias is None:
+        return dw, None
+    return dw, (sb if sb is not None else torch.empty(n_bias, device=w.device, dtype=torch.float32))
 
 
-def _ret(sink, g):
-    return None if sink is not None else g
+def _park_or_join(ctx, tensors):
+    """deferred mode: park the tensors a backward call's pending side chain still reads or writes until side_join, or
+    join now when a gradient goes back to autograd (it must be complete on this stream) instead of into a sink"""
+    if not _lib._deferred["on"]:
+        return
+    sw, sb = ctx.sinks
+    if sw is not None and (sb is not None or not ctx.has_bias):
+        _lib._deferred["keep"].append(tensors)
+    else:
+        _lib.side_join()
+
+
+def _ret(sinks, dw, db):
+    """backward's return values for (weight, bias): None for a gradient that went into its sink"""
+    sw, sb = sinks
+    return (None if sw is not None else dw), (None if sb is not None else db)
 
 
 def to_vertex_major(x: torch.Tensor) -> torch.Tensor:
@@ -86,9 +106,7 @@ class _ChebConvFn(torch.autograd.Function):
         dy = dy.contiguous()
         need_dx = ctx.needs_input_grad[0]
         dx = torch.empty_like(x_vm) if need_dx else None
-        sw, sb = ctx.sinks
-        dw = _grad_out(sw, w)
-        db = (sb if sb is not None else torch.empty(fout, device=w.device, dtype=torch.float32)) if ctx.has_bias else None
+        dw, db = _grad_outs(ctx.sinks, w, fout if ctx.has_bias else None)
         na = op.n_active
         ws_bytes = lib.mvb_cheb_bwd_workspace_bytes(n, b, fin, fout, k, na, 1 if need_dx else 0)
         ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
@@ -96,12 +114,8 @@ class _ChebConvFn(torch.autograd.Function):
                                ptr(basis) if (basis is not None and basis.numel()) else None, ptr(w), ptr(y) if ctx.relu else None,
                                ptr(dy), ptr(dx),
                                ptr(dw), ptr(db), ptr(ws), ws_bytes, stream_ptr()), "mvb_cheb_bwd")
-        if _lib._deferred["on"]:
-            if sw is not None and (sb is not None or not ctx.has_bias):
-                _lib._deferred["keep"].append((ws, x_vm, basis, w, y, dy, dw, db))      # read / written by the pending side chain
-            else:
-                _lib.side_join()
-        return dx, _ret(sw, dw), _ret(sb, db), None, None
+        _park_or_join(ctx, (ws, x_vm, basis, w, y, dy, dw, db))
+        return dx, *_ret(ctx.sinks, dw, db), None, None
 
 
 def cheb_conv(x_vm: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], op: MeshOperator,
@@ -158,15 +172,13 @@ class _ChebConvSelFn(torch.autograd.Function):
         n, b, fin = x_vm.shape
         k, _, fout = w.shape
         dy = dy.contiguous()
-        sw, sb = ctx.sinks
-        dw = _grad_out(sw, w)
-        db = (sb if sb is not None else torch.empty(fout, device=w.device, dtype=torch.float32)) if ctx.has_bias else None
+        dw, db = _grad_outs(ctx.sinks, w, fout if ctx.has_bias else None)
         ws_bytes = lib.mvb_cheb_sel_bwd_workspace_bytes(fin, fout, k)
         ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
         check(lib.mvb_cheb_sel_bwd(n, b, fin, fout, k, ptr(x_vm), ptr(basis) if basis.numel() else None, ptr(y) if ctx.relu else None,
                                    ptr(dy), ctx.d_op.n_rows, ptr(ctx.d_op.colidx), ptr(dw), ptr(db), ptr(ws), ws_bytes, stream_ptr()),
               "mvb_cheb_sel_bwd")
-        return None, _ret(sw, dw), _ret(sb, db), None, None, None
+        return None, *_ret(ctx.sinks, dw, db), None, None, None
 
 
 def cheb_conv_sel_supported(x_vm: torch.Tensor, weight: torch.Tensor, op: MeshOperator, d_op: Optional[MeshOperator]) -> bool:
@@ -453,17 +465,12 @@ class _LinearFn(torch.autograd.Function):
         m, k, n, x_vm_f, y_vm_f, relu, p = ctx.dims
         gy = gy.contiguous()
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-        sw, sb = ctx.sinks
-        dw = _grad_out(sw, w)
-        db = (sb if sb is not None else torch.empty(n, device=w.device, dtype=torch.float32)) if ctx.has_bias else None
+        dw, db = _grad_outs(ctx.sinks, w, n if ctx.has_bias else None)
         check(lib.mvb_linear_bwd(m, k, n, ptr(x), x_vm_f, ptr(w), ptr(y), ptr(gy), y_vm_f, 1 if relu else 0, p, ptr(dx), ptr(dw),
                                  ptr(db), stream_ptr()), "mvb_linear_bwd")
-        if _lib._deferred["on"] and dx is not None:
-            if sw is not None and (sb is not None or not ctx.has_bias):
-                _lib._deferred["keep"].append((x, w, y, gy, dw, db))        # the dW / db tiles may still be running on the side chain
-            else:
-                _lib.side_join()
-        return dx, _ret(sw, dw), _ret(sb, db), None, None, None, None, None
+        if dx is not None:          # without dx there is no split launch and nothing on the side chain
+            _park_or_join(ctx, (x, w, y, gy, dw, db))
+        return dx, *_ret(ctx.sinks, dw, db), None, None, None, None, None
 
 
 def linear(x, weight, bias=None, relu: bool = False, p: float = 0.0, rng=_NO_RNG, x_vm: bool = False, y_vm_f: int = 0):
@@ -511,19 +518,16 @@ class _VaeHeadsFn(torch.autograd.Function):
         h, y_onehot, eps, wc, wm, wv, y_hat, logvar = ctx.saved_tensors
         b, hd, z, c, p, seed, off_dev, off_host = ctx.cfg
         gs = [None if g is None else g.contiguous() for g in (g_yhat, g_mu, g_logvar, g_z, g_zcat)]
-        dev = h.device
         g_h = torch.empty_like(h)
         sk = ctx.sinks
-        dwc, dwm, dwv = _grad_out(sk[0], wc), _grad_out(sk[2], wm), _grad_out(sk[4], wv)
-        dbc = sk[1] if sk[1] is not None else torch.empty(c, device=dev, dtype=torch.float32)
-        dbm = sk[3] if sk[3] is not None else torch.empty(z, device=dev, dtype=torch.float32)
-        dbv = sk[5] if sk[5] is not None else torch.empty(z, device=dev, dtype=torch.float32)
+        dwc, dbc = _grad_outs(sk[0:2], wc, c)
+        dwm, dbm = _grad_outs(sk[2:4], wm, z)
+        dwv, dbv = _grad_outs(sk[4:6], wv, z)
         check(lib.mvb_vae_heads_bwd(b, hd, z, c, ptr(h), ptr(y_onehot), ptr(eps), ptr(wc), ptr(wm), ptr(wv), ptr(y_hat),
                                     ptr(logvar), p, seed, ptr(off_dev), off_host, ptr(gs[0]), ptr(gs[1]), ptr(gs[2]), ptr(gs[3]),
                                     ptr(gs[4]), ptr(g_h), ptr(dwc), ptr(dbc), ptr(dwm), ptr(dbm), ptr(dwv), ptr(dbv),
                                     stream_ptr()), "mvb_vae_heads_bwd")
-        return (g_h, None, None, _ret(sk[0], dwc), _ret(sk[1], dbc), _ret(sk[2], dwm), _ret(sk[3], dbm), _ret(sk[4], dwv),
-                _ret(sk[5], dbv), None, None)
+        return (g_h, None, None, *_ret(sk[0:2], dwc, dbc), *_ret(sk[2:4], dwm, dbm), *_ret(sk[4:6], dwv, dbv), None, None)
 
 
 def vae_heads(h, y_onehot, eps, classifier, z_mean, z_log_var, p: float = 0.0, rng=_NO_RNG):
@@ -549,17 +553,23 @@ def vae_heads(h, y_onehot, eps, classifier, z_mean, z_log_var, p: float = 0.0, r
 # ---------------------------------------------------------------------------------------------
 # mesh-resident fused layers for the coarse levels (models/cheb_VAE.py:264-265, 284-285)
 # ---------------------------------------------------------------------------------------------
-def cheb_layer_supported(n: int, b: int, fin: int, fout: int, k: int, l_op: MeshOperator, u_op: Optional[MeshOperator],
-                         d_op: Optional[MeshOperator]) -> bool:
+def _fused_layer_kind(n: int, b: int, fin: int, fout: int, k: int, l_op: MeshOperator, u_op: Optional[MeshOperator],
+                      d_op: Optional[MeshOperator]) -> Optional[str]:
+    """"mesh" (the mesh-resident kernels), "stream" (the row-streaming kernels) or None (neither covers the layer)"""
     if l_op.n_active != n or l_op.n_rows != n:
-        return False
+        return None
     if d_op is not None and not d_op.is_selection:
-        return False
+        return None
     n_in = u_op.n_cols if u_op is not None else n
     n_out = d_op.n_rows if d_op is not None else n
     if lib.mvb_cheb_layer_supported(n, b, fin, fout, k, l_op.nnz, n_in, u_op.nnz if u_op is not None else 0, n_out):
-        return True
-    return cheb_stream_supported(n, b, fin, fout, k, l_op, u_op, d_op)
+        return "mesh"
+    return "stream" if cheb_stream_supported(n, b, fin, fout, k, l_op, u_op, d_op) else None
+
+
+def cheb_layer_supported(n: int, b: int, fin: int, fout: int, k: int, l_op: MeshOperator, u_op: Optional[MeshOperator],
+                         d_op: Optional[MeshOperator]) -> bool:
+    return _fused_layer_kind(n, b, fin, fout, k, l_op, u_op, d_op) is not None
 
 
 def cheb_stream_supported(n: int, b: int, fin: int, fout: int, k: int, l_op: MeshOperator, u_op: Optional[MeshOperator],
@@ -612,9 +622,7 @@ class _ChebLayerFn(torch.autograd.Function):
         n_out = d_op.n_rows if d_op is not None else n
         dy = dy.contiguous()
         dx = torch.empty_like(x_vm) if ctx.needs_input_grad[0] else None
-        sw, sb = ctx.sinks
-        dw = _grad_out(sw, w)
-        db = (sb if sb is not None else torch.empty(fout, device=w.device, dtype=torch.float32)) if ctx.has_bias else None
+        dw, db = _grad_outs(ctx.sinks, w, fout if ctx.has_bias else None)
         ws_bytes = lib.mvb_cheb_layer_bwd_workspace_bytes(n, b, fin, fout, k, 1 if u is not None else 0)
         ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
         check(lib.mvb_cheb_layer_bwd(n, b, fin, fout, k, ptr(l_op.rowptr), ptr(l_op.colidx), ptr(l_op.vals), ptr(l_op.rowptr_t),
@@ -624,13 +632,8 @@ class _ChebLayerFn(torch.autograd.Function):
                                      u.nnz if u else 0, n_out, ptr(d_op.colidx) if d_op is not None else None, ptr(x_vm), ptr(w),
                                      ptr(y) if ctx.relu else None, ptr(dy), ptr(dx), ptr(dw), ptr(db), ptr(ws), ws_bytes,
                                      stream_ptr()), "mvb_cheb_layer_bwd")
-        if _lib._deferred["on"]:
-            if sw is not None and (sb is not None or not ctx.has_bias):
-                # the weight-gradient chain may still be running on the side stream: it reads ws / x and writes the sinks
-                _lib._deferred["keep"].append((ws, x_vm, w, dy, dw, db))
-            else:
-                _lib.side_join()          # gradients handed back to autograd must be complete on this stream
-        return dx, _ret(sw, dw), _ret(sb, db), None, None, None, None
+        _park_or_join(ctx, (ws, x_vm, w, dy, dw, db))
+        return dx, *_ret(ctx.sinks, dw, db), None, None, None, None
 
 
 class _ChebStreamFn(torch.autograd.Function):
@@ -674,9 +677,7 @@ class _ChebStreamFn(torch.autograd.Function):
         n = l_op.n_rows
         dy = dy.contiguous()
         dx = torch.empty_like(x_vm) if ctx.needs_input_grad[0] else None
-        sw, sb = ctx.sinks
-        dw = _grad_out(sw, w)
-        db = (sb if sb is not None else torch.empty(fout, device=w.device, dtype=torch.float32)) if ctx.has_bias else None
+        dw, db = _grad_outs(ctx.sinks, w, fout if ctx.has_bias else None)
         ws_bytes = lib.mvb_cheb_stream_bwd_workspace_bytes(n, b, fin, fout, k, 1 if u is not None else 0)
         ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
         check(lib.mvb_cheb_stream_bwd(n, b, fin, fout, k, ptr(l_op.rowptr_t), ptr(l_op.colidx_t), ptr(l_op.vals_t), l_op.nnz, n_in,
@@ -684,34 +685,37 @@ class _ChebStreamFn(torch.autograd.Function):
                                       ptr(u.rowptr_t) if u else None, ptr(u.colidx_t) if u else None, ptr(u.vals_t) if u else None,
                                       u.nnz if u else 0, ptr(x_vm), ptr(w), ptr(y) if ctx.relu else None, ptr(dy), ptr(dx), ptr(dw),
                                       ptr(db), ptr(ws), ws_bytes, stream_ptr()), "mvb_cheb_stream_bwd")
-        if _lib._deferred["on"]:
-            if sw is not None and (sb is not None or not ctx.has_bias):
-                _lib._deferred["keep"].append((ws, x_vm, w, dy, dw, db))      # the side chain still reads ws / x and writes the sinks
-            else:
-                _lib.side_join()
-        return dx, _ret(sw, dw), _ret(sb, db), None, None, None
+        _park_or_join(ctx, (ws, x_vm, w, dy, dw, db))
+        return dx, *_ret(ctx.sinks, dw, db), None, None, None
+
+
+def cheb_layer_fused(x_vm, weight, bias, l_op: MeshOperator, u_op: Optional[MeshOperator] = None,
+                     d_op: Optional[MeshOperator] = None, relu: bool = True) -> Optional[torch.Tensor]:
+    """cheb_layer as one fused kernel per direction - the mesh-resident kernels when the level fits shared memory, else
+    the row-streaming kernels - or None when neither covers the layer"""
+    if not x_vm.is_cuda:
+        return None
+    kind = _fused_layer_kind(l_op.n_rows, x_vm.shape[1], x_vm.shape[2], weight.shape[2], weight.shape[0], l_op, u_op, d_op)
+    if kind == "mesh":
+        return _ChebLayerFn.apply(x_vm, weight, bias, l_op, u_op, d_op, relu)
+    if kind == "stream":
+        return _ChebStreamFn.apply(x_vm, weight, bias, l_op, u_op, relu)
+    return None
 
 
 def cheb_layer(x_vm, weight, bias, l_op: MeshOperator, u_op: Optional[MeshOperator] = None,
                d_op: Optional[MeshOperator] = None, relu: bool = True):
     """[U prologue] -> Chebyshev conv (+bias, ReLU) -> [D row selection] on vertex-major tensors: the fused
-    one-launch kernel when the level fits shared memory (cheb_layer_supported), else the composition of
-    pool / cheb_conv / pool."""
-    n = l_op.n_rows
-    b, fin = x_vm.shape[1], x_vm.shape[2]
-    k, _, fout = weight.shape
-    if x_vm.is_cuda and cheb_layer_supported(n, b, fin, fout, k, l_op, u_op, d_op):
-        if cheb_stream_supported(n, b, fin, fout, k, l_op, u_op, d_op) and not lib.mvb_cheb_layer_supported(
-                n, b, fin, fout, k, l_op.nnz, x_vm.shape[0], u_op.nnz if u_op is not None else 0, n):
-            return _ChebStreamFn.apply(x_vm, weight, bias, l_op, u_op, relu)
-        return _ChebLayerFn.apply(x_vm, weight, bias, l_op, u_op, d_op, relu)
+    kernels when they cover the level (cheb_layer_fused), else the composition of pool / cheb_conv / pool."""
+    y = cheb_layer_fused(x_vm, weight, bias, l_op, u_op, d_op, relu)
+    if y is not None:
+        return y
     if u_op is not None:
         x_vm = pool(x_vm, u_op)
     y = cheb_conv(x_vm, weight, bias, l_op, relu)
     if d_op is not None:
         y = pool(y, d_op)
     return y
-
 
 
 def recon_error(recon, mean, std, s, R, m, gt_mesh, per_vertex: bool = False, mesh: bool = False):
