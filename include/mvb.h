@@ -385,10 +385,16 @@ int mvb_linear_bwd(int M, int K, int N, const float *x, int x_vm_f, const float 
  *   mu, logvar [B,Z] = cat(y, h) Wm^T + bm, cat(y, h) Wv^T + bv     :206-212  (Wm, Wv: [Z, C+H])
  *   z [B,Z]      = mu + eps * exp(logvar/2), or mu when eps == NULL  :215-221, :309-319
  *   zcat [B,C+Z] = cat(y, z)                                         :223
- *   y_onehot [B,C] int64 (main.py:71).  The classifier's dropout is the SECOND mask on h (quirk 8).
+ *   y_onehot [B,C] int64 (main.py:71).  The classifier's dropout is the SECOND mask on h (quirk 8):
+ *   a Philox4x32-10 mask keyed by (seed, offset, b*H + j), b the row within the call, offset as for
+ *   mvb_linear_fwd - so the first rows of a large call get the mask of a smaller call.
+ *   Shapes: any B, H, Z >= 1, C <= 32 (the softmax is one warp's), B*H < 2^32 (the mask counter).
+ *   One-launch kernels where the C + 2Z weight rows (forward) or the batch's small gradients
+ *   (backward) fit one block's shared memory (at H = 512, Z = 16, C = 2: any B forward, B <= 278
+ *   backward), tiled kernels elsewhere; both sum in the same order, so the results are the same bits.
  * mvb_vae_heads_bwd: from the upstream gradients of the five outputs (any may be NULL = zero) to
  *   g_h [B,H] and the six parameter gradients (OVERWRITTEN); same (p_drop, seed, offset) as the
- *   forward call so that the mask is regenerated, not stored. */
+ *   forward call so that the mask is regenerated, not stored.  No workspace, no atomics. */
 int mvb_vae_heads_fwd(int B, int H, int Z, int C, const float *h, const int64_t *y_onehot, const float *eps,
                       const float *Wc, const float *bc, const float *Wm, const float *bm, const float *Wv,
                       const float *bv, float p_drop, uint64_t seed, const int64_t *offset_dev,

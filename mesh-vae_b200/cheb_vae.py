@@ -136,12 +136,8 @@ class cheb_VAE(nn.Module):
         if self.fused_dense and x.is_cuda and not x.requires_grad and not (self.training and self.dropout.p > 0):
             # inference.py:88 / main.py:42-49 (classifier_): softmax(classifier_layer(x)) from the heads kernel
             # (its other outputs are discarded); no cuBLAS / ATen launch on the forward-only path
-            outs = []
-            for i in range(0, x.shape[0], Fn.VAE_HEADS_MAX_BATCH):
-                xi = x[i:i + Fn.VAE_HEADS_MAX_BATCH]
-                y0 = torch.zeros((xi.shape[0], self.num_class), device=x.device, dtype=torch.int64)
-                outs.append(Fn.vae_heads(xi, y0, None, self.classifier_layer, self.z_mean, self.z_log_var)[0])
-            return outs[0] if len(outs) == 1 else torch.cat(outs, 0)
+            y0 = torch.zeros((x.shape[0], self.num_class), device=x.device, dtype=torch.int64)
+            return Fn.vae_heads(x, y0, None, self.classifier_layer, self.z_mean, self.z_log_var)[0]
         return F.softmax(self.classifier_layer(self.dropout(x)), dim=1)
 
     def decoder(self, z):

@@ -539,6 +539,215 @@ vae_heads_bwd_kernel(int B, int H, int Z, int C, const float *__restrict__ h, co
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// The heads at any B, H and Z (C <= 32).  The one-launch kernels above stage all C + 2Z weight rows (forward) or the
+// whole batch's small gradients (backward) in one block's shared memory, which bounds H, Z and B.  These kernels
+// tile instead, and keep the summation order of the one-launch kernels, so a mesh's results are bit-identical
+// whichever pair computed them.
+//   forward: a block is HT_MESH meshes (a warp each) x one output tile: tile 0 holds the C classifier logits (the
+//   softmax stays in the epilogue), tile t >= 1 holds mu and logvar of the latents [16 (t-1), 16 t) (the
+//   reparameterisation and zcat stay in the epilogue).  The C + H inputs stream through shared memory in chunks of
+//   HT_KC columns; lane l sums the columns j = l (mod 32) in ascending order, then warp_sum - the order of
+//   vae_heads_fwd_kernel.
+// ---------------------------------------------------------------------------------------------
+constexpr int HT_MESH = 8, HT_OUT = 32, HT_ZT = HT_OUT / 2, HT_KC = 128, HT_BC = 32;
+
+__global__ void __launch_bounds__(256)
+vae_heads_fwd_tiled_kernel(int B, int H, int Z, int C, const float *__restrict__ h, const int64_t *__restrict__ yoh,
+                           const float *__restrict__ eps, const float *__restrict__ Wc, const float *__restrict__ bc,
+                           const float *__restrict__ Wm, const float *__restrict__ bm, const float *__restrict__ Wv,
+                           const float *__restrict__ bv, float p, uint64_t seed, const int64_t *off_dev, int64_t off_host,
+                           float *__restrict__ y_hat, float *__restrict__ mu, float *__restrict__ logvar,
+                           float *__restrict__ z_, float *__restrict__ zcat) {
+    pdl_trigger();
+    pdl_wait();
+    __shared__ float xs[HT_MESH][HT_KC];          // inputs: cat(y, h) rows, or (0, dropout(h)) for the classifier tile
+    __shared__ float ws[HT_OUT][HT_KC];           // weight rows of the tile's outputs (zero past the valid ones)
+    __shared__ float outs[HT_MESH][HT_OUT];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int b0 = blockIdx.x * HT_MESH;
+    const bool cls = blockIdx.y == 0;
+    const int z0 = ((int)blockIdx.y - 1) * HT_ZT;
+    const int K = C + H;
+    const uint64_t off = (uint64_t)(off_host + (off_dev ? *off_dev : 0));
+    const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
+    float acc[HT_OUT];
+#pragma unroll
+    for (int o = 0; o < HT_OUT; ++o) acc[o] = 0.f;
+    for (int k0 = 0; k0 < K; k0 += HT_KC) {
+        if (k0) __syncthreads();
+        for (int i = tid; i < HT_MESH * HT_KC; i += 256) {
+            const int r = i / HT_KC, jj = i % HT_KC, j = k0 + jj, b = b0 + r;
+            float v = 0.f;
+            if (b < B && j < K) {
+                if (j < C) v = cls ? 0.f : (float)yoh[(int64_t)b * C + j];
+                else {
+                    v = __ldg(h + (int64_t)b * H + j - C);
+                    if (cls && p > 0.f) v = drop_keep(seed, off, (uint32_t)b * (uint32_t)H + (uint32_t)(j - C), p) ? v * scale : 0.f;
+                }
+            }
+            xs[r][jj] = v;
+        }
+        for (int i = tid; i < HT_OUT * HT_KC; i += 256) {
+            const int o = i / HT_KC, jj = i % HT_KC, j = k0 + jj;
+            float w = 0.f;
+            if (j < K) {
+                if (cls) {
+                    if (o < C && j >= C) w = __ldg(Wc + (int64_t)o * H + j - C);
+                } else {
+                    const int zi = z0 + o % HT_ZT;
+                    if (zi < Z) w = __ldg((o < HT_ZT ? Wm : Wv) + (int64_t)zi * K + j);
+                }
+            }
+            ws[o][jj] = w;
+        }
+        __syncthreads();
+        const int kc = min(HT_KC, K - k0);
+        for (int jj = lane; jj < kc; jj += 32) {
+            const float x = xs[warp][jj];
+#pragma unroll
+            for (int o = 0; o < HT_OUT; ++o) acc[o] = fmaf(x, ws[o][jj], acc[o]);
+        }
+    }
+    float s = 0.f;                                 // lane o: output o of the tile for mesh b0 + warp
+#pragma unroll
+    for (int o = 0; o < HT_OUT; ++o) {
+        const float t = warp_sum(acc[o]);
+        if (lane == o) s = t;
+    }
+    const int b = b0 + warp;
+    if (b >= B) return;                            // warp-uniform, and no block barrier follows
+    if (cls) {
+        const float v = lane < C ? s + __ldg(bc + lane) : 0.f;
+        outs[warp][lane] = v;
+        __syncwarp();
+        if (lane < C) {                            // softmax in the order of vae_heads_fwd_kernel
+            float mx = outs[warp][0];
+            for (int c = 1; c < C; ++c) mx = fmaxf(mx, outs[warp][c]);
+            float den = 0.f;
+            for (int c = 0; c < C; ++c) den += expf(outs[warp][c] - mx);
+            y_hat[(int64_t)b * C + lane] = expf(v - mx) / den;
+            zcat[(int64_t)b * (C + Z) + lane] = (float)yoh[(int64_t)b * C + lane];
+        }
+    } else {
+        const int zi = z0 + lane % HT_ZT;
+        const float v = s + (zi < Z ? __ldg((lane < HT_ZT ? bm : bv) + zi) : 0.f);
+        const float lv = __shfl_down_sync(0xffffffffu, v, HT_ZT);
+        if (lane < HT_ZT && zi < Z) {
+            mu[(int64_t)b * Z + zi] = v;
+            logvar[(int64_t)b * Z + zi] = lv;
+            const float zz = eps ? fmaf(__ldg(eps + (int64_t)b * Z + zi), expf(0.5f * lv), v) : v;
+            z_[(int64_t)b * Z + zi] = zz;
+            zcat[(int64_t)b * (C + Z) + C + zi] = zz;
+        }
+    }
+}
+
+// backward.  Blocks [0, nwt): a tile of HT_OUT outputs x 32 columns of cat(y, h, 1) (column C + H is the bias) of the
+// weight gradients.  The block walks the batch in chunks of HT_BC meshes, recomputing their small gradients
+// (heads_small_grad), and a thread sums over b in ascending order - the order of vae_heads_bwd_kernel, with no batch
+// limit and no workspace.  Blocks [nwt, ..): g_h of HT_MESH meshes x 32 columns, a thread per element summing the
+// C + 2Z outputs in ascending order in chunks ([0, C), then 32 at a time), the classifier's dropout mask applied
+// after its C terms.
+__global__ void __launch_bounds__(256)
+vae_heads_bwd_tiled_kernel(int B, int H, int Z, int C, const float *__restrict__ h, const int64_t *__restrict__ yoh,
+                           const float *__restrict__ Wc, const float *__restrict__ Wm, const float *__restrict__ Wv,
+                           SmallIn gin, float p, uint64_t seed, const int64_t *off_dev, int64_t off_host,
+                           float *__restrict__ g_h, float *__restrict__ dWc, float *__restrict__ dbc, float *__restrict__ dWm,
+                           float *__restrict__ dbm, float *__restrict__ dWv, float *__restrict__ dbv, int nwt, int ncol_t) {
+    pdl_trigger();
+    pdl_wait();
+    __shared__ float sm[3][HT_BC][33];
+    const int tid = threadIdx.x, jl = tid & 31, tw = tid >> 5;
+    const int nout = C + 2 * Z;
+    const uint64_t off = (uint64_t)(off_host + (off_dev ? *off_dev : 0));
+    const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
+    if ((int)blockIdx.x < nwt) {
+        // ---- weight gradients: outputs o0 + tw + 8 t (t < 4) at column j ----
+        float(*gs)[33] = sm[0];                    // [HT_BC][HT_OUT]  small gradients of the chunk
+        float(*ht)[33] = sm[1];                    // [HT_BC][32]      columns j0.. of cat(y, h, 1)
+        float(*hdt)[33] = sm[2];                   // same, with the classifier's dropout mask
+        const int ot = blockIdx.x / ncol_t, ct = blockIdx.x - ot * ncol_t;
+        const int o0 = ot * HT_OUT, j0 = ct * 32, j = j0 + jl;
+        float acc[HT_OUT / 8] = {0.f, 0.f, 0.f, 0.f};
+        for (int c0 = 0; c0 < B; c0 += HT_BC) {
+            const int nb = min(HT_BC, B - c0);
+            if (c0) __syncthreads();
+#pragma unroll
+            for (int i = tid; i < HT_BC * 32; i += 256) {
+                const int r = i >> 5, o = o0 + (i & 31), jj = j0 + (i & 31), b = c0 + r;
+                gs[r][i & 31] = (r < nb && o < nout) ? heads_small_grad(o, b, Z, C, gin.y_hat, gin.logvar, gin.eps, gin.g_yhat,
+                                                                         gin.g_mu, gin.g_logvar, gin.g_z, gin.g_zcat) : 0.f;
+                float in = 0.f, ind = 0.f;
+                if (r < nb) {
+                    if (jj == C + H) in = ind = 1.f;
+                    else if (jj < C) in = (float)yoh[(int64_t)b * C + jj];
+                    else if (jj < C + H) {
+                        in = __ldg(h + (int64_t)b * H + jj - C);
+                        ind = (p > 0.f) ? (drop_keep(seed, off, (uint32_t)b * (uint32_t)H + (uint32_t)(jj - C), p) ? in * scale : 0.f) : in;
+                    }
+                }
+                ht[r][i & 31] = in;
+                hdt[r][i & 31] = ind;
+            }
+            __syncthreads();
+            for (int r = 0; r < nb; ++r) {
+                const float in = ht[r][jl], ind = hdt[r][jl];
+#pragma unroll
+                for (int t = 0; t < HT_OUT / 8; ++t) acc[t] = fmaf(gs[r][tw + 8 * t], o0 + tw + 8 * t < C ? ind : in, acc[t]);
+            }
+        }
+        if (j > C + H) return;
+#pragma unroll
+        for (int t = 0; t < HT_OUT / 8; ++t) {
+            const int o = o0 + tw + 8 * t;
+            if (o >= nout) break;
+            if (o < C) {
+                if (j == C + H) dbc[o] = acc[t];
+                else if (j >= C) dWc[(int64_t)o * H + j - C] = acc[t];
+            } else {
+                const int i = (o - C) % Z;
+                const bool is_mu = (o - C) < Z;
+                if (j == C + H) (is_mu ? dbm : dbv)[i] = acc[t];
+                else (is_mu ? dWm : dWv)[(int64_t)i * (C + H) + j] = acc[t];
+            }
+        }
+        return;
+    }
+    // ---- g_h of mesh b at column j ----
+    float(*gs)[33] = sm[0];                        // [HT_MESH][32]  small gradients of the output chunk
+    float(*wt)[33] = sm[1];                        // [32][32]       weight rows of the chunk, columns j0.. of h
+    const int bi = (int)blockIdx.x - nwt;
+    const int hts = (H + 31) / 32;
+    const int mt = bi / hts, jt = bi - mt * hts;
+    const int b0 = mt * HT_MESH, j0 = jt * 32;
+    const int b = b0 + tw, j = j0 + jl;
+    float a = 0.f;
+    for (int o0 = 0; o0 < nout;) {
+        const int n = o0 == 0 ? C : min(32, nout - o0);
+        if (o0) __syncthreads();
+        {
+            const int r = tid >> 5, oo = tid & 31;           // HT_MESH x 32 = 256 threads
+            gs[r][oo] = (oo < n && b0 + r < B) ? heads_small_grad(o0 + oo, b0 + r, Z, C, gin.y_hat, gin.logvar, gin.eps, gin.g_yhat,
+                                                                  gin.g_mu, gin.g_logvar, gin.g_z, gin.g_zcat) : 0.f;
+        }
+#pragma unroll
+        for (int i = tid; i < 32 * 32; i += 256) {
+            const int oo = i >> 5, col = j0 + (i & 31), o = o0 + oo;
+            float w = 0.f;
+            if (oo < n && col < H)
+                w = __ldg(o < C ? Wc + (int64_t)o * H + col
+                                : (o - C < Z ? Wm + (int64_t)(o - C) * (C + H) : Wv + (int64_t)(o - C - Z) * (C + H)) + C + col);
+            wt[oo][i & 31] = w;
+        }
+        __syncthreads();
+        for (int oo = 0; oo < n; ++oo) a = fmaf(gs[tw][oo], wt[oo][jl], a);
+        if (o0 == 0 && p > 0.f && b < B && j < H) a = drop_keep(seed, off, (uint32_t)b * (uint32_t)H + (uint32_t)j, p) ? a * scale : 0.f;
+        o0 += n;
+    }
+    if (b < B && j < H) g_h[(int64_t)b * H + j] = a;
+}
+
 }  // namespace mvb
 
 using namespace mvb;
@@ -630,10 +839,16 @@ extern "C" int mvb_vae_heads_fwd(int B, int H, int Z, int C, const float *h, con
                                  void *stream) {
     MVB_REQUIRE(B > 0 && H > 0 && Z > 0 && C > 0 && h && y_onehot && Wc && bc && Wm && bm && Wv && bv && y_hat && mu &&
                     logvar && z && zcat, "vae_heads_fwd: bad arguments");
-    MVB_REQUIRE(C + 2 * Z <= HEADS_MAX_OUT && C <= 32 && Z <= 224, "vae_heads_fwd: C=%d Z=%d too large", C, Z);
+    MVB_REQUIRE(C <= 32, "vae_heads_fwd: C=%d classes, at most 32 supported", C);
+    MVB_REQUIRE((int64_t)B * H < (1LL << 32), "vae_heads_fwd: B*H exceeds the dropout counter range");
     MVB_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "vae_heads_fwd: dropout p=%f outside [0,1)", p_drop);
-    const size_t smem = (size_t)(2 * (C + H) + (C + 2 * Z) * (C + H + 1)) * sizeof(float);
-    MVB_REQUIRE(smem <= 220 * 1024, "vae_heads_fwd: H=%d too large", H);
+    const size_t smem = (2 * (size_t)(C + H) + (size_t)(C + 2 * Z) * (C + H + 1)) * sizeof(float);
+    if (C + 2 * Z > HEADS_MAX_OUT || smem > 220 * 1024) {        // the weights do not fit one block: the tiled kernel
+        launch_pdl(vae_heads_fwd_tiled_kernel, dim3((B + HT_MESH - 1) / HT_MESH, 1 + (Z + HT_ZT - 1) / HT_ZT), dim3(256), 0,
+                   (cudaStream_t)stream, B, H, Z, C, h, y_onehot, eps, Wc, bc, Wm, bm, Wv, bv, p_drop, seed, offset_dev,
+                   offset_host, y_hat, mu, logvar, z, zcat);
+        return check_launch("mvb_vae_heads_fwd");
+    }
     static DevFlags granted;
     int rc = smem_optin(vae_heads_fwd_kernel, smem, granted, "vae_heads_fwd");
     if (rc) return rc;
@@ -650,20 +865,29 @@ extern "C" int mvb_vae_heads_bwd(int B, int H, int Z, int C, const float *h, con
                                  float *dbm, float *dWv, float *dbv, void *stream) {
     MVB_REQUIRE(B > 0 && H > 0 && Z > 0 && C > 0 && h && y_onehot && Wc && Wm && Wv && y_hat && logvar && g_h && dWc &&
                     dbc && dWm && dbm && dWv && dbv, "vae_heads_bwd: bad arguments");
-    MVB_REQUIRE(C + 2 * Z <= HEADS_MAX_OUT && C <= 32, "vae_heads_bwd: C=%d Z=%d too large", C, Z);
+    MVB_REQUIRE(C <= 32, "vae_heads_bwd: C=%d classes, at most 32 supported", C);
+    MVB_REQUIRE((int64_t)B * H < (1LL << 32), "vae_heads_bwd: B*H exceeds the dropout counter range");
+    MVB_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "vae_heads_bwd: dropout p=%f outside [0,1)", p_drop);
     const int nout = C + 2 * Z;
-    const size_t smA = (size_t)(nout * (C + H + 1) + HB_ROWS * nout + 4 + small_in_words(HB_ROWS, Z, C)) * sizeof(float);
-    const size_t smB = (size_t)(B * nout + 2 * B * 33 + 4 + small_in_words(B, Z, C)) * sizeof(float);
-    const size_t smem = smA > smB ? smA : smB;
-    MVB_REQUIRE(smem <= 220 * 1024, "vae_heads_bwd: batch %d / H=%d too large for one pass", B, H);
-    static DevFlags granted;
-    int rc = smem_optin(vae_heads_bwd_kernel, smem, granted, "vae_heads_bwd");
-    if (rc) return rc;
-    const int nbg = (B + HB_ROWS - 1) / HB_ROWS;
     const int ntile = (C + H + 1 + 31) / 32;
     SmallIn gin;
     gin.y_hat = y_hat; gin.logvar = logvar; gin.eps = eps; gin.g_yhat = g_yhat; gin.g_mu = g_mu; gin.g_logvar = g_logvar;
     gin.g_z = g_z; gin.g_zcat = g_zcat;
+    const size_t smA = ((size_t)nout * (C + H + 1) + HB_ROWS * nout + 4 + small_in_words(HB_ROWS, Z, C)) * sizeof(float);
+    const size_t smB = ((size_t)B * (nout + 2 * 33 + 2 * C + 5 * Z + C + Z) + 4 + 32) * sizeof(float);   // small_in_words(B, Z, C)
+    const size_t smem = smA > smB ? smA : smB;
+    if (nout > HEADS_MAX_OUT || smem > 220 * 1024) {    // the weights or the batch do not fit one block: the tiled kernel
+        const int nwt = ((nout + HT_OUT - 1) / HT_OUT) * ntile;
+        const int64_t nblk = (int64_t)nwt + (int64_t)((B + HT_MESH - 1) / HT_MESH) * ((H + 31) / 32);
+        MVB_REQUIRE(nblk < (1LL << 31), "vae_heads_bwd: B=%d H=%d needs too many blocks", B, H);
+        launch_pdl(vae_heads_bwd_tiled_kernel, dim3((unsigned)nblk), dim3(256), 0, (cudaStream_t)stream, B, H, Z, C, h, y_onehot,
+                   Wc, Wm, Wv, gin, p_drop, seed, offset_dev, offset_host, g_h, dWc, dbc, dWm, dbm, dWv, dbv, nwt, ntile);
+        return check_launch("mvb_vae_heads_bwd");
+    }
+    static DevFlags granted;
+    int rc = smem_optin(vae_heads_bwd_kernel, smem, granted, "vae_heads_bwd");
+    if (rc) return rc;
+    const int nbg = (B + HB_ROWS - 1) / HB_ROWS;
     launch_pdl(vae_heads_bwd_kernel, dim3(nbg + ntile), dim3(256), smem, (cudaStream_t)stream, B, H, Z, C, h, y_onehot, Wc, Wm, Wv, gin, p_drop, seed,
                                                                             offset_dev, offset_host, g_h, dWc, dbc, dWm, dbm, dWv,
                                                                             dbv, nbg);

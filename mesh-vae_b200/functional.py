@@ -418,7 +418,7 @@ class DropoutStream:
 
 
 _NO_RNG = (0, None, 0)
-VAE_HEADS_MAX_BATCH = 256      # the one-launch heads backward keeps the whole batch's small gradients in shared memory
+VAE_HEADS_MAX_BATCH = 256      # the largest batch of the one-launch heads kernels at the default shapes (larger: tiled kernels)
 
 
 class _LinearFn(torch.autograd.Function):
@@ -533,21 +533,10 @@ class _VaeHeadsFn(torch.autograd.Function):
 def vae_heads(h, y_onehot, eps, classifier, z_mean, z_log_var, p: float = 0.0, rng=_NO_RNG):
     """-> (y_hat, mu, logvar, z, cat(y, z)); `classifier`, `z_mean`, `z_log_var` are the model's
     nn.Linear modules (their Parameters receive the gradients); eps=None means z = mu (test mode).
-    Batches beyond VAE_HEADS_MAX_BATCH meshes (the one-launch backward keeps the batch's small gradients in shared
-    memory) run in chunks of that size: the outputs are concatenated and autograd adds the chunks' parameter gradients
-    (no gradient sinks on that path - the kernels OVERWRITE their dW outputs)."""
+    One call covers any batch, hidden width and latent size (at most 32 classes): the library picks the one-launch
+    kernels where they fit and the tiled ones elsewhere, with the same results and the same dropout mask."""
     args = (classifier.weight, classifier.bias, z_mean.weight, z_mean.bias, z_log_var.weight, z_log_var.bias)
-    b = h.shape[0]
-    if b <= VAE_HEADS_MAX_BATCH:
-        return _VaeHeadsFn.apply(h, y_onehot, eps, *args, float(p), rng)
-    if p > 0:
-        raise _lib.MvbError(f"vae_heads: dropout with more than {VAE_HEADS_MAX_BATCH} meshes per call is not supported "
-                            "(the mask is keyed by the row index inside a call)")
-    plain = tuple(t.view_as(t) for t in args)          # non-leaf aliases: no sink attribute, autograd accumulates
-    outs = [_VaeHeadsFn.apply(h[i:i + VAE_HEADS_MAX_BATCH], y_onehot[i:i + VAE_HEADS_MAX_BATCH],
-                              None if eps is None else eps[i:i + VAE_HEADS_MAX_BATCH], *plain, 0.0, rng)
-            for i in range(0, b, VAE_HEADS_MAX_BATCH)]
-    return tuple(torch.cat([o[j] for o in outs], 0) for j in range(5))
+    return _VaeHeadsFn.apply(h, y_onehot, eps, *args, float(p), rng)
 
 
 # ---------------------------------------------------------------------------------------------
