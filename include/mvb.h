@@ -142,7 +142,13 @@ int mvb_cheb_fwd(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, 
  * CSR arguments are L^T (for the symmetric L_hat of nn/conv.py:541-555 this equals L).
  * dx may be NULL (first encoder layer: the input needs no gradient), dbias may be NULL.
  * dweight [K,Fin,Fout] and dbias [Fout] are OVERWRITTEN (deterministic ordered reductions, no
- * atomics).  workspace: mvb_cheb_bwd_workspace_bytes(...) bytes, 16-byte aligned. */
+ * atomics).  workspace: mvb_cheb_bwd_workspace_bytes(...) bytes, 16-byte aligned.
+ * Width limit: the weight gradient is one reduction [M x n] over the rows, M = K*Fin (+1 for the bias) and n = Fout in
+ * the basis form, M = K*Fout and n = Fin in the adjoint form.  The tensor cores take it when M <= 128 and n <= 32 (16-
+ * or 4-wide planes with K <= 6 / 8, 32-wide with K <= 3); the FFMA reduction holds ceil(M/4) * ceil(n/4) <= 512
+ * register tiles.  Beyond both, mvb_cheb_bwd returns MVB_EINVAL ("wgrad: K*Fin x Fout ... too large") instead of launching it:
+ * at K = 6 a 32 -> 48 layer (49 x 12 tiles), 48 -> 32 (48 x 12) or 48 -> 48 (72 x 12) - e.g. num_conv_filters
+ * 16, 32, 48, 48, 48 trains no further than its first backward pass.  The forward pass has no such limit there. */
 int mvb_cheb_bwd_uses_basis(int Fin, int Fout, int need_dx);
 size_t mvb_cheb_bwd_workspace_bytes(int N, int B, int Fin, int Fout, int K, int n_active,
                                     int need_dx);
@@ -307,7 +313,8 @@ int mvb_cheb_sel_bwd(int N, int B, int Fin, int Fout, int K, const float *x, con
  * Two implementations behind the same entry points: the tensor-core mesh kernels (csrc/mvb_mesh_tc.cu: 16 / 32-wide
  *   features, up to 1280 vertices - levels 1-3 of the template; a cluster of 1-2 CTAs per mesh keeps the basis planes
  *   in shared memory in the UMMA operand layout and contracts them with tcgen05.mma into TMEM accumulators) and the
- *   FFMA mesh kernels (csrc/mvb_layer.cu: any multiple-of-4 width, a few hundred vertices).
+ *   FFMA mesh kernels (csrc/mvb_layer.cu: Fin and Fout of 4, 8, 16, 32 or 64 - a power-of-two number of 4-wide quads -
+ *   and a few hundred vertices).
  * mvb_cheb_layer_supported: 1 when one of them covers the level in both directions, else 0 - the caller then uses
  *   mvb_pool_* + mvb_cheb_*.
  * Backward: nothing but x and y is kept from the forward pass (the basis is recomputed in shared

@@ -536,7 +536,8 @@ using namespace mvb;
 
 extern "C" int mvb_cheb_layer_supported(int N, int B, int Fin, int Fout, int K, int L_nnz, int n_in, int U_nnz, int n_out) {
     // every layer has two implementations: the tensor-core mesh kernels (mvb_mesh_tc.cu; 16 / 32-wide features,
-    // up to 1280 vertices) and the FFMA mesh kernels of this file (any multiple of 4, levels of a few hundred vertices)
+    // up to 1280 vertices) and the FFMA mesh kernels of this file (4, 8, 16, 32 or 64 features in and out - a power-of-two
+    // number of quads, layer_check - and levels of a few hundred vertices)
     const bool fwd = mesh_tc_fwd_supported(N, B, Fin, Fout, K, L_nnz, n_in, n_out) ||
                      layer_check(N, B, Fin, Fout, K, L_nnz, n_in, U_nnz, n_out, false, nullptr, nullptr);
     const bool bwd = mesh_tc_bwd_supported(N, B, Fin, Fout, K, L_nnz, n_in, n_out, U_nnz > 0) ||

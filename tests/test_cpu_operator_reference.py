@@ -143,13 +143,18 @@ SMALL = {
 }
 
 
-@pytest.mark.parametrize("case", list(SMALL))
+# polygon_order 6 (the default config) on every case, and the other orders a config may ask for: K = 1 (T_0 alone) and
+# K = 2 (T_1 without a 2 L T - T step) are where a restated recurrence most easily goes wrong
+REF_ORDERS = [(c, 6) for c in SMALL] + [(c, k) for c in SMALL for k in (1, 2, 3, 8)]
+
+
+@pytest.mark.parametrize("case,K", REF_ORDERS, ids=[c if k == 6 else f"{c}-K{k}" for c, k in REF_ORDERS])
 @pytest.mark.parametrize("kind", ["plain", "enc", "dec", "wdec"])
-def test_reference_matches_oracle_float64(case, kind):
+def test_reference_matches_oracle_float64(case, kind, K):
     op = SMALL[case]()
     n = op.n_rows
-    rng = np.random.default_rng(len(case) * 7 + len(kind))
-    K, fin, fout, b = 6, 5, 7, 3
+    rng = np.random.default_rng(len(case) * 7 + len(kind) + (0 if K == 6 else 100 * K))
+    fin, fout, b = 5, 7, 3
     u = d = None
     n_in = n
     if kind == "enc":

@@ -200,13 +200,24 @@ def test_cheb_conv_vertex_counts(mvb, n):
     _check_layer("mvb_cheb", lambda a, b_, c: mvb.functional.cheb_conv(a, b_, c, lo, True), op, x, w, bias, True, rng=rng)
 
 
+def _k_ids(cases, k_col=-1):
+    """pytest ids of a case table with a polygon-order column: the K = 6 rows keep the ids they had before the column
+    existed, the other orders get a -K<k> suffix"""
+    return ["-".join(str(v) for i, v in enumerate(c) if i != k_col % len(c)) + ("" if c[k_col] == 6 else f"-K{c[k_col]}")
+            for c in cases]
+
+
+# (Fin, Fout, K): the default order, and K = 2 / 3 / 8 (no 2 L T - T step, one, and more steps than the default)
+RECUR_CASES = [(16, 16, 6), (16, 32, 6), (16, 16, 2), (16, 32, 3), (16, 16, 8), (16, 32, 8)]
+
+
 @pytest.mark.parametrize("case", ["irregular300", "directed1w", "tail300"])
-@pytest.mark.parametrize("fin,fout", [(16, 16), (16, 32)])
-def test_fused_recurrence_is_bit_identical_on_other_operators(mvb, case, fin, fout):
+@pytest.mark.parametrize("fin,fout,k", RECUR_CASES, ids=_k_ids(RECUR_CASES))
+def test_fused_recurrence_is_bit_identical_on_other_operators(mvb, case, fin, fout, k):
     """the one-kernel recurrence of small levels sums in the order of the step-by-step SpMM launches"""
     op = SQUARE[case]()
     lo = _l_op(mvb, op)
-    x, w, bias, rng = _inputs(7, op.n_rows, 6, fin, fout, 6)
+    x, w, bias, rng = _inputs(7, op.n_rows, 6, fin, fout, k)
     dy = _dev(rng.standard_normal((op.n_rows, 6, fout)))
     res = []
     try:
@@ -252,12 +263,24 @@ def test_cheb_conv_sel(mvb, case, repeat, fin):
 # mvb_cheb_layer_fwd / _bwd through cheb_layer
 # ---------------------------------------------------------------------------------------------
 MODES = ["mesh_tc=1,0", "mesh_tc=1,1", "mesh_tc=1,2", "mesh_tc=0,0"]
-# (operator, kind, B, Fin, Fout, relu)
-LAYER_CASES = [("directed2", "enc", 8, 16, 16, True), ("directed2", "dec", 8, 16, 32, True),
-               ("relabelled2", "enc", 16, 32, 32, True), ("irregular300", "plain", 4, 16, 16, True),
-               ("irregular300", "dec", 6, 32, 16, True), ("directed1w", "plain", 8, 16, 16, True),
-               ("irregular300", "wenc", 4, 16, 16, False), ("directed2", "enc_rep", 4, 16, 16, True),
-               ("tail300", "plain", 4, 16, 16, True)]
+LAYER_OPS = {**SQUARE, "relabelled3": lambda: C.relabelled(3, seed=14)}
+# (operator, kind, B, Fin, Fout, relu, K)
+LAYER_CASES = [("directed2", "enc", 8, 16, 16, True, 6), ("directed2", "dec", 8, 16, 32, True, 6),
+               ("relabelled2", "enc", 16, 32, 32, True, 6), ("irregular300", "plain", 4, 16, 16, True, 6),
+               ("irregular300", "dec", 6, 32, 16, True, 6), ("directed1w", "plain", 8, 16, 16, True, 6),
+               ("irregular300", "wenc", 4, 16, 16, False, 6), ("directed2", "enc_rep", 4, 16, 16, True, 6),
+               ("tail300", "plain", 4, 16, 16, True, 6)]
+# the orders a config may ask for (the tensor-core mesh kernels take K <= 16).  The backward reduces dW in plane groups of
+# at most 128 / Fout planes (csrc/mvb_mesh_tc.cu wgrad_group): one group on the tensor cores (Fout 16: K <= 6; Fout 32:
+# K <= 3), one group too wide for them that falls to the FFMA reduction (Fout 16: K 7-8; Fout 32: K 4), several groups
+# each finalized into its own slice of dW (Fout 16: K 9, 16; Fout 32: K 5-16).  Operators whose T_k stay bounded at
+# K = 16: row sums <= 0.95, or a symmetric normalised L_hat
+LAYER_CASES += [("irregular300", ("enc", "dec", "plain")[i % 3], 8, 16, 16, True, k) for i, k in enumerate((1, 2, 3, 4, 5, 7, 8, 9, 16))]
+LAYER_CASES += [("relabelled2", ("dec", "plain", "enc")[i % 3], 8, 32 if k % 2 else 16, 32, True, k)
+                for i, k in enumerate((1, 2, 3, 4, 5, 7, 8, 9, 16))]
+# widths only the FFMA mesh kernels take
+LAYER_CASES += [("directed2", "enc", 4, 8, 8, True, 2), ("irregular300", "dec", 4, 8, 8, False, 7),
+                ("relabelled3", "plain", 4, 64, 64, True, 3), ("relabelled3", "enc", 8, 64, 64, True, 9)]
 
 
 def _layer_ops(op, kind, seed):
@@ -299,14 +322,14 @@ def _run_layer_case(mvb, op, kind, b, fin, fout, relu, mode, k=6, expect_fused=N
 
 
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("case,kind,b,fin,fout,relu", LAYER_CASES)
-def test_cheb_layer(mvb, case, kind, b, fin, fout, relu, mode):
-    op = SQUARE[case]()
+@pytest.mark.parametrize("case,kind,b,fin,fout,relu,k", LAYER_CASES, ids=_k_ids(LAYER_CASES))
+def test_cheb_layer(mvb, case, kind, b, fin, fout, relu, k, mode):
+    op = LAYER_OPS[case]()
     mvb._lib.tune(mode)
     try:
         # a selection with a repeated vertex, a weighted D and an isolated tail are not the fused kernels' layers
         fits = kind not in ("wenc", "enc_rep") and case != "tail300"
-        _run_layer_case(mvb, op, kind, b, fin, fout, relu, mode,
+        _run_layer_case(mvb, op, kind, b, fin, fout, relu, mode, k=k,
                         expect_fused=(False if not fits else (True if mode == "mesh_tc=1,0" else None)))
     finally:
         _reset(mvb)
@@ -375,11 +398,15 @@ STREAM_OPS = {
     "hubband": (lambda: C.irregular(4998, seed=12, deg=(4, 8), hub_rows=np.arange(5, 1600, 400), hub_deg=(4200, 4400)),
                 "some"),
 }
-STREAM_CASES = [("directed0", "dec", 64, 16), ("directed0w", "plain", 64, 8), ("relabelled0", "dec", 64, 8),
-                ("dense", "plain", 64, 8), ("dense", "dec", 64, 16), ("hubband", "plain", 64, 8), ("hubband", "dec", 64, 16)]
+# (operator, kind, B, meshes per slab, K): the streaming kernel takes K <= 8
+STREAM_CASES = [("directed0", "dec", 64, 16, 6), ("directed0w", "plain", 64, 8, 6), ("relabelled0", "dec", 64, 8, 6),
+                ("dense", "plain", 64, 8, 6), ("dense", "dec", 64, 16, 6), ("hubband", "plain", 64, 8, 6),
+                ("hubband", "dec", 64, 16, 6),
+                ("directed0", "dec", 64, 16, 1), ("relabelled0", "plain", 64, 8, 2), ("hubband", "dec", 64, 16, 3),
+                ("dense", "plain", 64, 8, 8), ("relabelled0", "dec", 64, 16, 8)]
 
 
-def _run_stream_case(mvb, op, kind, b, sw, overflow=None):
+def _run_stream_case(mvb, op, kind, b, sw, overflow=None, k=6):
     sms = torch.cuda.get_device_properties(DEV).multi_processor_count
     if overflow is not None:
         bands = C.stream_bands(op, b, sw, sms)
@@ -390,11 +417,11 @@ def _run_stream_case(mvb, op, kind, b, sw, overflow=None):
     lo = _l_op(mvb, op)
     uo = _p_op(mvb, u) if u is not None else None
     n_in = u.n_cols if u is not None else op.n_rows
-    x, w, bias, rng = _inputs(sw + b, n_in, b, 16, 16, 6)
+    x, w, bias, rng = _inputs(sw + b + (0 if k == 6 else 100 * k), n_in, b, 16, 16, k)
     Fn = mvb.functional
     mvb._lib.tune(f"stream_tc=1,{sw}")
     try:
-        assert Fn.cheb_stream_supported(op.n_rows, b, 16, 16, 6, lo, uo, None)
+        assert Fn.cheb_stream_supported(op.n_rows, b, 16, 16, k, lo, uo, None)
         c0 = mvb._lib.lib.mvb_launch_count()
         _check_layer("mvb_cheb_stream", lambda a, b_, c: Fn.cheb_layer(a, b_, c, lo, uo, None, relu=True), op, x, w, bias,
                      True, u=u, rng=rng)
@@ -403,10 +430,10 @@ def _run_stream_case(mvb, op, kind, b, sw, overflow=None):
         _reset(mvb)
 
 
-@pytest.mark.parametrize("case,kind,b,sw", STREAM_CASES)
-def test_cheb_stream(mvb, case, kind, b, sw):
+@pytest.mark.parametrize("case,kind,b,sw,k", STREAM_CASES, ids=_k_ids(STREAM_CASES))
+def test_cheb_stream(mvb, case, kind, b, sw, k):
     mk, overflow = STREAM_OPS[case]
-    _run_stream_case(mvb, mk(), kind, b, sw, overflow)
+    _run_stream_case(mvb, mk(), kind, b, sw, overflow, k=k)
 
 
 def test_cheb_stream_smallest_and_ragged(mvb):
@@ -429,14 +456,19 @@ def test_cheb_stream_smallest_and_ragged(mvb):
 # ---------------------------------------------------------------------------------------------
 # run-to-run determinism on irregular operators
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("path", ["conv_adjoint", "conv_basis", "layer", "layer_ffma", "stream"])
-def test_bit_identical_run_to_run(mvb, path):
+# one other order per path: K = 9 and 16 reduce dW of the mesh kernels in several plane groups
+DET_CASES = [("conv_adjoint", 6), ("conv_basis", 6), ("layer", 6), ("layer_ffma", 6), ("stream", 6),
+             ("conv_adjoint", 2), ("conv_basis", 8), ("layer", 9), ("layer_ffma", 3), ("stream", 8), ("layer", 16)]
+
+
+@pytest.mark.parametrize("path,k", DET_CASES, ids=_k_ids(DET_CASES))
+def test_bit_identical_run_to_run(mvb, path, k):
     op = C.irregular(4998, seed=13, hubs=4, hub_deg=(900, 1000), isolated=20, dups=50, loops=20) if path == "stream" \
         else SQUARE["irregular300"]()
     lo = _l_op(mvb, op)
     fout = 32 if path == "conv_basis" else 16
     b = 64 if path == "stream" else 8
-    x, w, bias, rng = _inputs(17, op.n_rows, b, 16, fout, 6)
+    x, w, bias, rng = _inputs(17, op.n_rows, b, 16, fout, k)
     dy = _dev(rng.standard_normal((op.n_rows, b, fout)))
     Fn = mvb.functional
     if path == "stream":
@@ -450,7 +482,7 @@ def test_bit_identical_run_to_run(mvb, path):
             if path.startswith("conv"):
                 y = Fn.cheb_conv(xg, wg, bg, lo, True)
             else:
-                assert Fn.cheb_layer_supported(op.n_rows, b, 16, fout, 6, lo, None, None)
+                assert Fn.cheb_layer_supported(op.n_rows, b, 16, fout, k, lo, None, None)
                 y = Fn.cheb_layer(xg, wg, bg, lo, None, None, relu=True)
             y.backward(dy)
             outs.append((y.detach(), xg.grad, wg.grad, bg.grad))
