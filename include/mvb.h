@@ -179,6 +179,9 @@ int mvb_vae_reparam_bwd(int64_t n, const float *logvar, const float *eps, const 
  * backward).
  * Arithmetic is fp64 when x_gt is fp64 (as torch type promotion makes the reference do),
  * per-element fp32 with fp64 accumulation otherwise.  Deterministic (fixed-order reductions).
+ * Entry width: 8 vertices x 32 meshes of C x_gt values and recon_ld floats must fit 48 KB of shared memory - C = recon_ld
+ * up to 16 with fp64 x_gt, 24 with fp32; a wider entry returns MVB_EINVAL ("C too large").  No alignment is required of
+ * recon, x_gt or dnll (16-byte aligned buffers take the vector paths).
  * workspace: mvb_vae_loss_workspace_bytes(B, N) bytes. */
 size_t mvb_vae_loss_workspace_bytes(int B, int N);
 int mvb_vae_loss_fwd(int B, int N, int C, int Z, int ncls, const float *recon, int recon_ld, const void *x_gt,
@@ -210,7 +213,8 @@ int mvb_gaussian_nll_bwd(int64_t n, const float *mu, const void *x, int x_is_f64
 
 /* ---- input hand-off: mesh-major batch -> zero-padded vertex-major planes --------------------
  * out[n, b, 0:Cp] = (x[b, n, 0:C], 0...)   x [B,N,C] as the loader delivers it (models/cheb_VAE.py:195-200
- * reshape), out [N,B,Cp] with Cp >= C (4 for the 3-channel meshes): the layout every kernel works in. */
+ * reshape), out [N,B,Cp] with Cp >= C (4 for the 3-channel meshes): the layout every kernel works in.  C <= 8; no
+ * alignment is required (a 16-byte aligned out takes the vector stores when C = 3, Cp = 4). */
 int mvb_pack_vertex_major(int B, int N, int C, int Cp, const float *x, float *out, void *stream);
 
 /* ---- next row f3: per-batch reconstruction error  (main.py:88-93, :139-146; inference.py:100-127)
@@ -269,6 +273,7 @@ int mvb_adam_step_hp(int64_t n, float *p, const float *g, float *m, float *v, in
  *                       summed gradient.  tick = 1: the step counter is incremented first (the first exchange of a step).
  *                       Two buckets on two channels may be in flight at once (the early one on a side stream under the
  *                       rest of the backward pass); max_ctas > 0 caps the grid of such a background launch.
+ * p / m / v, grad_sum_out and every rank's gradient buffer must be 16-byte aligned (MVB_EALIGN otherwise).
  * state: mvb_dp_state_bytes() of LOCAL device memory, zero at creation (uint32 words: [0] epoch, [1] number of waits that
  * gave up after ~30 s because a peer never signalled - the results are then invalid; a healthy run keeps it 0).  Every
  * rank must issue the same sequence of begin / reduce calls.  Enqueue-only and CUDA-graph capturable (signals are epoch

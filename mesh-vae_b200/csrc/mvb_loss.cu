@@ -91,7 +91,8 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
         if (lane == 0) partial[(int64_t)blockIdx.x * B + b0 + b] = s;
     }
     __syncthreads();
-    if (ld == 4 && C == 3) {          // padded mesh coordinates: one 16-byte entry per (vertex, mesh), pad lane zeroed
+    // padded mesh coordinates: one 16-byte entry per (vertex, mesh), pad lane zeroed (an offset view of dnll: scalar path)
+    if (ld == 4 && C == 3 && (reinterpret_cast<uintptr_t>(dnll) & 15) == 0) {
         for (int i = tid; i < nv * nb; i += nthreads) {
             const int v = i / nb, b = i - v * nb;
             float4 r = *reinterpret_cast<const float4 *>(Rs + v * (BCH * 4) + b * 4);
@@ -238,7 +239,7 @@ pack_vertex_major_kernel(int B, int N, int C, int Cp, const float *__restrict__ 
     __shared__ float tile[8][32 * 8 + 1];
     const int v0 = blockIdx.x * 32, b0 = blockIdx.y * 8;
     const int nv = min(32, N - v0), nb = min(8, B - b0);
-    if (C == 3 && Cp == 4 && nv == 32 && nb == 8 && blockDim.x == 256) {
+    if (C == 3 && Cp == 4 && nv == 32 && nb == 8 && blockDim.x == 256 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
         // the mesh coordinates: 96 contiguous floats per mesh in, one float4 entry per (vertex, mesh) out, no divisions
         const int t = threadIdx.x;
 #pragma unroll
