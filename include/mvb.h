@@ -158,6 +158,31 @@ int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, 
                  float *dweight, float *dbias, void *workspace, size_t workspace_bytes,
                  void *stream);
 
+/* ---- A13b: gradient with respect to the operator values (nn/conv.py:557-581 with a `norm` that requires grad) -------
+ * An operator whose values change every step (computed from learned edge weights) keeps its pattern: CSR(L) and
+ * CSR(L^T) are built once, with perm[nnz] / perm_t[nnz] mapping each CSR(L) / CSR(L^T) slot to its COO entry (the
+ * stable counting sort of mvb_csr_from_coo_host: a stable argsort of the COO rows, resp. columns).
+ * mvb_csr_values: vals[j] = coo_vals[perm[j]], vals_t[j] = coo_vals[perm_t[j]] - one launch, enqueue only (capturable).
+ *
+ * mvb_cheb_bwd_op: everything mvb_cheb_bwd returns in the basis form - dx, dweight, dbias are the same bits - plus
+ *   d_coo_vals[e] = <G_1[r], T_0[c]> + 2 sum_{k=2}^{K-1} <G_k[r], T_{k-1}[c]>   (<a,b>: sum over the B*Fin entries of a
+ *   vertex row; G_k = dloss/dT_k of the basis form's reverse recurrence; (r, c) = (edge_index[1][e], edge_index[0][e]))
+ * OVERWRITTEN in COO order, deterministic (one store per entry, no atomics); all zero when K == 1.  Duplicate entries
+ * each receive the full value.  Always the basis form (the caller keeps `basis` from mvb_cheb_fwd whatever
+ * mvb_cheb_bwd_uses_basis says); the weight-gradient branch is joined before the call returns - it is never deferred
+ * (mvb_side_join has nothing to wait for).
+ * rowptr / colidx / perm: CSR(L) (the edge gradient); rowptr_t / colidx_t / vals_t: CSR(L^T) (the reverse recurrence).
+ * n_active as for mvb_cheb_fwd: every entry must lie in the active prefix.  dx may be NULL, dbias may be NULL.
+ * workspace: mvb_cheb_bwd_op_workspace_bytes(...) bytes, 16-byte aligned. */
+int mvb_csr_values(int nnz, const int32_t *perm, const int32_t *perm_t, const float *coo_vals, float *vals, float *vals_t,
+                   void *stream);
+size_t mvb_cheb_bwd_op_workspace_bytes(int N, int B, int Fin, int Fout, int K, int n_active);
+int mvb_cheb_bwd_op(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, const int32_t *rowptr,
+                    const int32_t *colidx, const int32_t *perm, const int32_t *rowptr_t, const int32_t *colidx_t,
+                    const float *vals_t, const float *x, const float *basis, const float *weight,
+                    const float *y_for_relu, const float *dy, float *dx, float *dweight, float *dbias,
+                    float *d_coo_vals, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- A9: reparameterisation  (models/cheb_VAE.py:309-319) ----------------------------------
  * z = eps * exp(0.5 * logvar) + mu  on n = B*Z elements; eps is supplied by the caller (the
  * reference draws it with the CPU generator, :316).  Backward: dmu = dz, dlogvar = dz*eps*0.5*std. */

@@ -53,6 +53,10 @@ SIGNATURES = {
     "mvb_cheb_bwd_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int, c_int]),
     "mvb_cheb_bwd": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                              _vp, c_size_t, _vp]),
+    "mvb_csr_values": (c_int, [c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mvb_cheb_bwd_op_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "mvb_cheb_bwd_op": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                _vp, _vp, _vp, _vp, _vp, _vp, c_size_t, _vp]),
     "mvb_vae_reparam_fwd": (c_int, [c_int64, _vp, _vp, _vp, _vp, _vp]),
     "mvb_vae_reparam_bwd": (c_int, [c_int64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mvb_vae_loss_workspace_bytes": (c_size_t, [c_int, c_int]),

@@ -7,7 +7,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libmvb_sm100a.so")
-SOURCES = ["mvb_api.cu", "mvb_spmm.cu", "mvb_contract.cu", "mvb_loss.cu", "mvb_optim.cu", "mvb_tc.cu", "mvb_dense.cu", "mvb_layer.cu", "mvb_mesh_tc.cu", "mvb_stream_tc.cu", "mvb_dp.cu"]
+SOURCES = ["mvb_api.cu", "mvb_spmm.cu", "mvb_contract.cu", "mvb_loss.cu", "mvb_optim.cu", "mvb_tc.cu", "mvb_dense.cu", "mvb_layer.cu", "mvb_mesh_tc.cu", "mvb_stream_tc.cu", "mvb_dp.cu", "mvb_opgrad.cu"]
 
 
 def _stale():

@@ -88,8 +88,11 @@ class cheb_VAE(nn.Module):
 
     def _layer(self, x, conv, lvl, up=None, down=None):
         """one step of the encoder loop (conv, relu, pool(D): models/cheb_VAE.py:264-265) or of the decoder
-        loop (pool(U), conv, relu: :284-285); coarse levels run as ONE mesh-resident kernel per direction"""
-        if self.fused_layers and x.is_cuda and conv.fuse_relu:
+        loop (pool(U), conv, relu: :284-285); coarse levels run as ONE mesh-resident kernel per direction.  An operator
+        computed from learned edge weights (A_norm[lvl] requires grad) takes the composition: only ChebConv_batch
+        differentiates its values"""
+        learned = self.A_norm[lvl].requires_grad and torch.is_grad_enabled()
+        if self.fused_layers and x.is_cuda and conv.fuse_relu and not learned:
             l_op = operators.from_edges(self.A_edge_index[lvl], self.A_norm[lvl], self.A_num_nodes[lvl], x.device)
             u_op = None if up is None else operators.from_sparse(up, x.device)
             d_op = None if down is None else operators.from_sparse(down, x.device)
@@ -159,8 +162,8 @@ class cheb_VAE(nn.Module):
         if x.is_cuda and not conv.fuse_relu:
             # the 3-channel output stays in its 4-float entries: the returned [B,N,3] tensor is a view, and
             # loss_function reads the padded buffer in place (handed over once through _recon_padded)
-            op = operators.from_edges(self.A_edge_index[-1], self.A_norm[-1], x.size(1), x.device)
-            y = Fn.cheb_conv(Fn.to_vertex_major(x), conv.weight, conv.bias, op, False, keep_padding=True)
+            op, vals = operators.edge_operator(self.A_edge_index[-1], self.A_norm[-1], x.size(1), x.device)
+            y = Fn.cheb_conv(Fn.to_vertex_major(x), conv.weight, conv.bias, op, False, keep_padding=True, norm=vals)
             fout = conv.weight.shape[2]
             if y.shape[2] != fout:
                 self._recon_padded = y

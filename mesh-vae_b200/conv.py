@@ -52,15 +52,12 @@ class ChebConv_batch(torch.nn.Module):
             edge_weight = torch.ones((edge_index.size(1),), dtype=dtype, device=edge_index.device)
         else:
             edge_weight = edge_weight[keep]
-        row, col = edge_index[0], edge_index[1]
-        deg = torch.zeros(num_nodes, dtype=edge_weight.dtype, device=edge_index.device).scatter_add_(0, row, edge_weight)
-        dis = deg.pow(-0.5)
-        dis[dis == float("inf")] = 0
-        return edge_index, -dis[row] * edge_weight * dis[col]
+        return edge_index, _sym_norm_values(edge_index, num_nodes, edge_weight)
 
     def forward(self, x, edge_index, norm, edge_weight=None):
-        op = operators.from_edges(edge_index, norm, x.size(1), x.device)
-        y = Fn.cheb_conv(Fn.to_vertex_major(x), self.weight, self.bias, op, self.fuse_relu)
+        """a `norm` that requires grad (computed from learned edge weights) receives its gradient, as in the reference"""
+        op, vals = operators.edge_operator(edge_index, norm, x.size(1), x.device)
+        y = Fn.cheb_conv(Fn.to_vertex_major(x), self.weight, self.bias, op, self.fuse_relu, norm=vals)
         return Fn.from_vertex_major(y)
 
     def __repr__(self):
@@ -94,14 +91,34 @@ class ChebConv(torch.nn.Module):
     def forward(self, x, edge_index, edge_weight: Optional[torch.Tensor] = None, batch=None, lambda_max=None):
         if self.normalization != "sym":
             raise NotImplementedError("only the 'sym' normalisation of models/cheb_cls.py:76 is implemented")
-        if edge_weight is not None or batch is not None or (lambda_max is not None and float(lambda_max) != 2.0):
-            raise NotImplementedError("ChebConv is only implemented for the call form of models/cheb_cls.py:95")
+        if batch is not None or (lambda_max is not None and float(lambda_max) != 2.0):
+            raise NotImplementedError("ChebConv is only implemented without `batch` and with lambda_max = 2")
         squeeze = x.dim() == 2
         if squeeze:
             x = x.unsqueeze(0)
-        op = self.mesh_operator(edge_index, x.size(-2), x.device, x.dtype)
-        y = Fn.from_vertex_major(Fn.cheb_conv(Fn.to_vertex_major(x), self.stacked_weight(), self.bias, op, self.fuse_relu))
+        n = x.size(-2)
+        vals = None
+        if edge_weight is None:
+            op = self.mesh_operator(edge_index, n, x.device, x.dtype)
+        else:
+            # the values change with the weights (and carry their gradient): the cached pattern of the self-loop-free
+            # edges, their values computed by differentiable torch ops (an index gather: no host synchronisation)
+            ei, kept = self._edges(edge_index, n)
+            vals = _sym_norm_values(ei, n, edge_weight[kept]).to(device=x.device, dtype=torch.float32)
+            op = operators.pattern_from_edges(ei, n, x.device)
+        y = Fn.cheb_conv(Fn.to_vertex_major(x), self.stacked_weight(), self.bias, op, self.fuse_relu, norm=vals)
+        y = Fn.from_vertex_major(y)
         return y.squeeze(0) if squeeze else y
+
+    @staticmethod
+    def _edges(edge_index, n):
+        """(edge_index without self loops, positions of the kept edges), cached per index tensor"""
+        key = ("pyg_edges", edge_index.data_ptr(), edge_index._version, int(edge_index.shape[1]), n)
+        cached = _PYG_NORM.get(key)
+        if cached is None:
+            kept = (edge_index[0] != edge_index[1]).nonzero().squeeze(1)
+            cached = _PYG_NORM[key] = (edge_index[:, kept], kept, edge_index)
+        return cached[0], cached[1]
 
     def mesh_operator(self, edge_index, n, device, dtype=torch.float32):
         """L_hat = 2 L_sym / lambda_max - I = -D^-1/2 A D^-1/2 (PyG's explicit +1/-1 diagonal cancels), cached"""
@@ -121,3 +138,13 @@ class ChebConv(torch.nn.Module):
 
 
 _PYG_NORM = {}
+
+
+def _sym_norm_values(edge_index, num_nodes, edge_weight):
+    """-deg^-1/2[row] w_e deg^-1/2[col] over self-loop-free edges, deg summed over the row index, inf -> 0
+    (nn/conv.py:548-555): plain torch ops, differentiable with respect to edge_weight"""
+    row, col = edge_index[0], edge_index[1]
+    deg = torch.zeros(num_nodes, dtype=edge_weight.dtype, device=edge_index.device).scatter_add_(0, row, edge_weight)
+    dis = deg.pow(-0.5)
+    dis[dis == float("inf")] = 0
+    return -dis[row] * edge_weight * dis[col]

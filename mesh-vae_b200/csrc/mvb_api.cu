@@ -400,13 +400,13 @@ extern "C" int mvb_side_join_lane(void *stream, int lane) {
 // first encoder layer, which needs no dX, keeps the basis form: its basis is only 3-4 columns wide).
 static bool adjoint_form(int Fin, int Fout, int need_dx) { return need_dx && 25 * Fout <= 30 * Fin && Fout % 4 == 0; }
 
-// workspace of the basis form: weight-gradient partials of the active prefix and of the empty rows, then (with dX)
-// the K planes P_k = dY W_k^T
+// workspace of the basis form: weight-gradient partials of the active prefix and of the empty rows, then (with dX or
+// the operator gradient: need_planes) the K planes P_k = dY W_k^T
 struct ChebBwdBasisWs {
     float *partA, *partB, *P;
     size_t partA_bytes, partB_bytes;
 };
-static ChebBwdBasisWs cheb_bwd_basis_ws(WsCarve &c, int N, int B, int Fin, int Fout, int K, int n_active, int need_dx) {
+static ChebBwdBasisWs cheb_bwd_basis_ws(WsCarve &c, int N, int B, int Fin, int Fout, int K, int n_active, int need_planes) {
     ChebBwdBasisWs w{};
     w.partA_bytes = align_up(wgrad_partial_bytes(K * Fin, Fout), 256);
     w.partA = c.take<float>(w.partA_bytes);
@@ -414,7 +414,7 @@ static ChebBwdBasisWs cheb_bwd_basis_ws(WsCarve &c, int N, int B, int Fin, int F
         w.partB_bytes = align_up(wgrad_partial_bytes(Fin, Fout), 256);
         w.partB = c.take<float>(w.partB_bytes);
     }
-    if (need_dx) w.P = c.take<float>((size_t)K * n_active * B * Fin * sizeof(float));
+    if (need_planes) w.P = c.take<float>((size_t)K * n_active * B * Fin * sizeof(float));
     return w;
 }
 
@@ -454,6 +454,16 @@ static int cheb_bwd_adjoint(int N, int B, int Fin, int Fout, int K, int n_active
                             const float *y_for_relu, const float *dy, float *dx, float *dweight, float *dbias, char *ws,
                             cudaStream_t st);
 
+// CSR(L) with its COO permutation and the COO gradient it is written to: the operator gradient of mvb_cheb_bwd_op
+struct OpGradArgs {
+    const int32_t *rowptr, *colidx, *perm;
+    float *d_coo_vals;
+};
+static int cheb_bwd_basis(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, const int32_t *rowptr_t,
+                          const int32_t *colidx_t, const float *vals_t, const float *x, const float *basis,
+                          const float *weight, const float *y_for_relu, const float *dy, float *dx, float *dweight,
+                          float *dbias, const OpGradArgs *og, char *ws, cudaStream_t st);
+
 extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active, int nnz,
                             const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
                             const float *x, const float *basis, const float *weight,
@@ -474,17 +484,52 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
         return cheb_bwd_adjoint(N, B, Fin, Fout, K, n_active, nnz, rowptr_t, colidx_t, vals_t, x, weight, y_for_relu, dy, dx,
                                 dweight, dbias, reinterpret_cast<char *>(workspace), st);
     }
+    return cheb_bwd_basis(N, B, Fin, Fout, K, n_active, nnz, rowptr_t, colidx_t, vals_t, x, basis, weight, y_for_relu, dy, dx,
+                          dweight, dbias, nullptr, reinterpret_cast<char *>(workspace), st);
+}
+
+// The operator gradient needs G_k = dloss/dT_k, which only the basis form's reverse recurrence produces: this entry point
+// always takes the basis form, whatever mvb_cheb_bwd_uses_basis says, and runs its weight-gradient branch beside the
+// caller's stream, joined before it returns (never deferred).
+extern "C" size_t mvb_cheb_bwd_op_workspace_bytes(int N, int B, int Fin, int Fout, int K, int n_active) {
+    WsCarve c;
+    cheb_bwd_basis_ws(c, N, B, Fin, Fout, K, n_active, 1);
+    return c.off;
+}
+
+extern "C" int mvb_cheb_bwd_op(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, const int32_t *rowptr,
+                               const int32_t *colidx, const int32_t *perm, const int32_t *rowptr_t, const int32_t *colidx_t,
+                               const float *vals_t, const float *x, const float *basis, const float *weight,
+                               const float *y_for_relu, const float *dy, float *dx, float *dweight, float *dbias,
+                               float *d_coo_vals, void *workspace, size_t workspace_bytes, void *stream) {
+    MVB_REQUIRE(N > 0 && B > 0 && Fin > 0 && Fout > 0 && K > 0 && nnz >= 0, "cheb_bwd_op: bad sizes");
+    MVB_REQUIRE(n_active >= 0 && n_active <= N, "cheb_bwd_op: n_active=%d outside [0,%d]", n_active, N);
+    MVB_REQUIRE(x && weight && dy && dweight && workspace && (nnz == 0 || d_coo_vals), "cheb_bwd_op: null pointer");
+    MVB_REQUIRE(K == 1 || n_active == 0 || (basis && rowptr && colidx && perm && rowptr_t && colidx_t && vals_t),
+                "cheb_bwd_op: null operator or basis pointer");
+    if (!aligned16(workspace)) return set_err(MVB_EALIGN, "cheb_bwd_op: workspace not 16-byte aligned");
+    const size_t need = mvb_cheb_bwd_op_workspace_bytes(N, B, Fin, Fout, K, n_active);
+    if (workspace_bytes < need) return set_err(MVB_EWORKSPACE, "cheb_bwd_op: workspace %zu < %zu", workspace_bytes, need);
+    const OpGradArgs og{rowptr, colidx, perm, d_coo_vals};
+    return cheb_bwd_basis(N, B, Fin, Fout, K, n_active, nnz, rowptr_t, colidx_t, vals_t, x, basis, weight, y_for_relu, dy, dx,
+                          dweight, dbias, &og, reinterpret_cast<char *>(workspace), (cudaStream_t)stream);
+}
+
+static int cheb_bwd_basis(int N, int B, int Fin, int Fout, int K, int n_active, int nnz, const int32_t *rowptr_t,
+                          const int32_t *colidx_t, const float *vals_t, const float *x, const float *basis,
+                          const float *weight, const float *y_for_relu, const float *dy, float *dx, float *dweight,
+                          float *dbias, const OpGradArgs *og, char *ws, cudaStream_t st) {
     const int64_t rows_act = (int64_t)n_active * B;
     const int64_t rows_in = (int64_t)(N - n_active) * B;
-    WsCarve c{reinterpret_cast<char *>(workspace)};
-    const ChebBwdBasisWs w = cheb_bwd_basis_ws(c, N, B, Fin, Fout, K, n_active, dx != nullptr);
+    WsCarve c{ws};
+    const ChebBwdBasisWs w = cheb_bwd_basis_ws(c, N, B, Fin, Fout, K, n_active, dx != nullptr || og != nullptr);
     const int has_bias = dbias != nullptr;
     int rc, nA = 0, m4A = 0, nB = 0, m4B = 0;
 
     // The weight-gradient branch (partials + ordered finalize) and the input-gradient branch
     // (P_k, reverse recurrence) are independent: fork the former onto a side stream so that the two
     // overlap (and become parallel branches of a captured CUDA graph), join before returning.
-    SideChain side(st, -1, dx != nullptr);
+    SideChain side(st, -1, dx != nullptr || og != nullptr);
     const cudaStream_t wst = side.stream();
 
     // dW_k = T_k^T dY, db = 1^T dY over the active prefix ...
@@ -517,7 +562,7 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
         if (rc) return rc;
     }
     rc = launch_wgrad_finalize(w.partA, nA, m4A, w.partB, nB, m4B, Fin, K * Fin, Fout, dweight, dbias, wst);
-    if (rc || !dx) return rc;
+    if (rc || !(dx || og)) return rc;
 
     if (rows_act > 0) {
         // P_k = dY W_k^T for all k in one pass (plane k of the workspace)
@@ -534,11 +579,22 @@ extern "C" int mvb_cheb_bwd(int N, int B, int Fin, int Fout, int K, int n_active
         a.out = w.P;
         rc = launch_contract(a, st);
         if (rc) return rc;
-        // reverse recurrence, in place on the P planes: dX = sum_k T_k(L^T) P_k
-        rc = launch_cheb_recurrence_bwd(n_active, nnz, K, rowptr_t, colidx_t, vals_t, w.P, dx, (int64_t)B * Fin, st);
+        // reverse recurrence, in place on the P planes: dX = sum_k T_k(L^T) P_k; for the operator gradient the planes
+        // G_k = dloss/dT_k (k >= 1) stay in P
+        rc = launch_cheb_recurrence_bwd(n_active, nnz, K, rowptr_t, colidx_t, vals_t, w.P, dx, (int64_t)B * Fin, st, og != nullptr);
         if (rc) return rc;
     }
-    if (rows_in > 0) {
+    if (og) {
+        // d_coo[e] = <G_1[r], T_0[c]> + 2 sum_{k>=2} <G_k[r], T_{k-1}[c]>; every entry lies in the active prefix
+        if (K > 1 && rows_act > 0) {
+            rc = launch_cheb_edge_grad(n_active, (int64_t)B * Fin, K, og->rowptr, og->colidx, og->perm, x, basis, w.P, og->d_coo_vals, st);
+        } else if (nnz > 0) {
+            const cudaError_t e = cudaMemsetAsync(og->d_coo_vals, 0, (size_t)nnz * sizeof(float), st);
+            rc = e == cudaSuccess ? MVB_OK : set_err(MVB_ECUDA, "cheb_bwd_op: memset: %s", cudaGetErrorString(e));
+        }
+        if (rc) return rc;
+    }
+    if (rows_in > 0 && dx) {
         // empty rows: dX = dY (sum_k c_k W_k)^T
         ContractArgs a{};
         a.rows = rows_in;

@@ -154,9 +154,20 @@ int launch_spmm(int n_rows, int n_src_rows, const int32_t *rowptr, const int32_t
 int launch_cheb_recurrence(int n, int nnz, int K, const int32_t *rowptr, const int32_t *colidx, const float *vals,
                            const float *t0, float *planes, int64_t ncols, cudaStream_t st);
 // its reverse: in place on the K planes P (G_k overwrites P_k), G_{K-1} = P_{K-1}, G_k = P_k + 2 L^T G_{k+1} - G_{k+2}
-// (k >= 1), dx = P_0 + L^T G_1 - G_2 (dx = P_0 when K == 1); CSR(L^T) in rowptr_t / colidx_t / vals_t
+// (k >= 1), dx = P_0 + L^T G_1 - G_2 (dx = P_0 when K == 1); CSR(L^T) in rowptr_t / colidx_t / vals_t.
+// keep_planes: G_1..G_{K-1} must be left in P for the caller (the step kernels: the fused kernel keeps them in shared
+// memory); dx may then be NULL, and the last step is skipped.
 int launch_cheb_recurrence_bwd(int n, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
-                               float *P, float *dx, int64_t ncols, cudaStream_t st);
+                               float *P, float *dx, int64_t ncols, cudaStream_t st, bool keep_planes = false);
+
+// mvb_opgrad.cu: vals[j] = coo_vals[perm[j]], vals_t[j] = coo_vals[perm_t[j]]
+int launch_csr_values(int nnz, const int32_t *perm, const int32_t *perm_t, const float *coo_vals, float *vals,
+                      float *vals_t, cudaStream_t st);
+// d_coo[perm[j]] = <G_1[r], T_0[c]> + 2 sum_{k=2}^{K-1} <G_k[r], T_{k-1}[c]> for CSR(L) entry j = (r, c), r < n_rows;
+// G: K planes [n_rows, ncols] (plane k = G_k, k >= 1), T_0 = x, T_k = basis plane k-1.  K >= 2.
+int launch_cheb_edge_grad(int n_rows, int64_t ncols, int K, const int32_t *rowptr, const int32_t *colidx,
+                          const int32_t *perm, const float *x, const float *basis, const float *G, float *d_coo,
+                          cudaStream_t st);
 
 // Generic small-matrix contraction over the rows of vertex-major activations:
 //   out[p_out][row][j] = act( sum_{p_in,i} in[p_in][row][i] * Wm[p_in*in_w + i][p_out*out_w + j] + bias )

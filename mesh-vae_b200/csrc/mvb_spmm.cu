@@ -401,16 +401,19 @@ int launch_cheb_recurrence(int n, int nnz, int K, const int32_t *rowptr, const i
 }
 
 int launch_cheb_recurrence_bwd(int n, int nnz, int K, const int32_t *rowptr_t, const int32_t *colidx_t, const float *vals_t,
-                               float *P, float *dx, int64_t ncols, cudaStream_t st) {
+                               float *P, float *dx, int64_t ncols, cudaStream_t st, bool keep_planes) {
     const int64_t plane = (int64_t)n * ncols;
     if (K == 1) {
+        if (!dx) return MVB_OK;
         const cudaError_t e = cudaMemcpyAsync(dx, P, (size_t)plane * sizeof(float), cudaMemcpyDeviceToDevice, st);
         if (e != cudaSuccess) return set_err(MVB_ECUDA, "cheb_bwd: memcpy: %s", cudaGetErrorString(e));
         return MVB_OK;
     }
-    const int fused = launch_cheb_recur_bwd(n, nnz, K, rowptr_t, colidx_t, vals_t, P, dx, ncols, st);
-    if (fused) return fused < 0 ? fused : MVB_OK;
-    for (int k = K - 2; k >= 0; --k) {
+    if (!keep_planes) {
+        const int fused = launch_cheb_recur_bwd(n, nnz, K, rowptr_t, colidx_t, vals_t, P, dx, ncols, st);
+        if (fused) return fused < 0 ? fused : MVB_OK;
+    }
+    for (int k = K - 2; k >= (dx ? 0 : 1); --k) {
         float *pk = P + (int64_t)k * plane;
         const float *gk1 = P + (int64_t)(k + 1) * plane;
         const float *gk2 = (k + 2 <= K - 1) ? P + (int64_t)(k + 2) * plane : nullptr;

@@ -69,10 +69,12 @@ def from_vertex_major(x_vm: torch.Tensor) -> torch.Tensor:
 
 
 class _ChebConvFn(torch.autograd.Function):
-    """mvb_cheb_fwd / mvb_cheb_bwd  (nn/conv.py:557-577 and its autograd)."""
+    """mvb_cheb_fwd / mvb_cheb_bwd  (nn/conv.py:557-577 and its autograd).  With `norm` (the COO values of an
+    operators.EdgePattern) the operator is bound to those values here, and when `norm` needs a gradient the backward
+    pass is mvb_cheb_bwd_op, which also returns d_norm."""
 
     @staticmethod
-    def forward(ctx, x_vm, weight, bias, op: MeshOperator, relu: bool):
+    def forward(ctx, x_vm, weight, bias, op, relu: bool, norm=None):
         _req_cuda(x_vm, "cheb_conv x")
         _req_cuda(weight, "cheb_conv weight")
         n, b, fin = x_vm.shape
@@ -81,6 +83,8 @@ class _ChebConvFn(torch.autograd.Function):
             raise _lib.MvbError(f"cheb_conv: x has {fin} features, weight expects {fin_w}")
         if op.n_rows != n or op.n_cols != n:
             raise _lib.MvbError(f"cheb_conv: operator is {op.n_rows}x{op.n_cols}, tensor has {n} vertices")
+        if norm is not None:
+            op = op.bind(norm)
         x_vm = x_vm.contiguous()
         w = weight.contiguous()
         bb = None if bias is None else bias.contiguous()
@@ -92,8 +96,10 @@ class _ChebConvFn(torch.autograd.Function):
               "mvb_cheb_fwd")
         ctx.op, ctx.relu, ctx.has_bias = op, relu, bias is not None
         ctx.sinks = (_sink(weight), _sink(bias))
-        # the adjoint-form backward recomputes its planes from dY: the forward basis is then a temporary
-        keep = bool(lib.mvb_cheb_bwd_uses_basis(fin, fout, 1 if ctx.needs_input_grad[0] else 0))
+        ctx.op_grad = norm is not None and ctx.needs_input_grad[5]
+        # the adjoint-form backward recomputes its planes from dY: the forward basis is then a temporary (the operator
+        # gradient reads it: always the basis form)
+        keep = ctx.op_grad or bool(lib.mvb_cheb_bwd_uses_basis(fin, fout, 1 if ctx.needs_input_grad[0] else 0))
         ctx.save_for_backward(x_vm, basis if keep else None, w, y if relu else None)
         return y
 
@@ -108,19 +114,33 @@ class _ChebConvFn(torch.autograd.Function):
         dx = torch.empty_like(x_vm) if need_dx else None
         dw, db = _grad_outs(ctx.sinks, w, fout if ctx.has_bias else None)
         na = op.n_active
+        basis_p = ptr(basis) if (basis is not None and basis.numel()) else None
+        if ctx.op_grad:
+            d_norm = torch.empty(op.nnz, device=w.device, dtype=torch.float32)
+            ws_bytes = lib.mvb_cheb_bwd_op_workspace_bytes(n, b, fin, fout, k, na)
+            ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
+            check(lib.mvb_cheb_bwd_op(n, b, fin, fout, k, na, op.nnz, ptr(op.rowptr), ptr(op.colidx), ptr(op.perm),
+                                      ptr(op.rowptr_t), ptr(op.colidx_t), ptr(op.vals_t), ptr(x_vm), basis_p, ptr(w),
+                                      ptr(y) if ctx.relu else None, ptr(dy), ptr(dx), ptr(dw), ptr(db), ptr(d_norm), ptr(ws),
+                                      ws_bytes, stream_ptr()), "mvb_cheb_bwd_op")
+            return dx, *_ret(ctx.sinks, dw, db), None, None, d_norm
         ws_bytes = lib.mvb_cheb_bwd_workspace_bytes(n, b, fin, fout, k, na, 1 if need_dx else 0)
         ws = torch.empty(ws_bytes, device=w.device, dtype=torch.uint8)
         check(lib.mvb_cheb_bwd(n, b, fin, fout, k, na, op.nnz, ptr(op.rowptr_t), ptr(op.colidx_t), ptr(op.vals_t), ptr(x_vm),
-                               ptr(basis) if (basis is not None and basis.numel()) else None, ptr(w), ptr(y) if ctx.relu else None,
+                               basis_p, ptr(w), ptr(y) if ctx.relu else None,
                                ptr(dy), ptr(dx),
                                ptr(dw), ptr(db), ptr(ws), ws_bytes, stream_ptr()), "mvb_cheb_bwd")
         _park_or_join(ctx, (ws, x_vm, basis, w, y, dy, dw, db))
-        return dx, *_ret(ctx.sinks, dw, db), None, None
+        return dx, *_ret(ctx.sinks, dw, db), None, None, None
 
 
 def cheb_conv(x_vm: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], op: MeshOperator,
-              relu: bool = False, pad_to_quads: bool = True, keep_padding: bool = False) -> torch.Tensor:
+              relu: bool = False, pad_to_quads: bool = True, keep_padding: bool = False,
+              norm: Optional[torch.Tensor] = None) -> torch.Tensor:
     """x_vm [N,B,Fin] -> [N,B,Fout] (vertex-major in, vertex-major out).
+
+    With `norm` (fp32 [nnz], COO order), `op` is an operators.EdgePattern and norm its values: the result is
+    differentiable with respect to norm.
 
     Feature widths that are not a multiple of 4 (the 3-channel mesh coordinates at the encoder
     input and the decoder output) are zero-padded to the next multiple of 4 around the kernel call,
@@ -133,12 +153,12 @@ def cheb_conv(x_vm: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Ten
         raise _lib.MvbError(f"cheb_conv: x has {fin_x} features, weight expects {fin}")
     pin, pout = (-fin) % 4, (-fout) % 4
     if not pad_to_quads or (pin == 0 and pout == 0):
-        return _ChebConvFn.apply(x_vm, weight, bias, op, relu)
+        return _ChebConvFn.apply(x_vm, weight, bias, op, relu, norm)
     if pin and fin_x == fin:             # (an input packed by pack_input already carries the zero column)
         x_vm = torch.nn.functional.pad(x_vm, (0, pin))
     w = torch.nn.functional.pad(weight, (0, pout, 0, pin))
     b = bias if (bias is None or pout == 0) else torch.nn.functional.pad(bias, (0, pout))
-    y = _ChebConvFn.apply(x_vm, w, b, op, relu)
+    y = _ChebConvFn.apply(x_vm, w, b, op, relu, norm)
     if pout and keep_padding:
         return y                         # [N,B,fout+pout]: the caller slices a view and hands the padded buffer to the loss
     return y[..., :fout] if pout else y
