@@ -63,10 +63,17 @@ int mvb_tune(const char *spec);
  *   lane 0: mvb_cheb_bwd in the adjoint form (mvb_cheb_bwd_uses_basis == 0), mvb_cheb_layer_bwd when its tensor-core
  *           kernel runs, mvb_cheb_stream_bwd;
  *   lane 1: mvb_linear_bwd with dx (its dW / db tiles run as a launch of their own).
- * No other call defers.  The caller must
- * (1) keep every buffer of the call (workspace, x, dweight, dbias) alive and untouched until it has called
- * mvb_side_join(stream), which makes `stream` wait for the pending chain, and (2) call it before reading any gradient
- * and before a stream capture ends.  Default off: every call joins before it returns. */
+ * No other call defers.  The pending chain of each call reads or writes:
+ *   mvb_cheb_bwd (adjoint form): workspace, x, dweight, and dy when y_for_relu is NULL (without ReLU the chain reduces
+ *           dy itself; with it, the masked copy in the workspace) - dbias is reduced on `stream` before the call returns;
+ *   mvb_cheb_layer_bwd, mvb_cheb_stream_bwd: workspace, dweight, dbias, and x when there is no U prologue (with one,
+ *           the up-sampled T_0 in the workspace);
+ *   mvb_linear_bwd: x, y, gy, dW, db.
+ * The caller must (1) keep those buffers alive and untouched until it has called mvb_side_join(stream), which makes
+ * `stream` wait for the pending chain (the Python package parks them, with the call's other buffers, in
+ * _lib._deferred["keep"]), and (2) call it before reading any gradient and before a stream capture ends.  Default off:
+ * every call joins before it returns.  Deferred or not, with PDL or without, captured or not, the results are the same
+ * bits (tests/test_gpu_step_modes.py). */
 int mvb_side_join(void *stream);
 /* the same for one lane of chains: 0 = convolution weight gradients, 1 = dense-layer weight gradients (mvb_linear_bwd) */
 int mvb_side_join_lane(void *stream, int lane);
