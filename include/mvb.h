@@ -230,6 +230,36 @@ int mvb_vae_loss_bwd(int B, int N, int C, int Z, int ncls, const float *dnll, co
                      const double *gloss, float *d_recon, float *d_mu, float *d_logvar,
                      float *d_yhat, void *stream);
 
+/* sigma-VAE decoder likelihood (Rybkin et al., "Simple and Effective VAE Training with Calibrated Decoders"): the same
+ * loss with a decoder log sigma that is computed on the device instead of passed by the host.  With
+ * sc(t) = -6 + softplus(t + 6), n = N*C and SSE = sum_b SSE_b the batch's squared error sum_(b,v,c) (recon - x_gt)^2:
+ *   sigma_mode MVB_SIGMA_OPTIMAL: log sigma = sc(0.5 log(SSE / (B n)))  (the gradient flows through sigma);
+ *   sigma_mode MVB_SIGMA_LEARNED: log sigma = sc(*s_param), s_param a DEVICE fp32 scalar (a parameter);
+ *   rec[b] = 0.5 SSE_b / sigma^2 + n (log sigma + 0.5 log(2 pi)), fp64 arithmetic after the per-element squares
+ *   (fp64 squares of differences taken in fp64 when x_gt is fp64, in fp32 otherwise).
+ * Arguments and other outputs as mvb_vae_loss_fwd, except dnll = recon - x_gt UNSCALED (zero in the padding).
+ * sigma_state: 8 fp64 of device memory written by the forward call, read by the backward call:
+ *   [0] log sigma, [1] sigma^-2, [2] SSE, [3] sc'(t) = sigmoid(t + 6), [4] coef (below),
+ *   [5] d(sum_b rec_b)/dt = (B n - SSE sigma^-2) sc'(t), [6..7] unused.
+ * A perfect reconstruction (SSE = 0) under the optimal sigma gives t = -inf: log sigma = -6, sc' = 0, finite results.
+ * No host round trip, no atomics: capturable, and bit-reproducible run to run.  The fixed-sigma entry points above are
+ * unaffected. */
+#define MVB_SIGMA_OPTIMAL 1
+#define MVB_SIGMA_LEARNED 2
+int mvb_vae_loss_sigma_fwd(int B, int N, int C, int Z, int ncls, const float *recon, int recon_ld, const void *x_gt,
+                           int x_is_f64, const float *mu, const float *logvar, const float *y_hat, const int64_t *y,
+                           int sigma_mode, const float *s_param, double *sigma_state, double *loss, float *kld,
+                           double *rec, int64_t *correct, float *dnll, void *workspace, size_t workspace_bytes,
+                           void *stream);
+/* d_recon = gloss/B * coef * dnll with coef = sigma^-2 (learned) or sigma^-2 + (B n - SSE sigma^-2) sc'/SSE (optimal,
+ * SSE > 0; sigma^-2 when SSE = 0); d_mu, d_logvar, d_yhat as mvb_vae_loss_bwd; d_s (fp32 scalar, learned sigma) =
+ * gloss/B * (B n - SSE sigma^-2) sc'(s), written (not accumulated): it may point into a flat gradient buffer.  C is the
+ * entry width of dnll.  Any output pointer may be NULL. */
+int mvb_vae_loss_sigma_bwd(int B, int N, int C, int Z, int ncls, const float *dnll, const double *sigma_state,
+                           const float *mu, const float *logvar, const float *y_hat, const int64_t *y,
+                           const double *gloss, float *d_recon, float *d_mu, float *d_logvar, float *d_yhat,
+                           float *d_s, void *stream);
+
 /* ---- logpdf.py drop-ins used when the reference's own loss_function runs unchanged ----------
  * KLD (logpdf.py:7-8): out[b] = -0.5 sum_j (1 + logvar - mu^2 - exp(logvar)); bwd as above.
  * gaussian_nll (logpdf.py:22-23), elementwise on n values with scalar log_sigma:
@@ -242,6 +272,17 @@ int mvb_gaussian_nll_fwd(int64_t n, const float *mu, const void *x, int x_is_f64
                          void *out, void *stream);
 int mvb_gaussian_nll_bwd(int64_t n, const float *mu, const void *x, int x_is_f64, float log_sigma,
                          const void *gout, float *d_mu, void *stream);
+/* gaussian_nll with log_sigma a DEVICE scalar, fp64 (ls_is_f64 != 0) or fp32 (a learned or batch-derived sigma, read
+ * without a host sync): sigma = exp(log_sigma) in the scalar's precision, as torch forms log_sigma.exp() (the fp32 exp
+ * correctly rounded), then converted to the arithmetic's precision (that of x).  The backward pass also returns
+ * d_log_sigma[0] (fp64) = sum_i g_i (1 - ((x_i - mu_i)/sigma)^2) from per-block partials and an ordered sum:
+ * deterministic.  workspace: mvb_gaussian_nll_sigma_workspace_bytes(n) bytes. */
+int mvb_gaussian_nll_sigma_fwd(int64_t n, const float *mu, const void *x, int x_is_f64, const void *log_sigma,
+                               int ls_is_f64, void *out, void *stream);
+size_t mvb_gaussian_nll_sigma_workspace_bytes(int64_t n);
+int mvb_gaussian_nll_sigma_bwd(int64_t n, const float *mu, const void *x, int x_is_f64, const void *log_sigma,
+                               int ls_is_f64, const void *gout, float *d_mu, double *d_log_sigma, void *workspace,
+                               size_t workspace_bytes, void *stream);
 
 /* ---- input hand-off: mesh-major batch -> zero-padded vertex-major planes --------------------
  * out[n, b, 0:Cp] = (x[b, n, 0:C], 0...)   x [B,N,C] as the loader delivers it (models/cheb_VAE.py:195-200

@@ -64,10 +64,15 @@ SIGNATURES = {
     "mvb_vae_loss_fwd": (c_int, [c_int, c_int, c_int, c_int, c_int, _vp, c_int, _vp, c_int, _vp, _vp, _vp, _vp, c_float,
                                  _vp, _vp, _vp, _vp, _vp, _vp, c_size_t, _vp]),
     "mvb_vae_loss_bwd": (c_int, [c_int, c_int, c_int, c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mvb_vae_loss_sigma_fwd": (c_int, [c_int] * 5 + [_vp, c_int, _vp, c_int] + [_vp] * 4 + [c_int] + [_vp] * 8 + [c_size_t, _vp]),
+    "mvb_vae_loss_sigma_bwd": (c_int, [c_int] * 5 + [_vp] * 13),
     "mvb_kld_fwd": (c_int, [c_int, c_int, _vp, _vp, _vp, _vp]),
     "mvb_kld_bwd": (c_int, [c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mvb_gaussian_nll_fwd": (c_int, [c_int64, _vp, _vp, c_int, c_float, _vp, _vp]),
     "mvb_gaussian_nll_bwd": (c_int, [c_int64, _vp, _vp, c_int, c_float, _vp, _vp, _vp]),
+    "mvb_gaussian_nll_sigma_fwd": (c_int, [c_int64, _vp, _vp, c_int, _vp, c_int, _vp, _vp]),
+    "mvb_gaussian_nll_sigma_workspace_bytes": (c_size_t, [c_int64]),
+    "mvb_gaussian_nll_sigma_bwd": (c_int, [c_int64, _vp, _vp, c_int, _vp, c_int, _vp, _vp, _vp, _vp, c_size_t, _vp]),
     "mvb_cheb_sel_supported": (c_int, [c_int] * 6),
     "mvb_cheb_sel_fwd": (c_int, [c_int] * 6 + [_vp] * 6 + [c_int, c_int] + [_vp] * 4),
     "mvb_cheb_sel_bwd_workspace_bytes": (c_size_t, [c_int] * 3),

@@ -63,7 +63,11 @@ class cheb_VAE(nn.Module):
         self.reset_parameters()
         self.type = model
         self.noise = "cpu"
+        # decoder Gaussian log sigma: the reference's constant (quirk 6; `model` above does not change it, as in the
+        # reference), or a sigma-VAE variant chosen with set_decoder_sigma
+        self.sigma_mode = "fixed"
         self.log_sigma = Fn.LOG_SIGMA_DEFAULT
+        self.last_log_sigma = None
         # fused dense bottleneck (row f2): one launch per Linear(+ReLU+dropout), one for the three heads
         self.fused_dense = True
         # coarse levels: pool + conv + ReLU (+ pool) as one mesh-resident kernel (Fn.cheb_layer)
@@ -73,6 +77,26 @@ class cheb_VAE(nn.Module):
         self.encoder_conv_out = None
         self.A_num_nodes = tuple(int(n) for n in num_nodes)
         self.dropout_stream = Fn.DropoutStream()
+
+    def set_decoder_sigma(self, mode: str, init: float = 0.0):
+        """The decoder likelihood's log sigma (Rybkin et al., "Simple and Effective VAE Training with Calibrated Decoders"):
+          "fixed"   - the reference's constant softclip(1, -6) (models/cheb_VAE.py:328-329), the default;
+          "optimal" - the batch's optimal sigma, sc(0.5 log(SSE / (B N C))), sc(t) = -6 + softplus(t + 6), computed on
+                      the device in the loss epilogue, with its gradient;
+          "learned" - sc(s) with s a scalar Parameter `log_sigma` initialised to `init`, trained with the others.
+        Only "learned" adds a state-dict key (`log_sigma`).  Choose the mode before an engine.TrainEngine is built on the
+        model: the engine lays out its flat parameter buffer from the parameters it finds then."""
+        if mode not in ("fixed", "optimal", "learned"):
+            raise ValueError(f"set_decoder_sigma: mode is 'fixed', 'optimal' or 'learned', got {mode!r}")
+        if "log_sigma" in self._parameters:
+            del self._parameters["log_sigma"]
+        if mode == "learned":
+            dev = next(self.parameters()).device
+            self.log_sigma = nn.Parameter(torch.full((), float(init), device=dev, dtype=torch.float32))
+        else:
+            self.log_sigma = Fn.LOG_SIGMA_DEFAULT if mode == "fixed" else "optimal"
+        self.sigma_mode = mode
+        self.last_log_sigma = None
 
     def reset_parameters(self):
         nn.init.normal_(self.enc_lin.weight, 0, 0.1)
@@ -186,12 +210,18 @@ class cheb_VAE(nn.Module):
         return Fn.reparameterize(mu, logvar, eps)
 
     def loss_function(self, x, recon_x, z, mu_z, logvar_z, y, y_hat):
+        """as the reference's; with a sigma-VAE decoder sigma the log sigma used is left in `last_log_sigma` (fp64 0-dim
+        device tensor)"""
         padded, self._recon_padded = self._recon_padded, None           # one-shot hand-over from decoder()
         if padded is not None and recon_x.data_ptr() == padded.data_ptr() and recon_x.shape[1] == padded.shape[0]:
-            loss, kld, rec, correct = Fn.vae_loss(padded, x, mu_z, logvar_z, y_hat, y, self.log_sigma,
-                                                  channels=recon_x.shape[2])
+            recon_vm, channels = padded, recon_x.shape[2]
         else:
-            loss, kld, rec, correct = Fn.vae_loss(Fn.to_vertex_major(recon_x), x, mu_z, logvar_z, y_hat, y, self.log_sigma)
+            recon_vm, channels = Fn.to_vertex_major(recon_x), None
+        out = Fn.vae_loss(recon_vm, x, mu_z, logvar_z, y_hat, y, self.log_sigma, channels=channels,
+                          return_log_sigma=self.sigma_mode != "fixed")
+        loss, kld, rec, correct = out[:4]
+        if self.sigma_mode != "fixed":
+            self.last_log_sigma = out[4]
         return loss, correct, kld, rec
 
     def forward_recon(self, data, y, m_type="test", eps: Optional[torch.Tensor] = None):

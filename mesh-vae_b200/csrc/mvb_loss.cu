@@ -7,6 +7,9 @@
 // global reads are coalesced, emits (recon - x)/sigma^2 for the backward pass in the same sweep
 // and reduces the NLL per mesh with a fixed-order warp reduction -> per-(vertex-chunk, mesh)
 // partials -> ordered final sum.  No atomics anywhere, bit-reproducible run to run.
+// The sigma-VAE variants (optimal and learned decoder sigma) share the partial kernel: it then sums the squared error per
+// mesh and keeps recon - x unscaled, and their finalize kernel derives log sigma on the device from the batch's error or
+// from a parameter (no host round trip: a captured step follows new inputs and Adam's updates of the parameter).
 // Roofline: HBM; algorithmic bytes = N*B*C*(4 + sizeof(x) + 4).
 #include "mvb_internal.cuh"
 
@@ -19,7 +22,9 @@ struct AccT { typedef float type; };
 template <>
 struct AccT<double> { typedef double type; };
 
-template <typename XT>
+// SSE = false: partial = sum of the NLL terms, dnll = (recon - x)/sigma^2 (the reference's constant sigma);
+// SSE = true: partial = sum of (recon - x)^2 (fp64 squares), dnll = recon - x (sigma is not known yet)
+template <typename XT, bool SSE>
 __global__ void __launch_bounds__(256)
 vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const float *__restrict__ recon,
                        const XT *__restrict__ xgt, float log_sigma, float sigma,
@@ -81,10 +86,15 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
             const int v = e / C, c = e - v * C;
             float *rp = Rs + v * (BCH * ld) + b * ld + c;
             const AT d = (AT)(*rp) - (AT)Xs[b * (VCH * C) + e];   // recon - x
-            const AT t = d * inv_sg;
-            const AT nll = (AT)0.5 * t * t + cst;
-            s += (double)nll;
-            *rp = (float)(d * inv_sg2);
+            if constexpr (SSE) {
+                s = fma((double)d, (double)d, s);
+                *rp = (float)d;
+            } else {
+                const AT t = d * inv_sg;
+                const AT nll = (AT)0.5 * t * t + cst;
+                s += (double)nll;
+                *rp = (float)(d * inv_sg2);
+            }
         }
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
@@ -108,15 +118,30 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
     }
 }
 
+// log sigma = sc(t) = -6 + softplus(t + 6) and sc'(t) = sigmoid(t + 6), both from exp(-|t + 6|): finite for every t,
+// t = -inf (a perfect reconstruction under the optimal sigma) included, where they are -6 and 0
+__device__ __forceinline__ void softclip_m6(double t, double &log_sigma, double &dsc) {
+    const double u = t + 6.0, e = exp(-fabs(u));
+    log_sigma = -6.0 + fmax(u, 0.0) + log1p(e);
+    dsc = (u >= 0.0 ? 1.0 : e) / (1.0 + e);
+}
+
+// SIGMA = false: the reference's constant sigma (the partials are NLL sums).  SIGMA = true: the partials are squared
+// errors; after phase 1 the block sums the per-mesh SSE_b in a fixed order, derives log sigma (sigma_mode 1: optimal,
+// from the batch's SSE; 2: learned, sc(*s_param)) and writes the state the backward pass reads, then phase 2 turns
+// SSE_b into rec_b = SSE_b / (2 sigma^2) + n_elem (log sigma + log(2 pi)/2).
+template <bool SIGMA>
 __global__ void __launch_bounds__(1024)
 vae_loss_finalize_kernel(int B, int Z, int ncls, int nchunks, const double *__restrict__ partial,
                          const float *__restrict__ mu, const float *__restrict__ logvar,
                          const float *__restrict__ y_hat, const int64_t *__restrict__ y,
-                         double *loss, float *kld, double *rec, int64_t *correct) {
+                         double *loss, float *kld, double *rec, int64_t *correct,
+                         int sigma_mode, double n_elem, const float *__restrict__ s_param, double *sigma_state) {
     pdl_trigger();
     pdl_wait();
     __shared__ double s_sum[1024];
     __shared__ int s_cnt[1024];
+    __shared__ double s_sig[2];
     const int tid = threadIdx.x;
     double lsum = 0.0;
     int lcnt = 0;
@@ -139,6 +164,35 @@ vae_loss_finalize_kernel(int B, int Z, int ncls, int nchunks, const double *__re
         if (lane == 0) rec[b] = r;
     }
     __syncthreads();
+    if constexpr (SIGMA) {
+        double e = 0.0;
+        for (int b = tid; b < B; b += blockDim.x) e += rec[b];
+        s_sum[tid] = e;
+        __syncthreads();
+        for (int off = blockDim.x >> 1; off > 0; off >>= 1) {
+            if (tid < off) s_sum[tid] += s_sum[tid + off];
+            __syncthreads();
+        }
+        if (tid == 0) {
+            const double sse = s_sum[0], bn = (double)B * n_elem;
+            const double t = sigma_mode == 1 ? (sse > 0.0 ? 0.5 * log(sse / bn) : -INFINITY) : (double)*s_param;
+            double ls, dsc;
+            softclip_m6(t, ls, dsc);
+            const double inv_s2 = exp(-2.0 * ls);
+            const double g_t = (bn - sse * inv_s2) * dsc;         // d(sum_b rec_b)/dt
+            sigma_state[0] = ls;
+            sigma_state[1] = inv_s2;
+            sigma_state[2] = sse;
+            sigma_state[3] = dsc;
+            // d(sum_b rec_b)/d(recon - x) = coef (recon - x): the optimal sigma adds its own dependence on the error
+            // (dt/d(recon - x) = (recon - x)/SSE); a zero SSE has t = -inf and sc' = 0, so nothing is added
+            sigma_state[4] = (sigma_mode == 1 && sse > 0.0) ? inv_s2 + g_t / sse : inv_s2;
+            sigma_state[5] = g_t;
+            s_sig[0] = ls;
+            s_sig[1] = inv_s2;
+        }
+        __syncthreads();
+    }
     // phase 2: 16 lanes per mesh for the per-mesh terms (the latent sums are lane-strided + a fixed xor tree; a single
     // thread per mesh walked 2 Z dependent global loads)
     constexpr int G = 16;
@@ -155,7 +209,11 @@ vae_loss_finalize_kernel(int B, int Z, int ncls, int nchunks, const double *__re
 #pragma unroll
         for (int off = G / 2; off > 0; off >>= 1) k += __shfl_xor_sync(0xffffffffu, k, off);
         if (!ok || sub != 0) continue;
-        const double r = rec[b];
+        double r = rec[b];
+        if constexpr (SIGMA) {
+            r = 0.5 * r * s_sig[1] + n_elem * (s_sig[0] + MVB_HALF_LOG_2PI);
+            rec[b] = r;
+        }
         k *= -0.5f;
         kld[b] = k;
         float q = 0.f;
@@ -189,18 +247,21 @@ vae_loss_finalize_kernel(int B, int Z, int ncls, int nchunks, const double *__re
     }
 }
 
+// COEF: the sigma-VAE backward, dst = (gloss/B * coef) src with coef from the forward pass's sigma state
+template <bool COEF>
 __global__ void scale_by_gloss_kernel(int64_t n, const float *__restrict__ src,
-                                      const double *__restrict__ gloss, double inv_b, float *dst) {
-    const float s = (float)(*gloss * inv_b);
+                                      const double *__restrict__ gloss, double inv_b, const double *__restrict__ coef, float *dst) {
+    const float s = COEF ? (float)(*gloss * inv_b * *coef) : (float)(*gloss * inv_b);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         dst[i] = s * src[i];
 }
 
+template <bool COEF>
 __global__ void scale4_by_gloss_kernel(int64_t n4, const float4 *__restrict__ src,
-                                       const double *__restrict__ gloss, double inv_b, float4 *dst) {
+                                       const double *__restrict__ gloss, double inv_b, const double *__restrict__ coef, float4 *dst) {
     pdl_trigger();
     pdl_wait();
-    const float s = (float)(*gloss * inv_b);
+    const float s = COEF ? (float)(*gloss * inv_b * *coef) : (float)(*gloss * inv_b);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         const float4 v = __ldg(src + i);
         dst[i] = make_float4(s * v.x, s * v.y, s * v.z, s * v.w);
@@ -212,11 +273,12 @@ __global__ void vae_loss_bwd_small_kernel(int B, int Z, int ncls, const float *_
                                           const float *__restrict__ y_hat,
                                           const int64_t *__restrict__ y,
                                           const double *__restrict__ gloss, float *d_mu,
-                                          float *d_logvar, float *d_yhat) {
+                                          float *d_logvar, float *d_yhat, const double *__restrict__ d_t, float *d_s) {
     pdl_trigger();
     pdl_wait();
     const float s = (float)(*gloss / (double)B);
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d_s && i == 0) *d_s = (float)(*gloss / (double)B * *d_t);        // learned sigma: gloss/B * d(sum_b rec_b)/ds
     if (i < B * Z) {
         if (d_mu) d_mu[i] = s * mu[i];
         if (d_logvar) d_logvar[i] = s * 0.5f * (expf(logvar[i]) - 1.f);
@@ -412,11 +474,23 @@ __global__ void kld_bwd_kernel(int B, int Z, const float *__restrict__ mu,
     if (d_logvar) d_logvar[i] = g * 0.5f * (expf(logvar[i]) - 1.f);
 }
 
+// log sigma read from device memory (fp64 when ls_f64, else fp32) and sigma = its exp as torch forms log_sigma.exp(): in
+// the scalar's own precision (the fp32 exp correctly rounded from fp64), then converted to the arithmetic's type
+template <typename AT>
+__device__ __forceinline__ void device_sigma(const void *ls_dev, int ls_f64, AT &ls, AT &sg) {
+    const double l = ls_f64 ? *reinterpret_cast<const double *>(ls_dev) : (double)*reinterpret_cast<const float *>(ls_dev);
+    ls = (AT)l;
+    sg = ls_f64 ? (AT)exp(l) : (AT)(float)exp(l);
+}
+
+// ls_dev: log sigma from device memory (device_sigma); NULL: log_sigma / sigma from the host
 template <typename XT>
 __global__ void nll_fwd_kernel(int64_t n, const float *__restrict__ mu, const XT *__restrict__ x,
-                               float log_sigma, float sigma, XT *out) {
+                               float log_sigma, float sigma, const void *__restrict__ ls_dev, int ls_f64, XT *out) {
     typedef typename AccT<XT>::type AT;
-    const AT sg = (AT)sigma, cst = (AT)log_sigma + (AT)MVB_HALF_LOG_2PI;
+    AT ls = (AT)log_sigma, sg = (AT)sigma;
+    if (ls_dev) device_sigma(ls_dev, ls_f64, ls, sg);
+    const AT cst = ls + (AT)MVB_HALF_LOG_2PI;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const AT t = ((AT)x[i] - (AT)mu[i]) / sg;
         out[i] = (XT)((AT)0.5 * t * t + cst);
@@ -429,6 +503,46 @@ __global__ void nll_bwd_kernel(int64_t n, const float *__restrict__ mu, const XT
     const AT sg2 = (AT)sigma * (AT)sigma;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         d_mu[i] = (float)((AT)gout[i] * ((AT)mu[i] - (AT)x[i]) / sg2);
+}
+
+// gaussian_nll backward with a device log sigma: d_mu as nll_bwd_kernel, and per-block partials of
+// d log_sigma = sum_i g_i (1 - ((x_i - mu_i)/sigma)^2) (fp64, fixed grid-stride order and tree) for an ordered finalize
+template <typename XT>
+__global__ void __launch_bounds__(256)
+nll_sigma_bwd_kernel(int64_t n, const float *__restrict__ mu, const XT *__restrict__ x, const void *__restrict__ ls_dev,
+                     int ls_f64, const XT *__restrict__ gout, float *d_mu, double *__restrict__ partial) {
+    typedef typename AccT<XT>::type AT;
+    __shared__ double sh[256];
+    AT ls, sg;
+    device_sigma(ls_dev, ls_f64, ls, sg);
+    const AT sg2 = sg * sg;
+    double acc = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const AT g = (AT)gout[i], d = (AT)x[i] - (AT)mu[i];
+        d_mu[i] = (float)(-g * d / sg2);
+        const double t = (double)(d / sg);
+        acc += (double)g * (1.0 - t * t);
+    }
+    sh[threadIdx.x] = acc;
+    __syncthreads();
+    for (int off = 128; off > 0; off >>= 1) {
+        if (threadIdx.x < off) sh[threadIdx.x] += sh[threadIdx.x + off];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) partial[blockIdx.x] = sh[0];
+}
+
+__global__ void __launch_bounds__(256) ordered_sum_kernel(int n, const double *__restrict__ partial, double *out) {
+    __shared__ double sh[256];
+    double acc = 0.0;
+    for (int i = threadIdx.x; i < n; i += 256) acc += partial[i];
+    sh[threadIdx.x] = acc;
+    __syncthreads();
+    for (int off = 128; off > 0; off >>= 1) {
+        if (threadIdx.x < off) sh[threadIdx.x] += sh[threadIdx.x + off];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = sh[0];
 }
 
 static inline unsigned ew_grid(int64_t n, int threads) {
@@ -481,12 +595,13 @@ extern "C" int mvb_vae_loss_fwd(int B, int N, int C, int Z, int ncls, const floa
     const float sigma = expf(log_sigma);
     double *partial = reinterpret_cast<double *>(workspace);
     if (x_is_f64)
-        launch_pdl(vae_rec_partial_kernel<double>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const double *)x_gt, log_sigma, sigma, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<double, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const double *)x_gt, log_sigma, sigma, partial, dnll);
     else
-        launch_pdl(vae_rec_partial_kernel<float>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const float *)x_gt, log_sigma, sigma, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<float, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const float *)x_gt, log_sigma, sigma, partial, dnll);
     int rc = check_launch("mvb_vae_loss_fwd partial");
     if (rc) return rc;
-    launch_pdl(vae_loss_finalize_kernel, dim3(1), dim3(1024), 0, st, B, Z, ncls, nch, partial, mu, logvar, y_hat, y, loss, kld, rec, correct);
+    launch_pdl(vae_loss_finalize_kernel<false>, dim3(1), dim3(1024), 0, st, B, Z, ncls, nch, partial, mu, logvar, y_hat, y, loss, kld, rec,
+               correct, 0, 0.0, (const float *)nullptr, (double *)nullptr);
     return check_launch("mvb_vae_loss_fwd finalize");
 }
 
@@ -500,17 +615,79 @@ extern "C" int mvb_vae_loss_bwd(int B, int N, int C, int Z, int ncls, const floa
         MVB_REQUIRE(dnll, "vae_loss_bwd: dnll is null");
         const int64_t n = (int64_t)N * B * C;
         if (n % 4 == 0 && aligned16(dnll) && aligned16(d_recon))
-            launch_pdl(scale4_by_gloss_kernel, dim3(ew_grid(n / 4, 256)), dim3(256), 0, st, n / 4, (const float4 *)dnll, gloss, 1.0 / B, (float4 *)d_recon);
+            launch_pdl(scale4_by_gloss_kernel<false>, dim3(ew_grid(n / 4, 256)), dim3(256), 0, st, n / 4, (const float4 *)dnll, gloss, 1.0 / B,
+                       (const double *)nullptr, (float4 *)d_recon);
         else
-            scale_by_gloss_kernel<<<ew_grid(n, 256), 256, 0, st>>>(n, dnll, gloss, 1.0 / B, d_recon);
+            scale_by_gloss_kernel<false><<<ew_grid(n, 256), 256, 0, st>>>(n, dnll, gloss, 1.0 / B, nullptr, d_recon);
         int rc = check_launch("mvb_vae_loss_bwd recon");
         if (rc) return rc;
     }
     if (d_mu || d_logvar || d_yhat) {
         MVB_REQUIRE(mu && logvar && y_hat && y, "vae_loss_bwd: null latent pointers");
         const int n = B * (Z > 1 ? Z : 1);
-        launch_pdl(vae_loss_bwd_small_kernel, dim3((n + 127) / 128), dim3(128), 0, st, B, Z, ncls, mu, logvar, y_hat, y, gloss, d_mu, d_logvar, d_yhat);
+        launch_pdl(vae_loss_bwd_small_kernel, dim3((n + 127) / 128), dim3(128), 0, st, B, Z, ncls, mu, logvar, y_hat, y, gloss, d_mu, d_logvar, d_yhat,
+                   (const double *)nullptr, (float *)nullptr);
         return check_launch("mvb_vae_loss_bwd latent");
+    }
+    return MVB_OK;
+}
+
+extern "C" int mvb_vae_loss_sigma_fwd(int B, int N, int C, int Z, int ncls, const float *recon, int recon_ld,
+                                      const void *x_gt, int x_is_f64, const float *mu, const float *logvar,
+                                      const float *y_hat, const int64_t *y, int sigma_mode, const float *s_param,
+                                      double *sigma_state, double *loss, float *kld, double *rec, int64_t *correct,
+                                      float *dnll, void *workspace, size_t workspace_bytes, void *stream) {
+    MVB_REQUIRE(B > 0 && N > 0 && C > 0 && Z > 0 && ncls > 0, "vae_loss_sigma_fwd: bad sizes");
+    MVB_REQUIRE(recon_ld >= C, "vae_loss_sigma_fwd: recon_ld=%d < C=%d", recon_ld, C);
+    MVB_REQUIRE(sigma_mode == MVB_SIGMA_OPTIMAL || sigma_mode == MVB_SIGMA_LEARNED, "vae_loss_sigma_fwd: sigma_mode=%d", sigma_mode);
+    MVB_REQUIRE(sigma_mode != MVB_SIGMA_LEARNED || s_param, "vae_loss_sigma_fwd: learned sigma without s_param");
+    MVB_REQUIRE(recon && x_gt && mu && logvar && y_hat && y && sigma_state && loss && kld && rec && correct && dnll && workspace,
+                "vae_loss_sigma_fwd: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    int VCH, BCH;
+    size_t smem;
+    loss_tiles(C, recon_ld, x_is_f64 ? 8 : 4, VCH, BCH, smem);
+    MVB_REQUIRE(VCH >= 8, "vae_loss_sigma_fwd: C=%d too large", C);
+    const int nch = (N + VCH - 1) / VCH;
+    if ((size_t)nch * B * sizeof(double) > workspace_bytes)
+        return set_err(MVB_EWORKSPACE, "vae_loss_sigma_fwd: workspace %zu < %zu", workspace_bytes, (size_t)nch * B * sizeof(double));
+    dim3 grid(nch, (B + BCH - 1) / BCH);
+    double *partial = reinterpret_cast<double *>(workspace);
+    if (x_is_f64)
+        launch_pdl(vae_rec_partial_kernel<double, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const double *)x_gt, 0.f, 1.f, partial, dnll);
+    else
+        launch_pdl(vae_rec_partial_kernel<float, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const float *)x_gt, 0.f, 1.f, partial, dnll);
+    int rc = check_launch("mvb_vae_loss_sigma_fwd partial");
+    if (rc) return rc;
+    launch_pdl(vae_loss_finalize_kernel<true>, dim3(1), dim3(1024), 0, st, B, Z, ncls, nch, partial, mu, logvar, y_hat, y, loss, kld, rec,
+               correct, sigma_mode, (double)N * C, s_param, sigma_state);
+    return check_launch("mvb_vae_loss_sigma_fwd finalize");
+}
+
+extern "C" int mvb_vae_loss_sigma_bwd(int B, int N, int C, int Z, int ncls, const float *dnll, const double *sigma_state,
+                                      const float *mu, const float *logvar, const float *y_hat, const int64_t *y,
+                                      const double *gloss, float *d_recon, float *d_mu, float *d_logvar, float *d_yhat,
+                                      float *d_s, void *stream) {
+    MVB_REQUIRE(B > 0 && N > 0 && C > 0 && gloss && sigma_state, "vae_loss_sigma_bwd: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    const double *coef = sigma_state + 4, *d_t = sigma_state + 5;
+    if (d_recon) {
+        MVB_REQUIRE(dnll, "vae_loss_sigma_bwd: dnll is null");
+        const int64_t n = (int64_t)N * B * C;
+        if (n % 4 == 0 && aligned16(dnll) && aligned16(d_recon))
+            launch_pdl(scale4_by_gloss_kernel<true>, dim3(ew_grid(n / 4, 256)), dim3(256), 0, st, n / 4, (const float4 *)dnll, gloss, 1.0 / B, coef,
+                       (float4 *)d_recon);
+        else
+            scale_by_gloss_kernel<true><<<ew_grid(n, 256), 256, 0, st>>>(n, dnll, gloss, 1.0 / B, coef, d_recon);
+        int rc = check_launch("mvb_vae_loss_sigma_bwd recon");
+        if (rc) return rc;
+    }
+    if (d_mu || d_logvar || d_yhat || d_s) {
+        MVB_REQUIRE(mu && logvar && y_hat && y, "vae_loss_sigma_bwd: null latent pointers");
+        const int n = B * (Z > 1 ? Z : 1);
+        launch_pdl(vae_loss_bwd_small_kernel, dim3((n + 127) / 128), dim3(128), 0, st, B, Z, ncls, mu, logvar, y_hat, y, gloss, d_mu, d_logvar, d_yhat,
+                   d_t, d_s);
+        return check_launch("mvb_vae_loss_sigma_bwd latent");
     }
     return MVB_OK;
 }
@@ -550,9 +727,9 @@ extern "C" int mvb_gaussian_nll_fwd(int64_t n, const float *mu, const void *x, i
     if (n == 0) return MVB_OK;
     const float sigma = expf(log_sigma);
     if (x_is_f64)
-        nll_fwd_kernel<double><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const double *)x, log_sigma, sigma, (double *)out);
+        nll_fwd_kernel<double><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const double *)x, log_sigma, sigma, nullptr, 0, (double *)out);
     else
-        nll_fwd_kernel<float><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const float *)x, log_sigma, sigma, (float *)out);
+        nll_fwd_kernel<float><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const float *)x, log_sigma, sigma, nullptr, 0, (float *)out);
     return check_launch("mvb_gaussian_nll_fwd");
 }
 
@@ -566,6 +743,39 @@ extern "C" int mvb_gaussian_nll_bwd(int64_t n, const float *mu, const void *x, i
     else
         nll_bwd_kernel<float><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const float *)x, sigma, (const float *)gout, d_mu);
     return check_launch("mvb_gaussian_nll_bwd");
+}
+
+extern "C" int mvb_gaussian_nll_sigma_fwd(int64_t n, const float *mu, const void *x, int x_is_f64, const void *log_sigma,
+                                          int ls_is_f64, void *out, void *stream) {
+    MVB_REQUIRE(n >= 0 && mu && x && log_sigma && out, "gaussian_nll_sigma_fwd: bad arguments");
+    if (n == 0) return MVB_OK;
+    if (x_is_f64)
+        nll_fwd_kernel<double><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const double *)x, 0.f, 1.f, log_sigma, ls_is_f64,
+                                                                                   (double *)out);
+    else
+        nll_fwd_kernel<float><<<ew_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(n, mu, (const float *)x, 0.f, 1.f, log_sigma, ls_is_f64,
+                                                                                  (float *)out);
+    return check_launch("mvb_gaussian_nll_sigma_fwd");
+}
+
+extern "C" size_t mvb_gaussian_nll_sigma_workspace_bytes(int64_t n) { return (size_t)ew_grid(n, 256) * sizeof(double); }
+
+extern "C" int mvb_gaussian_nll_sigma_bwd(int64_t n, const float *mu, const void *x, int x_is_f64, const void *log_sigma,
+                                          int ls_is_f64, const void *gout, float *d_mu, double *d_log_sigma, void *workspace,
+                                          size_t workspace_bytes, void *stream) {
+    MVB_REQUIRE(n >= 0 && mu && x && log_sigma && gout && d_mu && d_log_sigma && workspace, "gaussian_nll_sigma_bwd: bad arguments");
+    const unsigned grid = ew_grid(n, 256);
+    MVB_REQUIRE(workspace_bytes >= (size_t)grid * sizeof(double), "gaussian_nll_sigma_bwd: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    double *partial = reinterpret_cast<double *>(workspace);
+    if (x_is_f64)
+        nll_sigma_bwd_kernel<double><<<grid, 256, 0, st>>>(n, mu, (const double *)x, log_sigma, ls_is_f64, (const double *)gout, d_mu, partial);
+    else
+        nll_sigma_bwd_kernel<float><<<grid, 256, 0, st>>>(n, mu, (const float *)x, log_sigma, ls_is_f64, (const float *)gout, d_mu, partial);
+    int rc = check_launch("mvb_gaussian_nll_sigma_bwd");
+    if (rc) return rc;
+    ordered_sum_kernel<<<1, 256, 0, st>>>((int)grid, partial, d_log_sigma);
+    return check_launch("mvb_gaussian_nll_sigma_bwd sum");
 }
 
 extern "C" size_t mvb_recon_error_workspace_bytes(int B, int N) { return (size_t)2 * ((N + 255) / 256) * B * sizeof(double); }

@@ -114,6 +114,11 @@ class TrainEngine:
         self.dev = next(net.parameters()).device
         self.batch = batch
         self.world = dist.get_world_size() if (dist.is_available() and dist.is_initialized()) else 1
+        self.sigma_mode = getattr(net, "sigma_mode", "fixed")
+        if self.sigma_mode == "optimal" and self.world > 1:
+            # each rank would derive sigma from its own shard's error, not from the global batch's
+            raise _lib.MvbError("TrainEngine: the optimal decoder sigma needs the whole batch's error; it is not supported "
+                                f"with {self.world} data-parallel ranks (use 'fixed' or 'learned')")
         self.distributed = (self.world > 1) if distributed is None else distributed
         self.graph_comm = graph_comm            # data parallel: capture the all-reduces inside the step graph
         self.one_graph = False
@@ -197,6 +202,10 @@ class TrainEngine:
                 p.grad = v                      # the sink IS the gradient
         self.loss = torch.zeros((), device=self.dev, dtype=torch.float64)
         self.kld = self.rec = self.correct = self.recon = None
+        # the decoder log sigma of the last step (fp64 0-dim device tensor): the constant, or the sigma-VAE one the loss
+        # epilogue derived (a tensor of the step graph, updated by every replay like kld / rec / correct)
+        self.log_sigma = None if self.sigma_mode != "fixed" else \
+            torch.full((), float(torch.tensor(net.log_sigma, dtype=torch.float32)), device=self.dev, dtype=torch.float64)
         self.use_graph = use_graph
         self.g_fb = self.g_opt = self.g_enc = None
         self._cut = self._cut_grad = None
@@ -260,6 +269,8 @@ class TrainEngine:
             # per-batch statistics of main.py:83-85: the tensors stay device-resident (static addresses under
             # graph replay); stats() reduces them on demand instead of inside every step
             self.kld, self.rec, self.correct = kld, rec, correct
+            if self.sigma_mode != "fixed":
+                self.log_sigma = self.net.last_log_sigma
             self.recon = recon.detach()         # [B,N,3] view of the decoder buffer (no autograd graph attached)
             self._fwd_out = None
         _lib.defer_side_chains(True)          # weight-gradient chains of the conv layers run beside the following layers
@@ -298,7 +309,8 @@ class TrainEngine:
         self._loss_bwd()
 
     def stats(self):
-        """(mean kld, mean rec_loss, correct) of the last step - main.py:83-85 reads these per batch"""
+        """(mean kld, mean rec_loss, correct) of the last step - main.py:83-85 reads these per batch (the decoder log sigma
+        of the step is `log_sigma`)"""
         return float(self.kld.mean()), float(self.rec.mean()), int(self.correct)
 
     def _dp_begin(self):

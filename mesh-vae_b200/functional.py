@@ -297,33 +297,41 @@ def reparameterize(mu, logvar, eps):
     return _ReparamFn.apply(mu, logvar, eps)
 
 
+def _loss_operands(recon_vm, x_gt, mu, logvar, y_hat, y, channels: int):
+    """checked, contiguous operands of the loss epilogue, its sizes (n, b, c, z, ncls, ld, x_gt is fp64) and its
+    outputs (loss, kld, rec, correct, dnll, workspace, workspace bytes)"""
+    _req_cuda(recon_vm, "vae_loss recon")
+    _req_cuda(x_gt, "vae_loss x_gt", None)
+    if x_gt.dtype not in (torch.float32, torch.float64):
+        raise _lib.MvbError(f"vae_loss: x_gt must be fp32 or fp64, got {x_gt.dtype}")
+    n, b, ld = recon_vm.shape                    # entries of ld floats, the first `channels` are the reconstruction
+    c = channels
+    if tuple(x_gt.shape) != (b, n, c) or c > ld:
+        raise _lib.MvbError(f"vae_loss: x_gt is {tuple(x_gt.shape)}, expected {(b, n, c)}")
+    z = mu.shape[1]
+    ncls = y_hat.shape[1]
+    recon_vm, x_gt = recon_vm.contiguous(), x_gt.contiguous()
+    mu, logvar, y_hat = mu.contiguous(), logvar.contiguous(), y_hat.contiguous()
+    y = y.to(torch.int64).contiguous()
+    dev = recon_vm.device
+    f64 = x_gt.dtype == torch.float64
+    loss = torch.empty((), device=dev, dtype=torch.float64)
+    kld = torch.empty(b, device=dev, dtype=torch.float32)
+    rec = torch.empty(b, device=dev, dtype=torch.float64)
+    correct = torch.empty((), device=dev, dtype=torch.int64)
+    dnll = torch.empty_like(recon_vm)
+    ws_bytes = lib.mvb_vae_loss_workspace_bytes(b, n)
+    ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+    return (recon_vm, x_gt, mu, logvar, y_hat, y), (n, b, c, z, ncls, ld, f64), (loss, kld, rec, correct, dnll, ws, ws_bytes)
+
+
 class _VaeLossFn(torch.autograd.Function):
     """mvb_vae_loss_fwd / _bwd  (models/cheb_VAE.py:321-346)."""
 
     @staticmethod
     def forward(ctx, recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma: float, channels: int):
-        _req_cuda(recon_vm, "vae_loss recon")
-        _req_cuda(x_gt, "vae_loss x_gt", None)
-        if x_gt.dtype not in (torch.float32, torch.float64):
-            raise _lib.MvbError(f"vae_loss: x_gt must be fp32 or fp64, got {x_gt.dtype}")
-        n, b, ld = recon_vm.shape                    # entries of ld floats, the first `channels` are the reconstruction
-        c = channels
-        if tuple(x_gt.shape) != (b, n, c) or c > ld:
-            raise _lib.MvbError(f"vae_loss: x_gt is {tuple(x_gt.shape)}, expected {(b, n, c)}")
-        z = mu.shape[1]
-        ncls = y_hat.shape[1]
-        recon_vm, x_gt = recon_vm.contiguous(), x_gt.contiguous()
-        mu, logvar, y_hat = mu.contiguous(), logvar.contiguous(), y_hat.contiguous()
-        y = y.to(torch.int64).contiguous()
-        dev = recon_vm.device
-        f64 = x_gt.dtype == torch.float64
-        loss = torch.empty((), device=dev, dtype=torch.float64)
-        kld = torch.empty(b, device=dev, dtype=torch.float32)
-        rec = torch.empty(b, device=dev, dtype=torch.float64)
-        correct = torch.empty((), device=dev, dtype=torch.int64)
-        dnll = torch.empty_like(recon_vm)
-        ws_bytes = lib.mvb_vae_loss_workspace_bytes(b, n)
-        ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+        (recon_vm, x_gt, mu, logvar, y_hat, y), (n, b, c, z, ncls, ld, f64), (loss, kld, rec, correct, dnll, ws, ws_bytes) = \
+            _loss_operands(recon_vm, x_gt, mu, logvar, y_hat, y, channels)
         check(lib.mvb_vae_loss_fwd(b, n, c, z, ncls, ptr(recon_vm), ld, ptr(x_gt), 1 if f64 else 0, ptr(mu), ptr(logvar),
                                    ptr(y_hat), ptr(y), float(log_sigma), ptr(loss), ptr(kld), ptr(rec), ptr(correct),
                                    ptr(dnll), ptr(ws), ws_bytes, stream_ptr()), "mvb_vae_loss_fwd")
@@ -350,11 +358,78 @@ class _VaeLossFn(torch.autograd.Function):
         return d_recon, None, d_mu, d_lv, d_yh, None, None, None
 
 
-def vae_loss(recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma: float = LOG_SIGMA_DEFAULT, channels: Optional[int] = None):
+SIGMA_STATE_DOUBLES = 8          # include/mvb.h: mvb_vae_loss_sigma_fwd's sigma_state
+
+
+class _VaeLossSigmaFn(torch.autograd.Function):
+    """mvb_vae_loss_sigma_fwd / _bwd: the loss with the sigma-VAE decoder log sigma, optimal (s_param None) or learned
+    (sc(s_param), s_param a 1-element fp32 CUDA tensor whose gradient the backward kernel writes)."""
+
+    @staticmethod
+    def forward(ctx, recon_vm, x_gt, mu, logvar, y_hat, y, s_param, channels: int):
+        (recon_vm, x_gt, mu, logvar, y_hat, y), (n, b, c, z, ncls, ld, f64), (loss, kld, rec, correct, dnll, ws, ws_bytes) = \
+            _loss_operands(recon_vm, x_gt, mu, logvar, y_hat, y, channels)
+        if s_param is not None:
+            _req_cuda(s_param, "vae_loss log_sigma parameter")
+            if s_param.numel() != 1:
+                raise _lib.MvbError(f"vae_loss: a learned log_sigma has one element, got {tuple(s_param.shape)}")
+        state = torch.empty(SIGMA_STATE_DOUBLES, device=recon_vm.device, dtype=torch.float64)
+        s = None if s_param is None else s_param.detach().contiguous()
+        check(lib.mvb_vae_loss_sigma_fwd(b, n, c, z, ncls, ptr(recon_vm), ld, ptr(x_gt), 1 if f64 else 0, ptr(mu), ptr(logvar),
+                                         ptr(y_hat), ptr(y), 1 if s is None else 2, ptr(s), ptr(state), ptr(loss), ptr(kld),
+                                         ptr(rec), ptr(correct), ptr(dnll), ptr(ws), ws_bytes, stream_ptr()),
+              "mvb_vae_loss_sigma_fwd")
+        ctx.save_for_backward(dnll, state, mu, logvar, y_hat, y)
+        ctx.dims = (b, n, ld, z, ncls)
+        ctx.s_sink = _sink(s_param)
+        ctx.s_like = s_param
+        ctx.set_materialize_grads(False)
+        if not f64:
+            loss, rec = loss.float(), rec.float()
+        ctx.mark_non_differentiable(kld, rec, correct, state)
+        return loss, kld, rec, correct, state
+
+    @staticmethod
+    def backward(ctx, gloss, _gk, _gr, _gc, _gs):
+        dnll, state, mu, logvar, y_hat, y = ctx.saved_tensors
+        b, n, c, z, ncls = ctx.dims
+        g = gloss.to(torch.float64).contiguous()
+        need = ctx.needs_input_grad
+        d_recon = torch.empty_like(dnll) if need[0] else None
+        d_mu = torch.empty_like(mu) if need[2] else None
+        d_lv = torch.empty_like(logvar) if need[3] else None
+        d_yh = torch.empty_like(y_hat) if need[4] else None
+        d_s = None
+        if need[6]:
+            d_s = ctx.s_sink if ctx.s_sink is not None else torch.empty_like(ctx.s_like, memory_format=torch.contiguous_format)
+        check(lib.mvb_vae_loss_sigma_bwd(b, n, c, z, ncls, ptr(dnll), ptr(state), ptr(mu), ptr(logvar), ptr(y_hat), ptr(y),
+                                         ptr(g), ptr(d_recon), ptr(d_mu), ptr(d_lv), ptr(d_yh), ptr(d_s), stream_ptr()),
+              "mvb_vae_loss_sigma_bwd")
+        return d_recon, None, d_mu, d_lv, d_yh, None, (None if ctx.s_sink is not None else d_s), None
+
+
+def vae_loss(recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma=LOG_SIGMA_DEFAULT, channels: Optional[int] = None,
+             return_log_sigma: bool = False):
     """-> (loss, kld[B], rec_loss[B], correct); only `loss` carries gradient (as main.py:80 uses it).
-    recon_vm [N,B,ld]; `channels` (default ld) < ld: the decoder's padded output buffer is read in place."""
-    return _VaeLossFn.apply(recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma,
-                            int(recon_vm.shape[2] if channels is None else channels))
+    recon_vm [N,B,ld]; `channels` (default ld) < ld: the decoder's padded output buffer is read in place.
+
+    log_sigma, the decoder's Gaussian log sigma:
+      * a float: that constant (the reference's softclip(1, -6) by default);
+      * "optimal": the sigma-VAE optimal sigma, sc(0.5 log(SSE / (B N C))) with sc(t) = -6 + softplus(t + 6) and SSE the
+        batch's squared error, computed on the device; the gradient flows through it;
+      * a 1-element fp32 CUDA tensor s (a parameter): the learned sigma-VAE sigma sc(s); s receives its gradient.
+    return_log_sigma=True appends the log sigma used, an fp64 0-dim device tensor."""
+    c = int(recon_vm.shape[2] if channels is None else channels)
+    if isinstance(log_sigma, str) and log_sigma != "optimal":
+        raise _lib.MvbError(f"vae_loss: log_sigma is a float, 'optimal' or a parameter tensor, got {log_sigma!r}")
+    if isinstance(log_sigma, (str, torch.Tensor)):
+        out = _VaeLossSigmaFn.apply(recon_vm, x_gt, mu, logvar, y_hat, y, None if isinstance(log_sigma, str) else log_sigma, c)
+        return (*out[:4], out[4][0]) if return_log_sigma else out[:4]
+    out = _VaeLossFn.apply(recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma, c)
+    if not return_log_sigma:
+        return out
+    ls = float(torch.tensor(float(log_sigma), dtype=torch.float32))        # the kernel's log sigma is an fp32 argument
+    return (*out, torch.full((), ls, device=recon_vm.device, dtype=torch.float64))
 
 
 class _KldFn(torch.autograd.Function):
@@ -408,7 +483,50 @@ class _GaussianNllFn(torch.autograd.Function):
         return d_mu, None, None
 
 
-def gaussian_nll(mu, x, log_sigma: float):
+class _GaussianNllSigmaFn(torch.autograd.Function):
+    """mvb_gaussian_nll_sigma_fwd / _bwd: log_sigma a 0-dim fp32 / fp64 CUDA tensor, differentiable"""
+
+    @staticmethod
+    def forward(ctx, mu, x, log_sigma):
+        _req_cuda(mu, "gaussian_nll mu")
+        _req_cuda(x, "gaussian_nll x", None)
+        _req_cuda(log_sigma, "gaussian_nll log_sigma", None)
+        if x.dtype not in (torch.float32, torch.float64) or x.shape != mu.shape:
+            raise _lib.MvbError("gaussian_nll: x must be fp32/fp64 with the shape of mu")
+        if log_sigma.dtype not in (torch.float32, torch.float64):
+            raise _lib.MvbError(f"gaussian_nll: log_sigma must be fp32 or fp64, got {log_sigma.dtype}")
+        mu_c, x_c, ls = mu.contiguous(), x.contiguous(), log_sigma.contiguous()
+        out = torch.empty_like(x_c)
+        f64, ls64 = x.dtype == torch.float64, ls.dtype == torch.float64
+        check(lib.mvb_gaussian_nll_sigma_fwd(mu_c.numel(), ptr(mu_c), ptr(x_c), int(f64), ptr(ls), int(ls64), ptr(out),
+                                             stream_ptr()), "mvb_gaussian_nll_sigma_fwd")
+        ctx.save_for_backward(mu_c, x_c, ls)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        mu_c, x_c, ls = ctx.saved_tensors
+        n = mu_c.numel()
+        g = g.to(x_c.dtype).contiguous()
+        d_mu = torch.empty_like(mu_c)
+        d_ls = torch.empty((), device=mu_c.device, dtype=torch.float64)
+        ws_bytes = lib.mvb_gaussian_nll_sigma_workspace_bytes(n)
+        ws = torch.empty(max(ws_bytes, 8), device=mu_c.device, dtype=torch.uint8)
+        if n == 0:
+            d_ls.zero_()
+        else:
+            check(lib.mvb_gaussian_nll_sigma_bwd(n, ptr(mu_c), ptr(x_c), int(x_c.dtype == torch.float64), ptr(ls),
+                                                 int(ls.dtype == torch.float64), ptr(g), ptr(d_mu), ptr(d_ls), ptr(ws), ws_bytes,
+                                                 stream_ptr()), "mvb_gaussian_nll_sigma_bwd")
+        return d_mu, None, d_ls.to(ls.dtype)
+
+
+def gaussian_nll(mu, x, log_sigma):
+    """log_sigma a float (a host constant) or a 1-element CUDA tensor (read on the device, differentiable)"""
+    if isinstance(log_sigma, torch.Tensor):
+        if log_sigma.numel() != 1:
+            raise _lib.MvbError(f"gaussian_nll: log_sigma has {log_sigma.numel()} elements, expected 1")
+        return _GaussianNllSigmaFn.apply(mu, x, log_sigma.reshape(()))
     return _GaussianNllFn.apply(mu, x, log_sigma)
 
 

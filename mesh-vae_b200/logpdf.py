@@ -18,11 +18,16 @@ def softclip(tensor, min):  # noqa: A002  (reference signature)
 
 
 def gaussian_nll(mu, log_sigma, x):
-    """0.5 ((x - mu)/exp(log_sigma))^2 + log_sigma + 0.5 log(2 pi); log_sigma is the constant
-    1-element tensor of models/cheb_VAE.py:328-329 (no gradient flows to it)."""
+    """0.5 ((x - mu)/exp(log_sigma))^2 + log_sigma + 0.5 log(2 pi); log_sigma is a 1-element tensor: the constant of
+    models/cheb_VAE.py:328-329, or a sigma-VAE log sigma (a parameter, or the optimal
+    softclip(((x - mu)**2).mean().sqrt().log(), -6)) through which the gradient flows.  A CUDA log_sigma is read on the
+    device (no host synchronisation); a constant host one is passed by value as before."""
     if isinstance(log_sigma, torch.Tensor):
-        if log_sigma.numel() != 1 or log_sigma.requires_grad:
-            raise NotImplementedError("gaussian_nll: only a constant scalar log_sigma is supported")
-        log_sigma = float(log_sigma)
+        if log_sigma.numel() != 1:
+            raise ValueError(f"gaussian_nll: log_sigma must have one element, got {tuple(log_sigma.shape)}")
+        if log_sigma.is_cuda or log_sigma.requires_grad:
+            log_sigma = log_sigma.to(mu.device)
+        else:
+            log_sigma = float(log_sigma)
     mu_b, x_b = torch.broadcast_tensors(mu, x)
     return Fn.gaussian_nll(mu_b, x_b, log_sigma)
