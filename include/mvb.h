@@ -260,6 +260,35 @@ int mvb_vae_loss_sigma_bwd(int B, int N, int C, int Z, int ncls, const float *dn
                            const double *gloss, float *d_recon, float *d_mu, float *d_logvar, float *d_yhat,
                            float *d_s, void *stream);
 
+/* ---- importance-weighted estimate of the held-out log-likelihood log p(x | y) (no counterpart in the reference) ----
+ * With S samples z_(b,s) ~ q(z | x_b, y_b) per mesh and n = N*C:
+ *   log w_(b,s) = log p(x_b | z_(b,s), y_b) - (log q(z_(b,s) | x_b, y_b) - log p(z_(b,s)))
+ *   log p(x | z) = -SSE / (2 sigma^2) - n (log sigma + 0.5 log(2 pi)),  log p(x_b | y_b) ~ log mean_s exp(log w_(b,s)).
+ * Densities are those of the coordinates the model sees (z-scored).  All sums fp64 in a fixed order; no atomics, no
+ * host synchronisation: capturable and bit-reproducible run to run.
+ *
+ * mvb_iw_sample: mu, logvar [B,Z] fp32 (the heads at eval, z = mu there), eps [B,S,Z] fp32 N(0, I) from the caller,
+ *   y [B,C] int64 one-hot.  Writes the decoder input zcat [B*S, C+Z] fp32, mesh-major (row b*S + s = cat(y_b, z)) with
+ *   z = eps * exp(0.5 logvar) + mu in fp32 as mvb_vae_reparam_fwd computes it, and
+ *   log_r [B*S] fp64 = sum_j (-eps_j^2/2 - logvar_j/2 + z_j^2/2) = log q(z | x, y) - log p(z). */
+int mvb_iw_sample(int B, int S, int Z, int C, const float *mu, const float *logvar, const float *eps, const int64_t *y,
+                  float *zcat, double *log_r, void *stream);
+/* mvb_iw_log_weights: one chunk of S samples per mesh.  recon [N, B*S, recon_ld] fp32 VERTEX-MAJOR (the decoder output
+ *   of mvb_iw_sample's zcat: column b*S + s), x_gt [B,N,C] mesh-major fp64 (x_is_f64 != 0) or fp32, log_sigma a DEVICE
+ *   fp64 scalar, log_r [B*S] fp64 of the same chunk.  SSE per reconstruction as mvb_vae_loss_sigma_fwd sums it (the
+ *   same partial kernel: fp64 squares of differences taken in x_gt's precision), then
+ *   log_w[b*S_total + s0 + s] = log p(x_b | z) - log_r[b*S + s]   for s < S  (log_w [B, S_total] fp64, s0 + S <= S_total).
+ *   Entry width limits as mvb_vae_loss_fwd; B*S at most 65535*32 = 2097120 reconstructions per call (MVB_EINVAL beyond).
+ *   workspace: mvb_iw_log_weights_workspace_bytes(B, S, N) bytes. */
+size_t mvb_iw_log_weights_workspace_bytes(int B, int S, int N);
+int mvb_iw_log_weights(int B, int S, int N, int C, const float *recon, int recon_ld, const void *x_gt, int x_is_f64,
+                       const double *log_sigma, const double *log_r, int S_total, int s0, double *log_w, void *workspace,
+                       size_t workspace_bytes, void *stream);
+/* mvb_iw_reduce: log_w [B,S] fp64 -> per mesh (fp64 [B]) with m = max_s log w and e_s = exp(log w_s - m):
+ *   log_px = m + log sum_s e_s - log S ;  elbo = (1/S) sum_s log w_s ;  ess = (sum_s e_s)^2 / sum_s e_s^2.
+ *   log_w_out [B,S] (may be NULL): a copy of log_w for the caller. */
+int mvb_iw_reduce(int B, int S, const double *log_w, double *log_px, double *elbo, double *ess, double *log_w_out, void *stream);
+
 /* ---- logpdf.py drop-ins used when the reference's own loss_function runs unchanged ----------
  * KLD (logpdf.py:7-8): out[b] = -0.5 sum_j (1 + logvar - mu^2 - exp(logvar)); bwd as above.
  * gaussian_nll (logpdf.py:22-23), elementwise on n values with scalar log_sigma:

@@ -66,6 +66,10 @@ SIGNATURES = {
     "mvb_vae_loss_bwd": (c_int, [c_int, c_int, c_int, c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mvb_vae_loss_sigma_fwd": (c_int, [c_int] * 5 + [_vp, c_int, _vp, c_int] + [_vp] * 4 + [c_int] + [_vp] * 8 + [c_size_t, _vp]),
     "mvb_vae_loss_sigma_bwd": (c_int, [c_int] * 5 + [_vp] * 13),
+    "mvb_iw_sample": (c_int, [c_int] * 4 + [_vp] * 7),
+    "mvb_iw_log_weights_workspace_bytes": (c_size_t, [c_int] * 3),
+    "mvb_iw_log_weights": (c_int, [c_int] * 4 + [_vp, c_int, _vp, c_int, _vp, _vp, c_int, c_int, _vp, _vp, c_size_t, _vp]),
+    "mvb_iw_reduce": (c_int, [c_int, c_int] + [_vp] * 6),
     "mvb_kld_fwd": (c_int, [c_int, c_int, _vp, _vp, _vp, _vp]),
     "mvb_kld_bwd": (c_int, [c_int, c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mvb_gaussian_nll_fwd": (c_int, [c_int64, _vp, _vp, c_int, c_float, _vp, _vp]),

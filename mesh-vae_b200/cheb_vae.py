@@ -22,6 +22,7 @@ import torch.nn.functional as F
 
 from . import functional as Fn
 from . import operators
+from ._lib import MvbError
 from .conv import ChebConv_batch
 from .pool import SurfacePool
 
@@ -68,6 +69,7 @@ class cheb_VAE(nn.Module):
         self.sigma_mode = "fixed"
         self.log_sigma = Fn.LOG_SIGMA_DEFAULT
         self.last_log_sigma = None
+        self.train_log_sigma = None
         # fused dense bottleneck (row f2): one launch per Linear(+ReLU+dropout), one for the three heads
         self.fused_dense = True
         # coarse levels: pool + conv + ReLU (+ pool) as one mesh-resident kernel (Fn.cheb_layer)
@@ -97,6 +99,7 @@ class cheb_VAE(nn.Module):
             self.log_sigma = Fn.LOG_SIGMA_DEFAULT if mode == "fixed" else "optimal"
         self.sigma_mode = mode
         self.last_log_sigma = None
+        self.train_log_sigma = None
 
     def reset_parameters(self):
         nn.init.normal_(self.enc_lin.weight, 0, 0.1)
@@ -211,7 +214,8 @@ class cheb_VAE(nn.Module):
 
     def loss_function(self, x, recon_x, z, mu_z, logvar_z, y, y_hat):
         """as the reference's; with a sigma-VAE decoder sigma the log sigma used is left in `last_log_sigma` (fp64 0-dim
-        device tensor)"""
+        device tensor), and in training mode also in `train_log_sigma`: the sigma of the last training step, which an
+        evaluation forward does not replace (log_likelihood's optimal sigma)"""
         padded, self._recon_padded = self._recon_padded, None           # one-shot hand-over from decoder()
         if padded is not None and recon_x.data_ptr() == padded.data_ptr() and recon_x.shape[1] == padded.shape[0]:
             recon_vm, channels = padded, recon_x.shape[2]
@@ -222,6 +226,8 @@ class cheb_VAE(nn.Module):
         loss, kld, rec, correct = out[:4]
         if self.sigma_mode != "fixed":
             self.last_log_sigma = out[4]
+            if self.training:
+                self.train_log_sigma = out[4]
         return loss, correct, kld, rec
 
     def forward_recon(self, data, y, m_type="test", eps: Optional[torch.Tensor] = None):
@@ -249,6 +255,84 @@ class cheb_VAE(nn.Module):
             z = torch.cat([y, z_], -1)
         recon = self.decoder(z).reshape(batch_size, -1, self.filters[0])
         return recon, z, x_mean, x_var, z_, y_hat
+
+    def _likelihood_log_sigma(self, log_sigma, dev) -> torch.Tensor:
+        """the decoder log sigma of log_likelihood as a 0-dim fp64 device tensor (never read back to the host)"""
+        if isinstance(log_sigma, torch.Tensor):
+            Fn._req_cuda(log_sigma, "log_likelihood log_sigma", None)
+            if log_sigma.numel() != 1:
+                raise MvbError(f"log_likelihood: log_sigma has {log_sigma.numel()} elements, expected 1")
+            return log_sigma.detach().reshape(()).to(torch.float64)
+        if log_sigma is not None:
+            if isinstance(log_sigma, str):
+                raise MvbError(f"log_likelihood: log_sigma is a float or a 1-element CUDA tensor, got {log_sigma!r}")
+            return torch.full((), float(log_sigma), device=dev, dtype=torch.float64)
+        if self.sigma_mode == "learned":
+            t = self.log_sigma.detach().double() + 6.0
+            return -6.0 + torch.logaddexp(t, torch.zeros_like(t))
+        if self.sigma_mode == "optimal":
+            if self.train_log_sigma is None:
+                raise MvbError("log_likelihood: the optimal decoder sigma is taken from the last training step, and the model "
+                               "has not trained in this mode; pass log_sigma=")
+            return self.train_log_sigma.detach().reshape(()).to(dev, torch.float64)
+        return torch.full((), float(self.log_sigma), device=dev, dtype=torch.float64)
+
+    def log_likelihood(self, x, x_gt, y_onehot, samples: int, sample_chunk: Optional[int] = None,
+                       generator: Optional[torch.Generator] = None, log_sigma=None, return_log_w: bool = False):
+        """Importance-weighted estimate of log p(x | y) per mesh with `samples` (S) draws from q(z | x, y):
+        log w_s = log p(x | z_s, y) + log p(z_s) - log q(z_s | x, y), and
+          log_px = log (1/S) sum_s w_s   (a lower bound of log p(x | y) in expectation, tight as S grows),
+          elbo   = (1/S) sum_s log w_s   (the Monte-Carlo ELBO),
+          ess    = (sum_s w_s)^2 / sum_s w_s^2   (the effective sample size of the weights, between 1 and S),
+        each an fp64 [B] device tensor; return_log_w=True appends log w [B, S].  x [B,N,F] the (z-scored) input, x_gt
+        [B,N,F] fp32 / fp64 its ground truth, y_onehot [B, num_classes]; densities are those of these coordinates.
+
+        The model runs in eval mode (no dropout) under no_grad, and its mode is restored afterwards.  The encoder and heads
+        run once; eps = torch.randn((B, S, num_style), generator=generator, device=x.device) is drawn once, so the result
+        does not depend on `sample_chunk`; the decoder runs on sample_chunk * B meshes at a time (default: all S).  No host
+        synchronisation: the call can be captured in a CUDA graph (with the default generator, or one registered with it).
+
+        The decoder's log sigma: `log_sigma` (a float or a 1-element CUDA tensor) when given, else that of the model's
+        decoder sigma mode - the constant (fixed), sc(s) of the parameter (learned), or `train_log_sigma`, the sigma of the
+        last training step (optimal: MvbError when there is none; the sigma is never derived from the data scored)."""
+        if isinstance(x, torch.Tensor):
+            b = x.shape[0]
+        else:
+            x, b = x.x, x.num_graphs
+        Fn._req_cuda(x, "log_likelihood x")
+        Fn._req_cuda(x_gt, "log_likelihood x_gt", None)
+        Fn._req_cuda(y_onehot, "log_likelihood y", None)
+        s_total = int(samples)
+        chunk = s_total if sample_chunk is None else int(sample_chunk)
+        if s_total < 1 or chunk < 1:
+            raise MvbError(f"log_likelihood: samples={samples} and sample_chunk={sample_chunk} must be >= 1")
+        chunk = min(chunk, s_total)
+        x = x.reshape(b, -1, self.filters[0])
+        if x.shape[1] != self.A_num_nodes[0] or x_gt.dim() != 3 or tuple(x_gt.shape) != tuple(x.shape):
+            raise MvbError(f"log_likelihood: x {tuple(x.shape)} and x_gt {tuple(x_gt.shape)} must both be "
+                           f"({b}, {self.A_num_nodes[0]}, {self.filters[0]})")
+        dev = x.device
+        ls = self._likelihood_log_sigma(log_sigma, dev)
+        was_training = self.training
+        self.eval()
+        try:
+            with torch.no_grad():
+                h = self.encoder(x)
+                _, mu, logvar, _, _ = Fn.vae_heads(h, y_onehot, None, self.classifier_layer, self.z_mean, self.z_log_var)
+                eps = torch.randn((b, s_total, self.z), generator=generator, device=dev, dtype=torch.float32)
+                log_w = torch.empty((b, s_total), device=dev, dtype=torch.float64)
+                for s0 in range(0, s_total, chunk):
+                    zcat, log_r = Fn.iw_sample(mu, logvar, eps[:, s0:s0 + chunk], y_onehot)
+                    recon = self.decoder(zcat)
+                    padded, self._recon_padded = self._recon_padded, None
+                    if padded is not None and recon.data_ptr() == padded.data_ptr():
+                        recon_vm, channels = padded, recon.shape[2]
+                    else:
+                        recon_vm, channels = Fn.to_vertex_major(recon), None
+                    Fn.iw_log_weights(recon_vm, x_gt, ls, log_r, log_w, s0, channels)
+                return Fn.iw_reduce(log_w, return_log_w)
+        finally:
+            self.train(was_training)
 
     def forward(self, data, x_gt, y, supervise=True, m_type="test", eps: Optional[torch.Tensor] = None):
         self.supervise = supervise

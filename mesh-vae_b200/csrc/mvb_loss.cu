@@ -10,6 +10,7 @@
 // The sigma-VAE variants (optimal and learned decoder sigma) share the partial kernel: it then sums the squared error per
 // mesh and keeps recon - x unscaled, and their finalize kernel derives log sigma on the device from the batch's error or
 // from a parameter (no host round trip: a captured step follows new inputs and Adam's updates of the parameter).
+// The importance-weighted log-likelihood estimate (mvb_iw_*) shares it too: S reconstructions per ground-truth mesh.
 // Roofline: HBM; algorithmic bytes = N*B*C*(4 + sizeof(x) + 4).
 #include "mvb_internal.cuh"
 
@@ -23,10 +24,13 @@ template <>
 struct AccT<double> { typedef double type; };
 
 // SSE = false: partial = sum of the NLL terms, dnll = (recon - x)/sigma^2 (the reference's constant sigma);
-// SSE = true: partial = sum of (recon - x)^2 (fp64 squares), dnll = recon - x (sigma is not known yet)
+// SSE = true: partial = sum of (recon - x)^2 (fp64 squares), dnll = recon - x (sigma is not known yet).
+// B counts the reconstructions (columns of recon); S of them share one ground truth: column j is compared with mesh j / S
+// of xgt (S = 1: the loss epilogue; S > 1: the importance samples of mvb_iw_log_weights), and the block loads each
+// ground-truth row it needs once.  dnll = NULL: no dnll is written.
 template <typename XT, bool SSE>
 __global__ void __launch_bounds__(256)
-vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const float *__restrict__ recon,
+vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, int S, const float *__restrict__ recon,
                        const XT *__restrict__ xgt, float log_sigma, float sigma,
                        double *__restrict__ partial, float *__restrict__ dnll) {
     pdl_trigger();
@@ -38,6 +42,7 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
     const int tid = threadIdx.x, nthreads = blockDim.x;
     const int v0 = blockIdx.x * VCH, b0 = blockIdx.y * BCH;
     const int nv = min(VCH, N - v0), nb = min(BCH, B - b0);
+    const int m0 = b0 / S, nm = (b0 + nb - 1) / S - m0 + 1;     // the ground-truth meshes of the block's columns
     const int rw = nb * ld; // contiguous run per vertex in recon (entries of ld floats, the first C are data)
     const int xw = nv * C;  // contiguous run per mesh in x_gt
     // both tiles through cp.async: every element of the block's two tiles is in flight at once (one exposed
@@ -53,8 +58,8 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
                 for (int e = lane_; e < rw; e += 32) cp_async<1>(dst + e, src + e);
             }
         }
-        for (int b = warp_; b < nb; b += nwarps_) {
-            const XT *src = xgt + ((int64_t)(b0 + b) * N + v0) * C;
+        for (int b = warp_; b < nm; b += nwarps_) {
+            const XT *src = xgt + ((int64_t)(m0 + b) * N + v0) * C;
             XT *dst = Xs + b * (VCH * C);
             constexpr int PER16 = 16 / (int)sizeof(XT);
             if ((xw % PER16) == 0 && ((VCH * C) % PER16) == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0) {
@@ -81,11 +86,12 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
     const AT inv_sg = (AT)1 / sg, inv_sg2 = (AT)1 / (sg * sg);     // two multiplies per element instead of two (fp64) divisions
     const AT cst = (AT)log_sigma + (AT)MVB_HALF_LOG_2PI;
     for (int b = warp; b < nb; b += nwarps) {
+        const XT *xs = Xs + ((b0 + b) / S - m0) * (VCH * C);
         double s = 0.0;
         for (int e = lane; e < xw; e += 32) {
             const int v = e / C, c = e - v * C;
             float *rp = Rs + v * (BCH * ld) + b * ld + c;
-            const AT d = (AT)(*rp) - (AT)Xs[b * (VCH * C) + e];   // recon - x
+            const AT d = (AT)(*rp) - (AT)xs[e];   // recon - x
             if constexpr (SSE) {
                 s = fma((double)d, (double)d, s);
                 *rp = (float)d;
@@ -100,6 +106,7 @@ vae_rec_partial_kernel(int B, int N, int C, int ld, int VCH, int BCH, const floa
         for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
         if (lane == 0) partial[(int64_t)blockIdx.x * B + b0 + b] = s;
     }
+    if (!dnll) return;
     __syncthreads();
     // padded mesh coordinates: one 16-byte entry per (vertex, mesh), pad lane zeroed (an offset view of dnll: scalar path)
     if (ld == 4 && C == 3 && (reinterpret_cast<uintptr_t>(dnll) & 15) == 0) {
@@ -545,6 +552,107 @@ __global__ void __launch_bounds__(256) ordered_sum_kernel(int n, const double *_
     if (threadIdx.x == 0) *out = sh[0];
 }
 
+// ---- importance-weighted log-likelihood estimate: log p(x | y) from S posterior samples per mesh ---------------------
+// a warp per (mesh b, sample s) row r = b S + s: the decoder input zcat[r] = cat(y_b, z) with z the expression of
+// reparam_fwd_kernel, and log r = log q(z | x, y) - log p(z) = sum_j (-eps_j^2/2 - logvar_j/2 + z_j^2/2) in fp64 (the
+// 0.5 log(2 pi) terms cancel), lane-strided with a fixed xor tree
+__global__ void __launch_bounds__(256)
+iw_sample_kernel(int B, int S, int Z, int C, const float *__restrict__ mu, const float *__restrict__ logvar,
+                 const float *__restrict__ eps, const int64_t *__restrict__ y, float *__restrict__ zcat, double *__restrict__ log_r) {
+    pdl_trigger();
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (r >= (int64_t)B * S) return;
+    const int64_t b = r / S;
+    const float *m = mu + b * Z, *lv = logvar + b * Z, *e = eps + r * Z;
+    float *out = zcat + r * (C + Z);
+    for (int c = lane; c < C; c += 32) out[c] = (float)y[b * C + c];
+    double acc = 0.0;
+    for (int j = lane; j < Z; j += 32) {
+        const float ej = e[j], lj = lv[j];
+        const float z = fmaf(ej, expf(0.5f * lj), m[j]);
+        out[C + j] = z;
+        const double ed = ej, zd = z;
+        acc += 0.5 * (zd * zd - ed * ed) - 0.5 * (double)lj;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    if (lane == 0) log_r[r] = acc;
+}
+
+// a warp per reconstruction j = b S + s: SSE_j = the ordered sum of the vertex-chunk partials (the order of
+// vae_loss_finalize_kernel's phase 1), log p(x_b | z_j) = -SSE_j / (2 sigma^2) - n (log sigma + 0.5 log(2 pi)) with log sigma
+// read from device memory, log w = log p - log r, written to column s0 + s of row b of log_w [B, S_total]
+__global__ void __launch_bounds__(256)
+iw_log_weights_finalize_kernel(int BS, int S, int S_total, int s0, int nchunks, double n_elem, const double *__restrict__ partial,
+                               const double *__restrict__ log_sigma, const double *__restrict__ log_r, double *__restrict__ log_w) {
+    pdl_trigger();
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (j >= BS) return;
+    double r0 = 0.0, r1 = 0.0, r2 = 0.0, r3 = 0.0;
+    int ch = lane;
+    for (; ch + 96 < nchunks; ch += 128) {
+        r0 += partial[(int64_t)ch * BS + j];
+        r1 += partial[(int64_t)(ch + 32) * BS + j];
+        r2 += partial[(int64_t)(ch + 64) * BS + j];
+        r3 += partial[(int64_t)(ch + 96) * BS + j];
+    }
+    for (; ch < nchunks; ch += 32) r0 += partial[(int64_t)ch * BS + j];
+    double sse = (r0 + r1) + (r2 + r3);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) sse += __shfl_xor_sync(0xffffffffu, sse, off);
+    if (lane == 0) {
+        const double ls = *log_sigma;
+        const double log_px_z = -(0.5 * sse * exp(-2.0 * ls)) - n_elem * (ls + MVB_HALF_LOG_2PI);
+        const int b = j / S, s = j - b * S;
+        log_w[(int64_t)b * S_total + s0 + s] = log_px_z - log_r[j];
+    }
+}
+
+// a warp per mesh over its S log-weights (lane-strided, fixed xor trees; the max is exact in any order):
+// log_px = max + log sum_s exp(log w - max) - log S, elbo = mean_s log w, ess = (sum e)^2 / sum e^2 with e = exp(log w - max)
+__global__ void __launch_bounds__(256)
+iw_reduce_kernel(int B, int S, const double *__restrict__ log_w, double *__restrict__ log_px, double *__restrict__ elbo,
+                 double *__restrict__ ess, double *__restrict__ log_w_out) {
+    pdl_trigger();
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (b >= B) return;
+    const double *w = log_w + (int64_t)b * S;
+    double mx = -INFINITY, sum = 0.0;
+    for (int s = lane; s < S; s += 32) {
+        const double v = w[s];
+        mx = fmax(mx, v);
+        sum += v;
+        if (log_w_out) log_w_out[(int64_t)b * S + s] = v;
+    }
+    double e1 = 0.0, e2 = 0.0;
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, off));
+        sum += __shfl_xor_sync(0xffffffffu, sum, off);
+    }
+    for (int s = lane; s < S; s += 32) {
+        const double t = exp(w[s] - mx);
+        e1 += t;
+        e2 += t * t;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        e1 += __shfl_xor_sync(0xffffffffu, e1, off);
+        e2 += __shfl_xor_sync(0xffffffffu, e2, off);
+    }
+    if (lane == 0) {
+        log_px[b] = mx + log(e1) - log((double)S);
+        elbo[b] = sum / (double)S;
+        ess[b] = e1 * e1 / e2;
+    }
+}
+
 static inline unsigned ew_grid(int64_t n, int threads) {
     int64_t b = (n + threads - 1) / threads;
     const int64_t cap = (int64_t)num_sms() * 16;
@@ -595,9 +703,9 @@ extern "C" int mvb_vae_loss_fwd(int B, int N, int C, int Z, int ncls, const floa
     const float sigma = expf(log_sigma);
     double *partial = reinterpret_cast<double *>(workspace);
     if (x_is_f64)
-        launch_pdl(vae_rec_partial_kernel<double, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const double *)x_gt, log_sigma, sigma, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<double, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, 1, recon, (const double *)x_gt, log_sigma, sigma, partial, dnll);
     else
-        launch_pdl(vae_rec_partial_kernel<float, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const float *)x_gt, log_sigma, sigma, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<float, false>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, 1, recon, (const float *)x_gt, log_sigma, sigma, partial, dnll);
     int rc = check_launch("mvb_vae_loss_fwd partial");
     if (rc) return rc;
     launch_pdl(vae_loss_finalize_kernel<false>, dim3(1), dim3(1024), 0, st, B, Z, ncls, nch, partial, mu, logvar, y_hat, y, loss, kld, rec,
@@ -654,9 +762,9 @@ extern "C" int mvb_vae_loss_sigma_fwd(int B, int N, int C, int Z, int ncls, cons
     dim3 grid(nch, (B + BCH - 1) / BCH);
     double *partial = reinterpret_cast<double *>(workspace);
     if (x_is_f64)
-        launch_pdl(vae_rec_partial_kernel<double, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const double *)x_gt, 0.f, 1.f, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<double, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, 1, recon, (const double *)x_gt, 0.f, 1.f, partial, dnll);
     else
-        launch_pdl(vae_rec_partial_kernel<float, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, recon, (const float *)x_gt, 0.f, 1.f, partial, dnll);
+        launch_pdl(vae_rec_partial_kernel<float, true>, dim3(grid), dim3(256), smem, st, B, N, C, recon_ld, VCH, BCH, 1, recon, (const float *)x_gt, 0.f, 1.f, partial, dnll);
     int rc = check_launch("mvb_vae_loss_sigma_fwd partial");
     if (rc) return rc;
     launch_pdl(vae_loss_finalize_kernel<true>, dim3(1), dim3(1024), 0, st, B, Z, ncls, nch, partial, mu, logvar, y_hat, y, loss, kld, rec,
@@ -811,6 +919,61 @@ extern "C" int mvb_epoch_meter_add(int B, const void *loss, int loss_is_f64, con
     else
         mvb::epoch_meter_kernel<float><<<1, 256, 0, (cudaStream_t)stream>>>(B, l64, l32, kld, (const float *)rec, correct, mean_err, acc);
     return mvb::check_launch("mvb_epoch_meter_add");
+}
+
+extern "C" int mvb_iw_sample(int B, int S, int Z, int C, const float *mu, const float *logvar, const float *eps, const int64_t *y,
+                             float *zcat, double *log_r, void *stream) {
+    MVB_REQUIRE(B > 0 && S > 0 && Z > 0 && C > 0, "iw_sample: bad sizes B=%d S=%d Z=%d C=%d", B, S, Z, C);
+    MVB_REQUIRE(mu && logvar && eps && y && zcat && log_r, "iw_sample: null pointer");
+    const int64_t rows = (int64_t)B * S;
+    MVB_REQUIRE(rows <= (int64_t)1 << 30, "iw_sample: B*S=%lld too large", (long long)rows);
+    mvb::launch_pdl(mvb::iw_sample_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, (cudaStream_t)stream, B, S, Z, C, mu, logvar,
+                    eps, y, zcat, log_r);
+    return mvb::check_launch("mvb_iw_sample");
+}
+
+extern "C" size_t mvb_iw_log_weights_workspace_bytes(int B, int S, int N) { return mvb_vae_loss_workspace_bytes(B * S, N); }
+
+extern "C" int mvb_iw_log_weights(int B, int S, int N, int C, const float *recon, int recon_ld, const void *x_gt, int x_is_f64,
+                                  const double *log_sigma, const double *log_r, int S_total, int s0, double *log_w, void *workspace,
+                                  size_t workspace_bytes, void *stream) {
+    MVB_REQUIRE(B > 0 && S > 0 && N > 0 && C > 0, "iw_log_weights: bad sizes B=%d S=%d N=%d C=%d", B, S, N, C);
+    MVB_REQUIRE(recon_ld >= C, "iw_log_weights: recon_ld=%d < C=%d", recon_ld, C);
+    MVB_REQUIRE(s0 >= 0 && S_total >= s0 + S, "iw_log_weights: columns [%d, %d) outside [0, %d)", s0, s0 + S, S_total);
+    MVB_REQUIRE(recon && x_gt && log_sigma && log_r && log_w && workspace, "iw_log_weights: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    int VCH, BCH;
+    size_t smem;
+    mvb::loss_tiles(C, recon_ld, x_is_f64 ? 8 : 4, VCH, BCH, smem);
+    MVB_REQUIRE(VCH >= 8, "iw_log_weights: C=%d too large", C);
+    // the partial kernel's grid.y walks the B*S reconstructions in tiles of BCH (at most 65535 tiles)
+    MVB_REQUIRE(((int64_t)B * S + BCH - 1) / BCH <= 65535, "iw_log_weights: B*S=%lld reconstructions per call, at most %d: decode fewer "
+                "samples at a time", (long long)B * S, 65535 * BCH);
+    const int BS = B * S;
+    const int nch = (N + VCH - 1) / VCH;
+    if ((size_t)nch * BS * sizeof(double) > workspace_bytes)
+        return mvb::set_err(MVB_EWORKSPACE, "iw_log_weights: workspace %zu < %zu", workspace_bytes, (size_t)nch * BS * sizeof(double));
+    dim3 grid(nch, (BS + BCH - 1) / BCH);
+    double *partial = reinterpret_cast<double *>(workspace);
+    if (x_is_f64)
+        mvb::launch_pdl(mvb::vae_rec_partial_kernel<double, true>, grid, dim3(256), smem, st, BS, N, C, recon_ld, VCH, BCH, S, recon,
+                        (const double *)x_gt, 0.f, 1.f, partial, (float *)nullptr);
+    else
+        mvb::launch_pdl(mvb::vae_rec_partial_kernel<float, true>, grid, dim3(256), smem, st, BS, N, C, recon_ld, VCH, BCH, S, recon,
+                        (const float *)x_gt, 0.f, 1.f, partial, (float *)nullptr);
+    int rc = mvb::check_launch("mvb_iw_log_weights partial");
+    if (rc) return rc;
+    mvb::launch_pdl(mvb::iw_log_weights_finalize_kernel, dim3((unsigned)((BS + 7) / 8)), dim3(256), 0, st, BS, S, S_total, s0, nch,
+                    (double)N * C, (const double *)partial, log_sigma, log_r, log_w);
+    return mvb::check_launch("mvb_iw_log_weights finalize");
+}
+
+extern "C" int mvb_iw_reduce(int B, int S, const double *log_w, double *log_px, double *elbo, double *ess, double *log_w_out,
+                             void *stream) {
+    MVB_REQUIRE(B > 0 && S > 0 && log_w && log_px && elbo && ess, "iw_reduce: bad arguments");
+    mvb::launch_pdl(mvb::iw_reduce_kernel, dim3((unsigned)((B + 7) / 8)), dim3(256), 0, (cudaStream_t)stream, B, S, log_w, log_px, elbo,
+                    ess, log_w_out);
+    return mvb::check_launch("mvb_iw_reduce");
 }
 
 extern "C" int mvb_pack_vertex_major(int B, int N, int C, int Cp, const float *x, float *out, void *stream) {

@@ -432,6 +432,79 @@ def vae_loss(recon_vm, x_gt, mu, logvar, y_hat, y, log_sigma=LOG_SIGMA_DEFAULT, 
     return (*out, torch.full((), ls, device=recon_vm.device, dtype=torch.float64))
 
 
+# ---------------------------------------------------------------------------------------------
+# importance-weighted log-likelihood estimate (include/mvb.h: mvb_iw_*); forward only, no autograd
+# ---------------------------------------------------------------------------------------------
+def iw_sample(mu, logvar, eps, y_onehot):
+    """mu, logvar [B,Z] fp32, eps [B,S,Z] fp32, y_onehot [B,C] -> (zcat [B*S, C+Z] fp32, row b*S + s = cat(y_b, z) with
+    z = eps * exp(logvar/2) + mu; log_r [B*S] fp64 = log q(z | x, y) - log p(z))"""
+    for t, name in ((mu, "mu"), (logvar, "logvar"), (eps, "eps")):
+        _req_cuda(t, f"iw_sample {name}")
+    _req_cuda(y_onehot, "iw_sample y", None)
+    if mu.dim() != 2 or tuple(logvar.shape) != tuple(mu.shape):
+        raise _lib.MvbError(f"iw_sample: mu {tuple(mu.shape)} and logvar {tuple(logvar.shape)} must be the same [B, Z]")
+    b, z = mu.shape
+    if eps.dim() != 3 or eps.shape[0] != b or eps.shape[2] != z or eps.shape[1] < 1:
+        raise _lib.MvbError(f"iw_sample: eps is {tuple(eps.shape)}, expected ({b}, S, {z})")
+    if y_onehot.dim() != 2 or y_onehot.shape[0] != b:
+        raise _lib.MvbError(f"iw_sample: y is {tuple(y_onehot.shape)}, expected ({b}, C)")
+    s, c = eps.shape[1], y_onehot.shape[1]
+    mu, logvar, eps = mu.contiguous(), logvar.contiguous(), eps.contiguous()
+    y = y_onehot.to(torch.int64).contiguous()
+    zcat = torch.empty((b * s, c + z), device=mu.device, dtype=torch.float32)
+    log_r = torch.empty(b * s, device=mu.device, dtype=torch.float64)
+    check(lib.mvb_iw_sample(b, s, z, c, ptr(mu), ptr(logvar), ptr(eps), ptr(y), ptr(zcat), ptr(log_r), stream_ptr()),
+          "mvb_iw_sample")
+    return zcat, log_r
+
+
+def iw_log_weights(recon_vm, x_gt, log_sigma, log_r, log_w, s0: int = 0, channels: Optional[int] = None):
+    """Writes columns [s0, s0 + S) of log_w [B, S_total] (fp64, in place): log w = log p(x_b | z) - log_r with
+    log p(x | z) = -SSE / (2 sigma^2) - N C (log sigma + log(2 pi)/2).  recon_vm [N, B*S, ld] vertex-major (column b*S + s;
+    the first `channels` (default ld) floats of an entry are the reconstruction), x_gt [B,N,C] fp32 / fp64, log_sigma a
+    0-dim (or 1-element) fp64 CUDA tensor, log_r [B*S] fp64 from iw_sample.  -> log_w"""
+    _req_cuda(recon_vm, "iw_log_weights recon")
+    _req_cuda(x_gt, "iw_log_weights x_gt", None)
+    _req_cuda(log_sigma, "iw_log_weights log_sigma", torch.float64)
+    _req_cuda(log_r, "iw_log_weights log_r", torch.float64)
+    _req_cuda(log_w, "iw_log_weights log_w", torch.float64)
+    if x_gt.dtype not in (torch.float32, torch.float64):
+        raise _lib.MvbError(f"iw_log_weights: x_gt must be fp32 or fp64, got {x_gt.dtype}")
+    if log_sigma.numel() != 1:
+        raise _lib.MvbError(f"iw_log_weights: log_sigma has {log_sigma.numel()} elements, expected 1")
+    n, bs, ld = recon_vm.shape
+    c = int(ld if channels is None else channels)
+    b = x_gt.shape[0]
+    if x_gt.dim() != 3 or tuple(x_gt.shape[1:]) != (n, c) or c > ld or b < 1 or bs % b:
+        raise _lib.MvbError(f"iw_log_weights: x_gt is {tuple(x_gt.shape)}, recon {tuple(recon_vm.shape)}: expected x_gt (B, {n}, {c}) "
+                            f"with B dividing {bs}")
+    s = bs // b
+    if log_w.dim() != 2 or log_w.shape[0] != b or not log_w.is_contiguous() or s0 < 0 or s0 + s > log_w.shape[1]:
+        raise _lib.MvbError(f"iw_log_weights: log_w {tuple(log_w.shape)} has no contiguous columns [{s0}, {s0 + s}) for {b} meshes")
+    if tuple(log_r.shape) != (bs,):
+        raise _lib.MvbError(f"iw_log_weights: log_r is {tuple(log_r.shape)}, expected ({bs},)")
+    recon_vm, x_gt, log_r, ls = recon_vm.contiguous(), x_gt.contiguous(), log_r.contiguous(), log_sigma.contiguous()
+    ws_bytes = lib.mvb_iw_log_weights_workspace_bytes(b, s, n)
+    ws = torch.empty(ws_bytes, device=recon_vm.device, dtype=torch.uint8)
+    check(lib.mvb_iw_log_weights(b, s, n, c, ptr(recon_vm), ld, ptr(x_gt), int(x_gt.dtype == torch.float64), ptr(ls), ptr(log_r),
+                                 log_w.shape[1], int(s0), ptr(log_w), ptr(ws), ws_bytes, stream_ptr()), "mvb_iw_log_weights")
+    return log_w
+
+
+def iw_reduce(log_w, return_log_w: bool = False):
+    """log_w [B,S] fp64 -> (log_px, elbo, ess), fp64 [B]: log mean_s exp(log w), mean_s log w and the effective sample size
+    (sum_s w)^2 / sum_s w^2; return_log_w=True appends a copy of log_w"""
+    _req_cuda(log_w, "iw_reduce log_w", torch.float64)
+    if log_w.dim() != 2 or log_w.shape[0] < 1 or log_w.shape[1] < 1:
+        raise _lib.MvbError(f"iw_reduce: log_w is {tuple(log_w.shape)}, expected (B, S)")
+    b, s = log_w.shape
+    log_w = log_w.contiguous()
+    out = [torch.empty(b, device=log_w.device, dtype=torch.float64) for _ in range(3)]
+    copy = torch.empty_like(log_w) if return_log_w else None
+    check(lib.mvb_iw_reduce(b, s, ptr(log_w), ptr(out[0]), ptr(out[1]), ptr(out[2]), ptr(copy), stream_ptr()), "mvb_iw_reduce")
+    return (*out, copy) if return_log_w else tuple(out)
+
+
 class _KldFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mu, logvar):

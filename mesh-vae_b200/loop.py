@@ -173,6 +173,29 @@ def evaluate(n, model, test_loader, device, faces=None, checkpoint_dir=None, vis
     return r["loss"], r["kld"], r["rec_loss"], np.float64(r["accuracy"]), err, int(flipped) / total
 
 
+def log_likelihood(model, loader, device, samples, sample_chunk=None, seed=0, log_sigma=None):
+    """Held-out importance-weighted log-likelihood over a loader of the `evaluate` kind (`cheb_VAE.log_likelihood` per
+    batch, each mesh under its own label, samples drawn from one device generator seeded with `seed`).  Nothing is read
+    back before the end of the loop.  -> dict: per-mesh numpy fp64 arrays `log_px`, `elbo`, `ess`, their means
+    `log_px_mean`, `elbo_mean`, `ess_mean`, and the meshes' file `names` in loader order.  Densities are those of the
+    z-scored coordinates the model is trained on."""
+    gen = torch.Generator(device=device)
+    gen.manual_seed(int(seed))
+    names_all, parts = [], []
+    for data in loader:
+        x, x_gt, y, names, _, _, _, _ = _split(data)
+        x, x_gt = x.to(device, non_blocking=True), x_gt.to(device, non_blocking=True)
+        y_hot = F.one_hot(y, num_classes=model.num_class).to(device, non_blocking=True)
+        parts.append(torch.stack(model.log_likelihood(x, x_gt, y_hot, samples, sample_chunk, gen, log_sigma)))
+        names_all += list(names)
+    res = torch.cat(parts, 1).cpu().numpy() if parts else np.zeros((3, 0))
+    out = {"names": names_all}
+    for i, k in enumerate(("log_px", "elbo", "ess")):
+        out[k] = res[i]
+        out[k + "_mean"] = float(res[i].mean()) if res.shape[1] else float("nan")
+    return out
+
+
 def inference(net, output_path, mean, std, data_loader, faces, device, write_meshes=True):
     """inference.py:55-157 without its dataset construction: for every batch the predicted class of the (normalised)
     input, the reconstruction under that class and the sex-changed mesh under the opposite one; writes the
